@@ -3,6 +3,10 @@
 Mpixel*slices/s) on N B200s of one node.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload si001_1024] [--impl reference]
+                    [--dump-outputs DIR]
+
+--steps K sets the timed steps of `value` and `e2e`; the `stem` and `job` legs time one call each
+whatever K is.  --warmup W runs max(W, 3) untimed steps before `value` with --impl ours.
 
 A *step* is one pass of the hot path over one batch of synthetic input: `configs_per_step`
 frozen-phonon configurations of the workload specimen per GPU (400 for the default workload, so that
@@ -25,6 +29,11 @@ scaling; at N = 1 the same jobs give the single-GPU reference time).
                 (SURVEY 8d: 16 nZ + 80 B per pixel and slice) / the sum of their live CUDA-event launch
                 times, against the measured HBM peak and the nominal 8 TB/s of north_star; the
                 per-sweep table and the whole-step figure (value x bytes) are reported next to it.
+  --dump-outputs DIR  (rank 0) what the timed calls returned in their last step, as DIR/<name>.npy:
+                image (finish_k of the last step's configurations: the phonon-averaged image [n2, n1]),
+                e2e_image (FDES() [1, n2, n1]), stem_signals and the job outputs when those legs run.  The
+                inputs are generated from fixed seeds, so two builds run with the same arguments can be
+                compared output for output.
   cpu_baseline  the numpy/pocketfft restatement (oracle/fdes_oracle.py) on this box's host cores,
                 bounded sample, rank 0 at N=1 only.  Reported baseline, not a target.
 
@@ -166,6 +175,7 @@ def run_ours(a):
     for _ in range(a.warmup):
         sim.bench_configs(0, cps)
     sim.counters(reset=True)
+    outputs = {}
     with ClockSampler(local) as clk:
         time.sleep(0.3)            # let the sampler take its first reading before the timed region
         barrier()
@@ -176,6 +186,8 @@ def run_ours(a):
         barrier()
         t_wall = (time.perf_counter() - t_wall) * 1e3
     cnt = sim.counters()
+    if a.dump_outputs:
+        outputs["image"] = sim.finish_k(0)[0]       # detector tail of the intensity the last step accumulated
     t = torch.tensor([dev_ms, t_wall], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -221,9 +233,11 @@ def run_ours(a):
     e2e_ms = float(t[0])
     e2e_value = world * px * slices_per_step * a.steps / (e2e_ms * 1e-3) / 1e6
     assert np.isfinite(img).all() and img.mean() > 0.1, "FDES() returned an implausible image"
+    if a.dump_outputs:
+        outputs["e2e_image"] = img.copy()
 
-    stem = None if a.no_stem else run_stem(a, fb, specimens, tmp, local, world, barrier, dist, torch)
-    job = None if a.no_job else run_jobs(a, fb, specimens, tmp, local, rank, world, barrier, dist, torch)
+    stem = None if a.no_stem else run_stem(a, fb, specimens, tmp, local, world, barrier, dist, torch, outputs)
+    job = None if a.no_job else run_jobs(a, fb, specimens, tmp, local, rank, world, barrier, dist, torch, outputs)
     if rank != 0:
         if world > 1:
             dist.destroy_process_group()
@@ -281,12 +295,14 @@ def run_ours(a):
         line["job"] = job
     if world == 1 and not a.no_cpu:
         line["cpu_baseline"] = cpu_baseline(cnf, a.cpu_seconds)
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, outputs)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
 
 
-def run_stem(a, fb, specimens, tmp, local, world, barrier, dist, torch):
+def run_stem(a, fb, specimens, tmp, local, world, barrier, dist, torch, outputs):
     """Second metric of BASELINE.json: STEM probes/s on configs[3] (SrTiO3, 512^2 probe grid, 40 slices,
     HAADF + ABF detectors).  Every rank scans its own `probes_per_gpu` positions of the raster (weak
     scaling: 8 x 8192 = the 256 x 256 scan); the transmission stack is built once per call, inside the
@@ -314,6 +330,7 @@ def run_stem(a, fb, specimens, tmp, local, world, barrier, dist, torch):
     peak, _ = peaks()
     alg = 40.0 * m1 * m1 * m3 * n * world / (dev_ms * 1e-3) / 1e9      # A_prop = 40 B/px/slice (SURVEY 8d)
     assert np.isfinite(sig).all() and sig[:, 0].min() > 0
+    outputs["stem_signals"] = sig
     return {"metric": "stem_probes_per_s", "value": round(world * n / (dev_ms * 1e-3), 1), "unit": "probes/s",
             "e2e": {"value": round(world * n / (wall_ms * 1e-3), 1), "unit": "probes/s",
                     "h2d_bytes_per_step": int(mine.nbytes), "d2h_bytes_per_step": int(sig.nbytes)},
@@ -325,7 +342,7 @@ def run_stem(a, fb, specimens, tmp, local, world, barrier, dist, torch):
             "haadf_mean": float(sig[:, 0].mean()), "abf_mean": float(sig[:, 1].mean())}
 
 
-def run_jobs(a, fb, specimens, tmp, local, rank, world, barrier, dist, torch):
+def run_jobs(a, fb, specimens, tmp, local, rank, world, barrier, dist, torch, outputs):
     """Strong scaling: ONE job sharded over the `world` ranks, collective inside the timed region.
       au_2048_x32   BASELINE configs[2]: Au cuboctahedron 2048^2, 32 frozen-phonon configurations; the ranks
                     run 32/world configurations each, all-reduce (NCCL) of the partial intensity, detector tail.
@@ -349,6 +366,7 @@ def run_jobs(a, fb, specimens, tmp, local, rank, world, barrier, dist, torch):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms, coll = float(t[0]), float(t[1])
     assert np.isfinite(img).all() and img.mean() > 0.1
+    outputs["job_au_2048_x32_image"] = img
     out["au_2048_x32"] = {"configs": 32, "grid": [2048, 2048], "slices": 12, "ms": round(ms, 3),
                           "value": round(2048 * 2048 * 12 * 32 / (ms * 1e-3) / 1e6, 1), "unit": UNIT,
                           "collective": "all_reduce(SUM) of the partial intensity, 2048^2 float32",
@@ -369,11 +387,23 @@ def run_jobs(a, fb, specimens, tmp, local, rank, world, barrier, dist, torch):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t[0])
         assert sig.shape == (len(pos), 2) and np.isfinite(sig).all()
+        outputs["job_stem_256x256_signals"] = sig
         out["stem_256x256"] = {"probes": int(len(pos)), "grid": [512, 512], "slices": 40, "ms": round(ms, 3),
                                "value": round(len(pos) / (ms * 1e-3), 1), "unit": "probes/s",
                                "collective": "all_gather of the detector signals [probes][2] float32"}
     out["scaling"] = "strong"
     return out
+
+
+def dump_outputs(directory, outputs):
+    """--dump-outputs: one float32 / float64 .npy per array, 64 MB in all at most."""
+    d = pathlib.Path(directory)
+    d.mkdir(parents=True, exist_ok=True)
+    arrays = {name: np.ascontiguousarray(v) for name, v in outputs.items()}
+    assert all(v.dtype in (np.float32, np.float64) for v in arrays.values())
+    assert sum(v.nbytes for v in arrays.values()) <= 64 << 20, {n: v.nbytes for n, v in arrays.items()}
+    for name, v in arrays.items():
+        np.save(d / f"{name}.npy", v)
 
 
 def cpu_baseline(cnf, budget_s):
@@ -468,7 +498,11 @@ def main():
     ap.add_argument("--no-stem", action="store_true")
     ap.add_argument("--stem-probes", type=int, default=8192)
     ap.add_argument("--stem-batch", type=int, default=37)   # 24 column tiles x 37 probes = 6.0 waves of 148 SMs
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed calls returned in their last step to DIR/<name>.npy")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     a.warmup = max(a.warmup, 3) if a.impl == "ours" else a.warmup
     if a.impl == "reference":
         run_reference(a)

@@ -5,7 +5,13 @@ variant each with `pixel_dose: 0` (deterministic detector tail).  Shared by tool
 
 Golden content per case (reductions keep the repository small): the image of the measurements K_KEEP,
 mean and L2 norm of every image, a central crop of the coherent exit wave of the same measurements and
-the sum of |psi|^2 of every exit wave."""
+the sum of |psi|^2 of every exit wave.  <case>.npz holds the per-image statistics,
+<case>.k<i>.<array>.<j>.npz the rows of chunk j of an array of the i-th kept measurement.
+
+The shipped EMD file (Au_cubeoctahedron_emd/Auparticle.emd, 2.6 MB, almost all of it unused HDF5 space)
+is stored xz-compressed as tests/golden/shipped_inputs/Auparticle.emd.xz; au_particle_emd() gives its exact
+bytes back."""
+import lzma
 import pathlib
 import re
 import shutil
@@ -27,6 +33,8 @@ CASES = {
     "srtio3_qsc_dose0": ("ExampleSpecimens/SrTiO3_qsc/SrTiO3.qsc", 0.0),
 }
 CROP = 96          # half-width of the central exit-wave crop
+PER_K = ("image_keep", "ew_crop", "ew_crop_fp64")     # arrays stored per kept measurement, in row chunks
+CHUNK = 800_000    # bytes of a stored chunk: every golden file stays under 1 MB
 # focused probe through 400 sub-slices: the goldens also carry a float64 evaluation of the model
 DEEP_PROBE_CASES = ("bin_test_qsc", "bin_test_qsc_dose0", "srtio3_qsc", "srtio3_qsc_dose0")
 
@@ -68,3 +76,33 @@ def reduce(image: np.ndarray, exitwave: np.ndarray) -> dict:
         "ew_power": (np.abs(exitwave.reshape(n3, -1).astype(np.complex128)) ** 2).sum(axis=1),
         "shape": np.array([n3, image.shape[1], image.shape[2], m2, m1], np.int32),
     }
+
+
+def au_particle_emd(workdir: pathlib.Path) -> pathlib.Path:
+    """The reference's shipped ExampleSpecimens/Au_cubeoctahedron_emd/Auparticle.emd, unpacked into workdir."""
+    src = SHIPPED.parent.parent / "golden" / "shipped_inputs" / "Auparticle.emd.xz"
+    workdir.mkdir(parents=True, exist_ok=True)
+    dst = workdir / "Auparticle.emd"
+    dst.write_bytes(lzma.decompress(src.read_bytes()))
+    return dst
+
+
+def save_golden(directory: pathlib.Path, case: str, g: dict) -> None:
+    np.savez_compressed(directory / f"{case}.npz", **{k: v for k, v in g.items() if k not in PER_K})
+    for key in PER_K:
+        for i, a in enumerate(g.get(key, [])):
+            for j, part in enumerate(np.array_split(a, -(-a.nbytes // CHUNK), axis=0)):
+                np.savez_compressed(directory / f"{case}.k{i}.{key}.{j}.npz", a=part)
+
+
+def load_golden(directory: pathlib.Path, case: str) -> dict:
+    g = dict(np.load(directory / f"{case}.npz"))
+    for key in PER_K:
+        per_k = []
+        for i in range(len(g["k_keep"])):
+            parts = sorted(directory.glob(f"{case}.k{i}.{key}.*.npz"), key=lambda f: int(f.stem.rsplit(".", 1)[1]))
+            if parts:
+                per_k.append(np.concatenate([np.load(f)["a"] for f in parts]))
+        if per_k:
+            g[key] = np.stack(per_k)
+    return g

@@ -7,19 +7,19 @@ representative header messages in tests/golden/emd_structure.json.  The product'
 (fdes_b200/csrc/emd.cpp) must produce files that (a) h5min parses, (b) have the same groups,
 datasets, dtypes and attributes in the same order, (c) carry byte-identical header messages for
 identical content, (d) hold the arrays in the reference's transposed layouts, and (e) read back
-through the product's own reader (the .emd input path).  Where /root/reference is mounted the
-product's reader is also run on the real file and compared with its .cnf twin."""
+through the product's own reader (the .emd input path).  The product's reader is also run on the
+real file (shipped_cases.au_particle_emd: its exact bytes, stored compressed under
+tests/golden/shipped_inputs/) and compared with its .cnf twin."""
 import json
-import pathlib
 
 import numpy as np
 import pytest
 
 import h5min
+import shipped_cases as sc
 from conftest import DATA, GOLDEN, ROOT
 
-REAL = pathlib.Path("/root/reference/ExampleSpecimens/Au_cubeoctahedron_emd/Auparticle.emd")
-REAL_CNF = pathlib.Path("/root/reference/ExampleSpecimens/Au_cubeoctahedron_cnf/dataFDES_Auparticle.cnf")
+REAL_CNF = sc.SHIPPED / "ExampleSpecimens" / "Au_cubeoctahedron_cnf" / "dataFDES_Auparticle.cnf"
 FIX = json.loads((GOLDEN / "emd_structure.json").read_text())
 
 
@@ -150,13 +150,13 @@ def test_reader_rejects_what_is_not_an_emd(fb, tmp_path):
     assert lib.fdes_b200_parse_cnf(str(cut).encode(), None, None, None, None, 0) == -1
 
 
-@pytest.mark.skipif(not REAL.exists(), reason="reference tree not mounted")
-def test_h5min_and_product_reader_on_the_real_libhdf5_file(fb):
+def test_h5min_and_product_reader_on_the_real_libhdf5_file(fb, tmp_path):
     """The file libhdf5 wrote: h5min's structure equals the committed fixture, and the product's
     reader returns what the .cnf twin of the same specimen holds (SURVEY section 8c: same parameters)."""
-    f = h5min.File(REAL)
+    real = sc.au_particle_emd(tmp_path)
+    f = h5min.File(real)
     assert {p: n for p, n in ((p, list(n.attrs)) for p, n in f.root.walk())} == {p: v["attrs"] for p, v in FIX["paths"].items()}
-    e = fb.parse_cnf(REAL)
+    e = fb.parse_cnf(real)
     c = fb.parse_cnf(REAL_CNF)
     for k in ("n1", "n2", "n3", "m1", "m2", "m3", "nZ", "frPh", "mode", "lam", "sigma", "gamma", "d1", "d2", "d3", "E0", "imPot"):
         assert e[k] == c[k], k
@@ -215,9 +215,8 @@ def test_reader_survives_corrupted_files(fb, tmp_path):
     """The .emd input path is reachable from FDES() and the CLI: truncated or corrupted HDF5 bytes
     (undefined addresses 0xFF..FF, broken B-tree / heap offsets, unterminated names) must end in an error
     code or in parsed values, never in an out-of-bounds read."""
-    import shipped_cases as sc
     lib = fb.load_library()
-    src = (sc.SHIPPED / "ExampleSpecimens" / "Au_cubeoctahedron_emd" / "Auparticle.emd").read_bytes()
+    src = sc.au_particle_emd(tmp_path).read_bytes()
     rng = np.random.default_rng(0)
     rejected = 0
     for i in range(120):

@@ -251,13 +251,11 @@ def test_srtio3_800_qsc_against_live_reference(ncell_z, tol_wave, fb, orc, qorc,
     wave -- our exit wave and image against the unmodified reference run here, N = 5 (100 sub-slices),
     held to the north-star bound of 1e-5.  The full depth (N = 20, 400 sub-slices) is examined in
     tests/test_reference_live_gpu.py::test_srtio3_800_400_subslices_error_budget against a float64
-    evaluation of the model."""
+    evaluation of the model.  Without the reference build: the comparison with the oracle."""
     import subprocess
-    from conftest import ROOT
+    from conftest import ROOT, live_reference_missing
     from fdes_b200 import specimens
     harness = ROOT / "oracle" / "_ref" / "ref_harness"
-    if not harness.exists():
-        pytest.skip("oracle/_ref/ref_harness not built")
     qsc = specimens.config_srtio3_qsc_800(tmp_path, ncell_z=ncell_z)
     cwd = os.getcwd()
     os.chdir(tmp_path)
@@ -268,16 +266,21 @@ def test_srtio3_800_qsc_against_live_reference(ncell_z, tol_wave, fb, orc, qorc,
         p, Z, xyz, dwf, occ = qorc.read_qsc(str(qsc))
     finally:
         os.chdir(cwd)
+    res = orc.build_measurements(p, Z, xyz, dwf, occ) if ncell_z == 5 else None
+    if res is not None:
+        print(f"srtio3_800 N={ncell_z}: ours-vs-oracle {rel_l2(ew, res.exitwave):.3e}, image {rel_l2(img, res.image):.3e}")
+        assert rel_l2(ew, res.exitwave) < tol_wave
+        assert rel_l2(img, res.image) < TOL_INTENSITY
+    if live_reference_missing(harness):
+        return
     out = tmp_path / "ref"
     subprocess.run([str(harness), "run", str(qsc), str(out), "2"], check=True, capture_output=True)
     rimg = np.fromfile(out / "image.f32", np.float32).reshape(img.shape)
     rew = np.fromfile(out / "exitwave.f32", np.float32).view(np.complex64).reshape(ew.shape)
     d_ref = rel_l2(ew, rew)
     print(f"srtio3_800 N={ncell_z}: ours-vs-reference exit wave {d_ref:.3e}, image {rel_l2(img, rimg):.3e}")
-    if ncell_z == 5:
-        res = orc.build_measurements(p, Z, xyz, dwf, occ)
-        print(f"   ours-vs-oracle {rel_l2(ew, res.exitwave):.3e}, reference-vs-oracle {rel_l2(rew, res.exitwave):.3e}")
-        assert rel_l2(ew, res.exitwave) < tol_wave
+    if res is not None:
+        print(f"   reference-vs-oracle {rel_l2(rew, res.exitwave):.3e}")
     assert d_ref < tol_wave
     assert rel_l2(img, rimg) < TOL_INTENSITY
 

@@ -10,7 +10,11 @@ see oracle/ref_harness.cu), at sizes the numpy oracle would need minutes for:
   * configs[0]  SrTiO3 800^2 from .qsc, 400 sub-slices: three-way distances with a float64 evaluation
                 of the same model (oracle.exit_wave_fp64) and two runs of the reference
 
-Bounds are north_star's: exit waves rel-L2 <= 1e-5, detector intensities <= 1e-4.
+Bounds are north_star's: exit waves rel-L2 <= 1e-5, detector intensities <= 1e-4.  Where the reference
+build is absent, each test compares the library on the same input with the numpy oracle instead (the
+independent float32 restatement of the reference that tests/test_oracle_golden.py pins to the
+reference's recorded outputs), under the same bounds, and a warning says that the live comparison did
+not run.
 """
 import os
 import subprocess
@@ -18,11 +22,21 @@ import subprocess
 import numpy as np
 import pytest
 
-from conftest import ROOT, TOL_INTENSITY, TOL_WAVE, rel_l2
+from conftest import ROOT, TOL_INTENSITY, TOL_WAVE, live_reference_missing, rel_l2
 
 pytestmark = pytest.mark.gpu
 HARNESS = ROOT / "oracle" / "_ref" / "ref_harness"
-needs_ref = pytest.mark.skipif(not HARNESS.exists(), reason="oracle/_ref/ref_harness not built (needs /root/reference)")
+# rel-L2 of the reference's exit wave to the float64 evaluation at BASELINE configs[0] (400 sub-slices, plane
+# wave), measured in the live comparison of test_srtio3_800_400_subslices_error_budget (DESIGN.md)
+REF_FP64_SRTIO3_400 = 1.8e-5
+
+
+def _against_oracle(orc, cnf, img, ew):
+    p, Z, xyz, dwf, occ = orc.read_cnf(str(cnf))
+    res = orc.build_measurements(p, Z, xyz, dwf, occ)
+    d_ew, d_img = rel_l2(ew, res.exitwave), rel_l2(img, res.image)
+    print(f"{cnf.name} against the oracle: exit wave {d_ew:.3e}, image {d_img:.3e}")
+    assert d_ew < TOL_WAVE and d_img < TOL_INTENSITY
 
 
 def _ref_run(cnf, out, shape_img, shape_ew):
@@ -32,22 +46,22 @@ def _ref_run(cnf, out, shape_img, shape_ew):
     return rimg, rew
 
 
-@needs_ref
-def test_au_2048_frozen_phonons_against_live_reference(fb, tmp_path):
+def test_au_2048_frozen_phonons_against_live_reference(fb, orc, tmp_path):
     from fdes_b200 import specimens
     cnf = tmp_path / "au.cnf"
     specimens.config_au_2048(cnf, frozen_phonons=3)
     with fb.Simulation(cnf, want_exitwave=True) as sim:
         assert (sim.m1, sim.configs) == (2048, 3)
         img, ew = sim.simulate()
+    if live_reference_missing(HARNESS):
+        return _against_oracle(orc, cnf, img, ew)
     rimg, rew = _ref_run(cnf, tmp_path / "ref", img.shape, ew.shape)
     d_ew, d_img = rel_l2(ew, rew), rel_l2(img, rimg)
     print(f"au_2048 x 3 phonon configurations: exit wave {d_ew:.3e}, image {d_img:.3e}")
     assert d_ew < TOL_WAVE and d_img < TOL_INTENSITY
 
 
-@needs_ref
-def test_slab_4096_three_species_50_slices_against_live_reference(fb, tmp_path):
+def test_slab_4096_three_species_50_slices_against_live_reference(fb, orc, tmp_path):
     from fdes_b200 import specimens
     cnf = tmp_path / "slab.cnf"
     atoms = specimens.random_slab(10_000, 4096 * 0.1e-10, 50 * 2e-10)
@@ -56,13 +70,14 @@ def test_slab_4096_three_species_50_slices_against_live_reference(fb, tmp_path):
     with fb.Simulation(cnf, want_exitwave=True) as sim:
         assert (sim.m1, sim.m3, sim.nZ) == (4096, 50, 3)
         img, ew = sim.simulate()
+    if live_reference_missing(HARNESS):
+        return _against_oracle(orc, cnf, img, ew)
     rimg, rew = _ref_run(cnf, tmp_path / "ref", img.shape, ew.shape)
     d_ew, d_img = rel_l2(ew, rew), rel_l2(img, rimg)
     print(f"slab_4096, 3 species x 50 slices: exit wave {d_ew:.3e}, image {d_img:.3e}")
     assert d_ew < TOL_WAVE and d_img < TOL_INTENSITY
 
 
-@needs_ref
 def test_stem_512_offcentre_probes_against_live_reference(fb, orc, tmp_path):
     from fdes_b200 import specimens
     N, d = 512, 19.525e-10 / 512
@@ -77,6 +92,14 @@ def test_stem_512_offcentre_probes_against_live_reference(fb, orc, tmp_path):
     with fb.Simulation(cnf, batch=4) as sim:
         assert (sim.m1, sim.m3) == (512, 40)
         got, ms = sim.stem_scan(pos, det)
+    if live_reference_missing(HARNESS):
+        from test_parity_gpu import _oracle_stem     # the reference algorithm per probe: translated atoms, mode 2
+        p, Z, xyz, dwf, occ = orc.read_cnf(str(cnf))
+        want = _oracle_stem(orc, p, Z, [xyz], occ, pos, det)
+        print("STEM 512^2 x 40 slices, ours / oracle per probe and detector:\n", got / want)
+        assert np.all(want[:, 2] > 1.0)
+        np.testing.assert_allclose(got, want, rtol=TOL_INTENSITY, atol=1e-4 * want.max())
+        return
     p = orc.read_cnf(str(cnf))[0]
     lam = np.float32(p.lam)
     kx = (orc.ow(N).astype(np.float32) / np.float32(N * np.float32(d)))[None, :]
@@ -100,12 +123,13 @@ def test_stem_512_offcentre_probes_against_live_reference(fb, orc, tmp_path):
     np.testing.assert_allclose(got, want, rtol=TOL_INTENSITY, atol=1e-4 * want.max())
 
 
-@needs_ref
 def test_srtio3_800_400_subslices_error_budget(fb, orc, qorc, tmp_path):
     """BASELINE configs[0] at its full depth (400 sub-slices = 1600 chained float32 transforms in both
     programs).  Whose rounding is it?  Distances to the float64 evaluation of the same model:
     the library must be within 1e-5 of the reference, or at least as close to the exact result as
-    the reference itself is (x 1.25 for run-to-run scatter of the reference's float atomics)."""
+    the reference itself is (x 1.25 for run-to-run scatter of the reference's float atomics).  Without the
+    reference build: at least as close to the float64 evaluation as the reference was when measured live
+    (REF_FP64_SRTIO3_400), and the image against the oracle's."""
     from fdes_b200 import specimens
     qsc = specimens.config_srtio3_qsc_800(tmp_path, ncell_z=20)
     cwd = os.getcwd()
@@ -117,9 +141,17 @@ def test_srtio3_800_400_subslices_error_budget(fb, orc, qorc, tmp_path):
         p, Z, xyz, dwf, occ = qorc.read_qsc(str(qsc))
     finally:
         os.chdir(cwd)
+    truth = orc.exit_wave_fp64(p, Z, xyz, occ).reshape(ew.shape)
+    if live_reference_missing(HARNESS):
+        res = orc.build_measurements(p, Z, xyz, dwf, occ)
+        d = {"ours-fp64": rel_l2(ew, truth), "image ours-oracle": rel_l2(img, res.image)}
+        print("srtio3_800, 400 sub-slices: " + ", ".join(f"{k} {v:.3e}" for k, v in d.items()))
+        assert d["ours-fp64"] <= 1.25 * REF_FP64_SRTIO3_400, d
+        assert d["ours-fp64"] < 3 * TOL_WAVE
+        assert d["image ours-oracle"] < TOL_INTENSITY
+        return
     rimg1, rew1 = _ref_run(qsc, tmp_path / "ref1", img.shape, ew.shape)
     rimg2, rew2 = _ref_run(qsc, tmp_path / "ref2", img.shape, ew.shape)
-    truth = orc.exit_wave_fp64(p, Z, xyz, occ).reshape(ew.shape)
     d = {"ours-ref": rel_l2(ew, rew1), "ours-fp64": rel_l2(ew, truth), "ref-fp64": rel_l2(rew1, truth),
          "ref-ref": rel_l2(rew1, rew2), "image ours-ref": rel_l2(img, rimg1)}
     print("srtio3_800, 400 sub-slices: " + ", ".join(f"{k} {v:.3e}" for k, v in d.items()))
@@ -129,9 +161,8 @@ def test_srtio3_800_400_subslices_error_budget(fb, orc, qorc, tmp_path):
     assert d["image ours-ref"] < TOL_INTENSITY
 
 
-@needs_ref
 @pytest.mark.parametrize("seed", [1, 2, 3, 4, 5, 6, 7])
-def test_random_grid_sizes_against_live_reference(seed, fb, tmp_path):
+def test_random_grid_sizes_against_live_reference(seed, fb, orc, tmp_path):
     """Any sample size the reference accepts (seeds 5 .. 7: odd sizes) (m = n + 2 dn, src/paramStructure.cu:650-651): random
     image / border sizes, random mode, 3 species, against the unmodified reference run on the same input.
     Sizes without a register-resident instantiation take the generic run-time-N sweeps."""
@@ -150,6 +181,8 @@ def test_random_grid_sizes_against_live_reference(seed, fb, tmp_path):
     with fb.Simulation(cnf, want_exitwave=True) as sim:
         assert sim.m1 == m
         img, ew = sim.simulate()
+    if live_reference_missing(HARNESS):
+        return _against_oracle(orc, cnf, img, ew)
     rimg, rew = _ref_run(cnf, tmp_path / "ref", img.shape, ew.shape)
     d_ew, d_img = rel_l2(ew, rew), rel_l2(img, rimg)
     print(f"grid {m} = {n} + 2 x {dn}, mode {mode}: exit wave {d_ew:.3e}, image {d_img:.3e}")

@@ -35,7 +35,7 @@ def _golden(case):
     f = GOLDEN / "shipped" / f"{case}.npz"
     if not f.exists():
         pytest.fail(f"{f} missing (tools/make_shipped_golden.py)")
-    return np.load(f)
+    return sc.load_golden(f.parent, case)
 
 
 def _run(fb, path, workdir):
@@ -90,6 +90,6 @@ def test_shipped_emd_input_matches_its_cnf_twin(fb, tmp_path):
     """ExampleSpecimens/Au_cubeoctahedron_emd/Auparticle.emd (written by libhdf5 for the reference) read by
     the library's own HDF5 parser: same parameters and atoms as the .cnf twin (SURVEY 8c), so the golden
     of that file applies."""
-    emd = sc.SHIPPED / "ExampleSpecimens" / "Au_cubeoctahedron_emd" / "Auparticle.emd"
+    emd = sc.au_particle_emd(tmp_path)
     img, ew = _run(fb, emd, tmp_path)
     _compare("au_particle_cnf", img, ew, noisy=True)

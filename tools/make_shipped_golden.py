@@ -63,7 +63,7 @@ def main():
                 g["ew_crop_fp64"], g["ew_power_fp64"] = r64["ew_crop"], r64["ew_power"]
             g["meta_keys"] = np.array(sorted(meta))
             g["meta_vals"] = np.array([meta[k] for k in sorted(meta)], np.float64)
-            np.savez_compressed(out / f"{case}.npz", **g)
+            sc.save_golden(out, case, g)
             print(f"golden {case}: {m1}x{m2}, m3={int(meta.get('m3', 0))}, n3={n3}, mode={int(meta.get('mode', -1))}, "
                   f"reference took {time.time() - t0:.1f} s", flush=True)
 
