@@ -25,10 +25,6 @@
 #include <cuda.h>
 #include <cstdint>
 
-#ifndef FDES_SPLIT_2048
-#define FDES_SPLIT_2048 1
-#endif
-
 namespace fdes {
 
 // ---------------------------------------------------------------------------------------------
@@ -112,7 +108,7 @@ struct PipeCfg {
     static constexpr size_t SMEM = OFF_BAR + 64;
     static constexpr bool WARP_SYNC = (T <= 32);
     // 2048-point columns as TWO 1024-point transforms, each inside one warp (see ColPipe::acquire_fft)
-    static constexpr bool SPLIT = (N == 2048) && (FDES_SPLIT_2048 != 0);
+    static constexpr bool SPLIT = (N == 2048);
     static_assert(N >= 512 && (N & (N - 1)) == 0 && N <= 4096, "pipelined column tiles: N = 512 .. 4096, power of two");
     static_assert(T % 8 == 0, "swizzle phase of a thread must not depend on m");
 };
@@ -136,10 +132,10 @@ struct PipeSync {
 //                         starts the store
 // finish() before the kernel exits.
 // DBG (microbenchmarks only): bit 0 = no tile loads, bit 1 = no tile stores.
-template <int N, int DBG = 0, bool ALLOW_SPLIT = true>
+template <int N, int DBG = 0>
 struct ColPipe {
     using C = PipeCfg<N>;
-    static constexpr bool SPLIT = C::SPLIT && ALLOW_SPLIT;
+    static constexpr bool SPLIT = C::SPLIT;
     static constexpr int E = C::E, T = C::T;
     unsigned char* base;       // 1024-byte aligned shared memory
     uint64_t *full, *sfree;
@@ -305,7 +301,7 @@ struct ColPipe {
                     x[m] = padd(v0, v1);
                 }
             } else {
-                split_first_odd<0>(x, p, lane, twd, keep, twd.template at<SPLIT_TW>(lane));
+                split_first_odd<0>(x, p, lane, twd, keep);
             }
             __syncthreads();                       // every thread has its points: L may be overwritten
             if (threadIdx.x == 0 && have_next) issue_load(map, x0_next, z_next);
@@ -319,31 +315,23 @@ struct ColPipe {
     }
     // x[M] = (f[j] - f[j + N/2]) W^j, j = lane + 32 M (compile-time table offsets)
     template <int M, class TW, class Keep>
-    __device__ __forceinline__ void split_first_odd(cpx (&x)[E], const unsigned char* p, int lane, TW twd, Keep keep, cpx wlane) const
+    __device__ __forceinline__ void split_first_odd(cpx (&x)[E], const unsigned char* p, int lane, TW twd, Keep keep) const
     {
         if constexpr (M < E) {
             cpx v0 = *reinterpret_cast<const cpx*>(p + M * (32 * C::ROWB));
             cpx v1 = *reinterpret_cast<const cpx*>(p + M * (32 * C::ROWB) + (N / 2) * C::ROWB);
             if (!keep.split(M)) v0 = make_float2(0.f, 0.f);
             if (!keep.split(M + E)) v1 = make_float2(0.f, 0.f);
-#if FDES_SPLIT_TW_CONST_COLS
-            x[M] = split_twiddle<N, E, -1, M>(psub(v0, v1), wlane);
-#else
             x[M] = cmul(psub(v0, v1), twd.template at<SPLIT_TW + 32 * M>(lane));
-#endif
-            split_first_odd<M + 1>(x, p, lane, twd, keep, wlane);
+            split_first_odd<M + 1>(x, p, lane, twd, keep);
         }
     }
     template <int M, class TW>
-    __device__ __forceinline__ void split_last_odd(cpx (&x)[E], int lane, TW twd, cpx wlane) const
+    __device__ __forceinline__ void split_last_odd(cpx (&x)[E], int lane, TW twd) const
     {
         if constexpr (M < E) {
-#if FDES_SPLIT_TW_CONST_COLS
-            x[M] = split_twiddle<N, E, 1, M>(x[M], wlane);
-#else
             x[M] = cmul_conj(x[M], twd.template at<SPLIT_TW + 32 * M>(lane));
-#endif
-            split_last_odd<M + 1>(x, lane, twd, wlane);
+            split_last_odd<M + 1>(x, lane, twd);
         }
     }
     // inverse transform (skipped for an all-zero spectrum: do_fft = false), optional scale, and hand-over
@@ -375,7 +363,7 @@ struct ColPipe {
 #pragma unroll
                 for (int m = 0; m < E / 2; m++) mine[m * 32 + lane] = x[m + E / 2];
             } else {
-                split_last_odd<0>(x, lane, twd, twd.template at<SPLIT_TW>(lane));
+                split_last_odd<0>(x, lane, twd);
 #pragma unroll
                 for (int m = 0; m < E / 2; m++) mine[m * 32 + lane] = x[m];
             }

@@ -538,9 +538,8 @@ void Engine::run_slices_plain(int nb)
         if (!skip_s5) launch_multiply_rows(g_, Psi_, Dp, d_stride, nb, first_full && slice == 0, st_);
         if (!skip_s5 && !with_ctf) { launch_propagate_cols(g_, Psi_, Pq_, nb, st_); return; }
         const int img_stride = skip_s5 ? (int)(d_stride / NN) : 1;
-        if (!launch_propagate_cols_from(g_, with_ctf ? W_ : Psi_, skip_s5 ? Dp : Psi_, img_stride, img_stride * nb, Pq_, nb,
-                                        skip_s5, with_ctf ? lens_ : nullptr, st_))
-            throw std::runtime_error("propagate_cols_from missing although the column sweeps are pipelined");
+        launch_propagate_cols_from(g_, with_ctf ? W_ : Psi_, skip_s5 ? Dp : Psi_, img_stride, img_stride * nb, Pq_, nb,
+                                   skip_s5, with_ctf ? lens_ : nullptr, st_);
     };
     // The potential / transmission sweeps S1..S4 run once per PAIR of slices (the two densities
     // share one complex transform); S5/S6 then advance the wave through the two slices in turn.

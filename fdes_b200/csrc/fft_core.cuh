@@ -83,31 +83,22 @@ __device__ __forceinline__ cpx ld_nc_at(const cpx* p)
 }
 // The quarter tables (propagator, scattering factors) are re-read by every tile of every image while the
 // wave functions stream through L2 once per sweep: an evict_last policy keeps the tables resident.
-#ifndef FDES_TABLE_KEEP
-#define FDES_TABLE_KEEP 1
-#endif
 __device__ __forceinline__ uint64_t l2_keep_policy()
 {
     uint64_t pol;
     asm("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
     return pol;
 }
-// KEEP: the callers' switch (quarter_table_apply: FDES_TABLE_KEEP_MAXN)
-template <int OFF, bool KEEP = true>
+template <int OFF>
 __device__ __forceinline__ cpx ld_tab_at(const cpx* p)
 {
-#if FDES_TABLE_KEEP
-    if constexpr (!KEEP) return ld_nc_at<OFF>(p);
     cpx v;
     asm volatile("ld.global.nc.L2::cache_hint.v2.f32 {%0,%1}, [%2+%3], %4;" : "=f"(v.x), "=f"(v.y) : "l"(p), "n"(OFF * 8), "l"(l2_keep_policy()));
     return v;
-#else
-    return ld_nc_at<OFF>(p);
-#endif
 }
 // (the real scattering-factor tables of S2 are nZ x (N/2+1)^2 floats -- 50 MB for three species at 4096^2: kept
 // resident they crowd the tiles out of L2, S2 1643 -> 1943 us; they take the default policy)
-template <int OFF, bool KEEP = false>
+template <int OFF>
 __device__ __forceinline__ float ld_tab_at(const float* p)
 {
     float v;
@@ -211,7 +202,7 @@ __device__ __forceinline__ cpx mul_w32(cpx a)
     else return cmul_const(a, cos32(n), DIR < 0 ? -sin32(n) : sin32(n));
 }
 
-// cos / sin of 2 pi n / 64, n = 0..16 (radix-64 butterflies: a 2048-point row inside one warp)
+// cos / sin of 2 pi n / 64, n = 0..16 (the W^{32 m} factors of the split 2048-point lines, split_twiddle)
 __device__ __forceinline__ constexpr float cos64(int n)
 {
     constexpr float c[17] = {1.00000000000000000000f, 0.99518472667219692873f, 0.98078528040323043058f, 0.95694033573220882438f, 0.92387953251128673848f, 0.88192126434835504956f, 0.83146961230254523567f, 0.77301045336273699338f, 0.70710678118654757274f, 0.63439328416364548779f, 0.55557023301960228867f, 0.47139673682599780857f, 0.38268343236508983729f, 0.29028467725446233105f, 0.19509032201612833135f, 0.09801714032956077016f, 0.00000000000000006123f};
@@ -251,12 +242,11 @@ __device__ __forceinline__ cpx mul_w20(cpx a)
     else if constexpr (n == 15) return mul_di<-DIR>(a);
     else return cmul_const(a, cos20(n), DIR < 0 ? -sin20(n) : sin20(n));
 }
-// v *= exp(DIR * 2 pi i * n / R) with compile-time n; R divides 32 or 20, or is 64
+// v *= exp(DIR * 2 pi i * n / R) with compile-time n; R divides 32 or 20
 template <int DIR, int R, int n>
 __device__ __forceinline__ cpx mul_wR(cpx a)
 {
-    if constexpr (R == 64) return mul_w64<DIR, n>(a);
-    else if constexpr (32 % R == 0) return mul_w32<DIR, (32 / R) * n>(a);
+    if constexpr (32 % R == 0) return mul_w32<DIR, (32 / R) * n>(a);
     else return mul_w20<DIR, (20 / R) * n>(a);
 }
 
@@ -311,7 +301,7 @@ struct Dft<5, DIR> {
 template <int R, int DIR>
 struct Dft {
     static constexpr int R1 = R % 4 == 0 ? 4 : (R % 5 == 0 ? 5 : 2), R2 = R / R1;
-    static_assert(R == 8 || R == 16 || R == 32 || R == 64 || R == 10 || R == 20, "radix 2, 4, 5, 8, 10, 16, 20, 32, 64");
+    static_assert(R == 8 || R == 16 || R == 32 || R == 10 || R == 20, "radix 2, 4, 5, 8, 10, 16, 20, 32");
     __device__ __forceinline__ static void run(cpx (&v)[R])
     {
         cpx y[R1][R2];
@@ -503,14 +493,9 @@ __device__ __forceinline__ void fft_line(cpx (&x)[E], cpx* sm, int theta, const 
 template <int N, int E>
 __host__ __device__ constexpr int split_tw_offset() { return twiddle_offset<N, E, N / 2>() + N / 2; }
 
-// FDES_SPLIT_TW_CONST=1: W^j, j = lane + 32 m, as (compile-time W^{32 m}) x (per-thread W^lane) -- two
-// register multiplications instead of a table load and one multiplication
-#ifndef FDES_SPLIT_TW_CONST
-#define FDES_SPLIT_TW_CONST 1      // rows: S5 at 2048^2 232 -> 211 us (the table loads go through the same L1 as the row loads)
-#endif
-#ifndef FDES_SPLIT_TW_CONST_COLS
-#define FDES_SPLIT_TW_CONST_COLS 0 // pipelined columns (table in shared memory): no gain measured
-#endif
+// W^j, j = lane + 32 m, as (compile-time W^{32 m}) x (per-thread W^lane) -- two register multiplications
+// instead of a table load and one multiplication: S5 at 2048^2 232 -> 211 us (the table loads go through the
+// same L1 as the row loads).  (The pipelined columns keep the table, in shared memory: no gain measured there.)
 template <int N, int E, int DIR, int M>
 __device__ __forceinline__ cpx split_twiddle(cpx v, cpx wlane)
 {
@@ -518,18 +503,13 @@ __device__ __forceinline__ cpx split_twiddle(cpx v, cpx wlane)
     const cpx u = mul_w64<DIR, M>(v);
     return DIR < 0 ? cmul(u, wlane) : cmul_conj(u, wlane);
 }
-template <int N, int E, int DIR, int M, class TW, class Load>
-__device__ __forceinline__ void split_dif_odd(cpx (&x)[E], int lane, TW tw, Load load, cpx wlane)
+template <int N, int E, int DIR, int M, class Load>
+__device__ __forceinline__ void split_dif_odd(cpx (&x)[E], int lane, Load load, cpx wlane)
 {
     if constexpr (M < E) {
         const cpx d = psub(load(lane, M), load(lane, M + E));
-#if FDES_SPLIT_TW_CONST
         x[M] = split_twiddle<N, E, DIR, M>(d, wlane);
-#else
-        const cpx wv = tw.template at<split_tw_offset<N, E>() + 32 * M>(lane);
-        x[M] = DIR < 0 ? cmul(d, wv) : cmul_conj(d, wv);
-#endif
-        split_dif_odd<N, E, DIR, M + 1>(x, lane, tw, load, wlane);
+        split_dif_odd<N, E, DIR, M + 1>(x, lane, load, wlane);
     }
 }
 // load(lane, blk) = f[lane + 32 blk], blk = 0 .. 2E-1 (blk is a compile-time constant after unrolling)
@@ -542,20 +522,15 @@ __device__ __forceinline__ void split_dif(cpx (&x)[E], int w, int lane, TW tw, L
         for (int m = 0; m < E; m++) x[m] = padd(load(lane, m), load(lane, m + E));
     } else {
         const cpx wlane = tw.template at<split_tw_offset<N, E>()>(lane);
-        split_dif_odd<N, E, DIR, 0>(x, lane, tw, load, wlane);
+        split_dif_odd<N, E, DIR, 0>(x, lane, load, wlane);
     }
 }
-template <int N, int E, int DIR, int M, class TW>
-__device__ __forceinline__ void split_twiddle_all(cpx (&x)[E], int lane, TW tw, cpx wlane)
+template <int N, int E, int DIR, int M>
+__device__ __forceinline__ void split_twiddle_all(cpx (&x)[E], cpx wlane)
 {
     if constexpr (M < E) {
-#if FDES_SPLIT_TW_CONST
         x[M] = split_twiddle<N, E, DIR, M>(x[M], wlane);
-#else
-        const cpx wv = tw.template at<split_tw_offset<N, E>() + 32 * M>(lane);
-        x[M] = DIR < 0 ? cmul(x[M], wv) : cmul_conj(x[M], wv);
-#endif
-        split_twiddle_all<N, E, DIR, M + 1>(x, lane, tw, wlane);
+        split_twiddle_all<N, E, DIR, M + 1>(x, wlane);
     }
 }
 // mine / other: 16 x 32 exchange slots of this warp / of the partner warp; pair_sync: barrier of the two
@@ -570,7 +545,7 @@ __device__ __forceinline__ void split_dit_combine(cpx (&x)[E], int w, int lane, 
 #pragma unroll
         for (int m = 0; m < E / 2; m++) mine[m * 32 + lane] = x[m + E / 2];
     } else {
-        split_twiddle_all<N, E, DIR, 0>(x, lane, tw, tw.template at<split_tw_offset<N, E>()>(lane));
+        split_twiddle_all<N, E, DIR, 0>(x, tw.template at<split_tw_offset<N, E>()>(lane));
 #pragma unroll
         for (int m = 0; m < E / 2; m++) mine[m * 32 + lane] = x[m];
     }

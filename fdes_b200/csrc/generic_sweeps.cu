@@ -650,7 +650,7 @@ const SweepVTable* generic_sweep_vtable()
 {
     static const SweepVTable vt = {0, 1, 1, 0, &gen_density_rows, &gen_potential_cols, &gen_transmit_rows, &gen_bandlimit_cols, &gen_multiply_rows,
                                    &gen_propagate_cols, &gen_rows_fft, &gen_rows_fft_sum, &gen_cols_fft, &gen_probe_cols, &gen_detector_tiles,
-                                   &gen_detector_cols, &gen_twiddles, nullptr, nullptr};
+                                   &gen_detector_cols, &gen_twiddles, nullptr, false};
     return &vt;
 }
 

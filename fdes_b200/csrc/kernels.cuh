@@ -63,9 +63,8 @@ void launch_propagate_cols(const SweepGeom& g, cpx* Psi, const cpx* Pq, int batc
 //     band-limited FFT_row(t) that S4 left in D;
 //   lens (table [kx][ky]): the CTF of the image formation (applyLensFunction, src/multisliceSimulation.cu:614-622)
 //     applied in the last slice's column transform pair, out = the CTF-filtered wave.
-// Returns false when the size has no such kernel (generic sweeps, register-staged column kernels; see
-// sweeps_pipelined): the caller then runs the separate sweeps.
-bool launch_propagate_cols_from(const SweepGeom& g, cpx* out, const cpx* src, int src_img_stride, int src_images,
+// Only where sweeps_pipelined(N); throws for any other size (the caller runs the separate sweeps there).
+void launch_propagate_cols_from(const SweepGeom& g, cpx* out, const cpx* src, int src_img_stride, int src_images,
                                 const cpx* Pq, int batch, bool times_n, const cpx* lens, cudaStream_t st);
 
 // ---- STEM probe scan ----------------------------------------------------------------------

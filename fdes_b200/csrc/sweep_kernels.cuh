@@ -22,7 +22,6 @@
 #include <atomic>
 #include <cmath>
 #include <cstdio>
-#include <cstdlib>
 #include <stdexcept>
 #include <string>
 #include <vector>
@@ -65,16 +64,11 @@ struct DeviceOnce {
 // batch): a sweep is launched with programmatic stream serialisation, signals at its very start that its
 // dependents may be scheduled, and waits for its own prerequisites before it touches memory.  The CTAs of
 // sweep i+1 are then resident (index arithmetic, barrier set-up done) when the last CTAs of sweep i drain,
-// instead of being launched after the grid has completed.  FDES_B200_NO_PDL=1 switches it off.
+// instead of being launched after the grid has completed.
 __device__ __forceinline__ void pdl_prologue()
 {
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     asm volatile("griddepcontrol.wait;" ::: "memory");
-}
-static bool pdl_enabled()
-{
-    static const bool on = [] { const char* e = getenv("FDES_B200_NO_PDL"); return !(e && e[0] == '1'); }();
-    return on;
 }
 template <class... KArgs, class... Args>
 void launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args)
@@ -83,7 +77,7 @@ void launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cu
     cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
     cudaLaunchAttribute at[1];
     at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = pdl_enabled() ? 1 : 0;
+    at[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = at; cfg.numAttrs = 1;
     FDES_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...));
 }
@@ -105,11 +99,10 @@ struct LineCfg {
     static constexpr int T = N / E;                     // threads per line
     static constexpr int LS = line_smem_elems<E>(N);    // padded line buffer [elements]
 };
-template <int N, int E_>
-struct RowCfgE {
-    static constexpr int E = E_, T = N / E_;
-    // lines (rows) per CTA; with 64 points per thread a line's buffers are 16 KB + 16 KB, two lines per CTA
-    static constexpr int RPB = E == 64 ? 2 : ((T & (T - 1)) != 0 ? 4 : ((128 / T) > 0 ? (128 / T) : 1));
+template <int N>
+struct RowCfg {
+    static constexpr int E = LineCfg<N>::E, T = N / E;
+    static constexpr int RPB = (T & (T - 1)) != 0 ? 4 : ((128 / T) > 0 ? (128 / T) : 1);   // lines (rows) per CTA
     static constexpr int THREADS = RPB * T;
     static constexpr int LSTRIDE = line_smem_elems<E>(N);
     static constexpr size_t SMEM = (size_t)RPB * LSTRIDE * sizeof(cpx);
@@ -117,19 +110,11 @@ struct RowCfgE {
     static constexpr bool NAMED_SYNC = (T % 32 == 0);  // a line is a whole number of warps
     static constexpr int MIN_CTAS = (N >= 2048 || !WARP_SYNC) ? 2 : FDES_ROW_MIN_CTAS;   // long lines need the registers
 };
-template <int N>
-using RowCfg = RowCfgE<N, LineCfg<N>::E>;
-// S5 at 2048: 64 points per thread -- the 2048-point row is 64 x 32 (two passes, one exchange, the whole row
-// inside ONE warp) instead of 32 x 32 x 2 with named barriers between two warps: 16 % faster although only six
-// warps fit an SM.  (Measured and not adopted: the same for S3, S6 and for 4096-point lines, DESIGN.md section 8.)
-template <int N>
-struct MultiplyRowsCfg { using type = RowCfg<N>; };
-template <>
-struct MultiplyRowsCfg<2048> { using type = RowCfgE<2048, 64>; };
 // threads of one row line: warp-level sync when the line fits a warp, a named barrier when it is a
 // whole number of warps, else (T = 40, 50: lines straddle warps) the whole CTA
-template <int N, class C = RowCfg<N>>
+template <int N>
 struct RowSync {
+    using C = RowCfg<N>;
     int id;
     __device__ __forceinline__ explicit RowSync(int line) : id(line + 1) {}
     __device__ __forceinline__ void operator()() const
@@ -162,18 +147,15 @@ using ColCtx = ColTile<N, LineCfg<N>::E, ColCfg<N>::CW, ColCfg<N>::STAGED>;
 // |ky| fastest: the T threads of a column read consecutive entries): the first half of the points
 // sits at lo + m*T, the second at hi + (N - m*T) with lo = tab + ax*Q + theta and
 // hi = tab + ax*Q - theta -- compile-time offsets.
-// largest grid size whose complex quarter table (the propagator) is read with the evict_last L2 policy
-// (fft_core.cuh: ld_tab_at).  4096^2, 34 MB table: S6 929 -> 861 us per slice of 10 images, S2 unchanged.
-#ifndef FDES_TABLE_KEEP_MAXN
-#define FDES_TABLE_KEEP_MAXN 4096
-#endif
+// A complex table (the propagator) is read with the evict_last L2 policy (fft_core.cuh: ld_tab_at).
+// 4096^2, 34 MB table: S6 929 -> 861 us per slice of 10 images.
 template <int N, int E, int M, class TabT, class F>
 __device__ __forceinline__ void quarter_table_apply(cpx (&x)[E], const TabT* lo, const TabT* hi, F f)
 {
     constexpr int T = N / E;
     if constexpr (M < E) {
-        if constexpr (M < E / 2) x[M] = f(x[M], ld_tab_at<M * T, (N <= FDES_TABLE_KEEP_MAXN)>(lo));
-        else x[M] = f(x[M], ld_tab_at<N - M * T, (N <= FDES_TABLE_KEEP_MAXN)>(hi));
+        if constexpr (M < E / 2) x[M] = f(x[M], ld_tab_at<M * T>(lo));
+        else x[M] = f(x[M], ld_tab_at<N - M * T>(hi));
         quarter_table_apply<N, E, M + 1>(x, lo, hi, f);
     }
 }
@@ -227,7 +209,7 @@ static int band_cols(const SweepGeom& g)
 // together, so that a quarter-table row is fetched once per launch, was measured and gained nothing.)
 struct TileOrder {
     int tiles_x;
-    __device__ __forceinline__ TileOrder(int tiles_x_, int) : tiles_x(tiles_x_) {}
+    __device__ __forceinline__ explicit TileOrder(int tiles_x_) : tiles_x(tiles_x_) {}
     __device__ __forceinline__ int xt(int t) const { return t % tiles_x; }      // column tile
     __device__ __forceinline__ int img(int t) const { return t / tiles_x; }     // image
 };
@@ -237,12 +219,6 @@ constexpr bool pipe_supported() { return N == 512 || N == 1024 || N == 2048 || N
 // (N = 2048 / 4096: tile rows of 32 / 16 bytes.  With generic LD/ST, 255 registers and four-instruction
 // complex multiplies the pipelined kernels were no faster than the register-staged ones there; since those
 // were fixed they are 21 % / 35 % faster: tools/microbench/col_bench.cu, profiles/r2_v4_col_bench.txt)
-// FDES_B200_NO_TMA=1 selects the register-staged column kernels (A/B comparisons)
-static bool pipe_enabled()
-{
-    static const bool on = [] { const char* e = getenv("FDES_B200_NO_TMA"); return !(e && e[0] == '1'); }();
-    return on;
-}
 static int pipe_grid(int ntiles)
 {
     static std::atomic<int> sms[64];
@@ -396,7 +372,7 @@ k_potential_cols_tma(const __grid_constant__ CUtensorMap mapA, const __grid_cons
     constexpr int Q = N / 2 + 1;
     constexpr int E = C::E;
     ColPipe<N> pipe(pipe_smem, tw);
-    const TileOrder ord(tiles_x, ntiles);
+    const TileOrder ord(tiles_x);
     using Pipe = ColPipe<N>;
     const int ky0 = pipe.ky0();                 // x[m] <-> ky = ky0 + m*T
     // positions of this thread's row-mask words
@@ -481,24 +457,21 @@ void launch_potential_cols_n(const SweepGeom& g, cpx* B, const cpx* A, const flo
 {
     if (g.mask_off <= 0) throw std::runtime_error("S2 needs the row masks of the deposit records (SweepGeom::mask_off)");
     if constexpr (pipe_supported<NN>()) {
-        if (pipe_enabled()) {
-            using P = PipeCfg<NN>;
-            FDES_ALLOW_SMEM((k_potential_cols_tma<NN>), P::SMEM);
-            const int tiles_x = NN / P::CW, ntiles = tiles_x * batch;
-            CUtensorMap mapA, mapB;
-            tile_map(&mapA, A, NN, batch * nZ, P::CW, P::BR);
-            tile_map(&mapB, B, NN, batch, P::CW, P::BR);
-            launch_pdl(k_potential_cols_tma<NN>, dim3(pipe_grid(ntiles)), dim3(P::THREADS), P::SMEM, st, mapA, mapB, Gq, rowptr, slice, slice2,
-                                                                                  nZ, rowptr_stride, g.mask_off, cfg_stride, cfg_off2, tiles_x, ntiles, g.tw);
-            FDES_LAUNCH_CHECK();
-            return;
-        }
+        using P = PipeCfg<NN>;
+        FDES_ALLOW_SMEM((k_potential_cols_tma<NN>), P::SMEM);
+        const int tiles_x = NN / P::CW, ntiles = tiles_x * batch;
+        CUtensorMap mapA, mapB;
+        tile_map(&mapA, A, NN, batch * nZ, P::CW, P::BR);
+        tile_map(&mapB, B, NN, batch, P::CW, P::BR);
+        launch_pdl(k_potential_cols_tma<NN>, dim3(pipe_grid(ntiles)), dim3(P::THREADS), P::SMEM, st, mapA, mapB, Gq, rowptr, slice, slice2,
+                                                                              nZ, rowptr_stride, g.mask_off, cfg_stride, cfg_off2, tiles_x, ntiles, g.tw);
+    } else {
+        using C = ColCfg<NN>;
+        FDES_ALLOW_SMEM((k_potential_cols<NN>), C::SMEM);
+        dim3 grid(NN / C::CW, batch);
+        launch_pdl(k_potential_cols<NN>, dim3(grid), dim3(C::THREADS), C::SMEM, st, B, A, Gq, rowptr, slice, slice2, nZ,
+                                                               rowptr_stride, g.mask_off, cfg_stride, cfg_off2, g.tw);
     }
-    using C = ColCfg<NN>;
-    FDES_ALLOW_SMEM((k_potential_cols<NN>), C::SMEM);
-    dim3 grid(NN / C::CW, batch);
-    launch_pdl(k_potential_cols<NN>, dim3(grid), dim3(C::THREADS), C::SMEM, st, B, A, Gq, rowptr, slice, slice2, nZ,
-                                                           rowptr_stride, g.mask_off, cfg_stride, cfg_off2, g.tw);
     FDES_LAUNCH_CHECK();
 }
 
@@ -669,14 +642,6 @@ k_transmit_rows(const cpx* __restrict__ W, cpx* __restrict__ D, int npair, float
 #define FDES_SPLIT_ROWS_MIN_CTAS 3
 #endif
 template <int N>
-constexpr bool row_split_supported() { return N == 2048 && FDES_SPLIT_2048 != 0; }
-// FDES_B200_NO_SPLIT=1 selects the three-pass row kernels (A/B comparisons)
-static bool row_split_enabled()
-{
-    static const bool on = [] { const char* e = getenv("FDES_B200_NO_SPLIT"); return !(e && e[0] == '1'); }();
-    return on;
-}
-template <int N>
 struct SplitRowCfg {
     static constexpr int E = 32, H = N / 2, RPB = 2, THREADS = RPB * 64;
     static constexpr int HLS = line_smem_elems<E>(H);                 // exchange region of one warp
@@ -758,23 +723,19 @@ template <int NN>
 void launch_transmit_rows_n(const SweepGeom& g, const cpx* W, cpx* D, int npair, float imPot, int batch,
                           cudaStream_t st)
 {
-    using C = RowCfg<NN>;
-    if constexpr (row_split_supported<NN>()) {
-        if (row_split_enabled()) {
-            using S = SplitRowCfg<NN>;
-            const size_t smem = S::SMEM_FFT + (size_t)S::RPB * NN * 2 * sizeof(float);
-            FDES_ALLOW_SMEM((k_transmit_rows_split<NN>), smem);
-            Band<NN>::check(g);
-            launch_pdl(k_transmit_rows_split<NN>, dim3(NN / S::RPB, batch), dim3(S::THREADS), smem, st, W, D, npair, imPot, g.tw);
-            FDES_LAUNCH_CHECK();
-            return;
-        }
-    }
-    const size_t smem = C::SMEM + (size_t)C::RPB * NN * 2 * sizeof(float);
-    FDES_ALLOW_SMEM((k_transmit_rows<NN>), smem);
-    dim3 grid(NN / C::RPB, batch);
     Band<NN>::check(g);
-    launch_pdl(k_transmit_rows<NN>, dim3(grid), dim3(C::THREADS), smem, st, W, D, npair, imPot, g.tw);
+    if constexpr (NN == 2048) {
+        using S = SplitRowCfg<NN>;
+        const size_t smem = S::SMEM_FFT + (size_t)S::RPB * NN * 2 * sizeof(float);
+        FDES_ALLOW_SMEM((k_transmit_rows_split<NN>), smem);
+        launch_pdl(k_transmit_rows_split<NN>, dim3(NN / S::RPB, batch), dim3(S::THREADS), smem, st, W, D, npair, imPot, g.tw);
+    } else {
+        using C = RowCfg<NN>;
+        const size_t smem = C::SMEM + (size_t)C::RPB * NN * 2 * sizeof(float);
+        FDES_ALLOW_SMEM((k_transmit_rows<NN>), smem);
+        dim3 grid(NN / C::RPB, batch);
+        launch_pdl(k_transmit_rows<NN>, dim3(grid), dim3(C::THREADS), smem, st, W, D, npair, imPot, g.tw);
+    }
     FDES_LAUNCH_CHECK();
 }
 
@@ -823,7 +784,7 @@ k_bandlimit_cols_tma(const __grid_constant__ CUtensorMap map, int npair, int lo_
     extern __shared__ __align__(1024) unsigned char pipe_smem[];
     constexpr int E = C::E;
     ColPipe<N> pipe(pipe_smem, tw);
-    const TileOrder ord(tiles_x, ntiles);
+    const TileOrder ord(tiles_x);
     const int ky0 = pipe.ky0();                 // x[m] <-> ky = ky0 + m*T
     // image y of the tile list -> entry (b, p) of a [batch][2] stack (npair = 0: plain [batch])
     auto entry = [npair](int y) { return npair == 0 ? y : (y / npair) * 2 + y % npair; };
@@ -858,23 +819,20 @@ template <int NN>
 void launch_bandlimit_cols_n(const SweepGeom& g, cpx* W, int batch, int npair, cudaStream_t st)
 {
     if constexpr (pipe_supported<NN>()) {
-        if (pipe_enabled()) {
-            using P = PipeCfg<NN>;
-            FDES_ALLOW_SMEM((k_bandlimit_cols_tma<NN>), P::SMEM);
-            const int nimg = npair == 0 ? batch : 2 * batch;     // images in the stack
-            const int tiles_x = band_cols(g) / P::CW, ntiles = tiles_x * (npair == 0 ? batch : batch * npair);
-            CUtensorMap map;
-            tile_map(&map, W, NN, nimg, P::CW, P::BR);
-            launch_pdl(k_bandlimit_cols_tma<NN>, dim3(pipe_grid(ntiles)), dim3(P::THREADS), P::SMEM, st, map, npair, g.lo_end, g.hi_start,
-                                                                                  tiles_x, ntiles, g.tw);
-            FDES_LAUNCH_CHECK();
-            return;
-        }
+        using P = PipeCfg<NN>;
+        FDES_ALLOW_SMEM((k_bandlimit_cols_tma<NN>), P::SMEM);
+        const int nimg = npair == 0 ? batch : 2 * batch;     // images in the stack
+        const int tiles_x = band_cols(g) / P::CW, ntiles = tiles_x * (npair == 0 ? batch : batch * npair);
+        CUtensorMap map;
+        tile_map(&map, W, NN, nimg, P::CW, P::BR);
+        launch_pdl(k_bandlimit_cols_tma<NN>, dim3(pipe_grid(ntiles)), dim3(P::THREADS), P::SMEM, st, map, npair, g.lo_end, g.hi_start,
+                                                                              tiles_x, ntiles, g.tw);
+    } else {
+        using C = ColCfg<NN>;
+        FDES_ALLOW_SMEM((k_bandlimit_cols<NN>), C::SMEM);
+        dim3 grid(band_cols(g) / C::CW, npair == 0 ? batch : batch * npair);
+        launch_pdl(k_bandlimit_cols<NN>, dim3(grid), dim3(C::THREADS), C::SMEM, st, W, npair, g.lo_end, g.hi_start, g.tw);
     }
-    using C = ColCfg<NN>;
-    FDES_ALLOW_SMEM((k_bandlimit_cols<NN>), C::SMEM);
-    dim3 grid(band_cols(g) / C::CW, npair == 0 ? batch : batch * npair);
-    launch_pdl(k_bandlimit_cols<NN>, dim3(grid), dim3(C::THREADS), C::SMEM, st, W, npair, g.lo_end, g.hi_start, g.tw);
     FDES_LAUNCH_CHECK();
 }
 
@@ -885,17 +843,17 @@ void launch_bandlimit_cols_n(const SweepGeom& g, cpx* W, int batch, int npair, c
 // an inverse transform is swap(FFT(swap(.))), real and imaginary parts exchanged on the way in and
 // out (see k_transmit_rows).
 template <int N>
-__global__ void __launch_bounds__(MultiplyRowsCfg<N>::type::THREADS, MultiplyRowsCfg<N>::type::MIN_CTAS)
+__global__ void __launch_bounds__(RowCfg<N>::THREADS, RowCfg<N>::MIN_CTAS)
 k_multiply_rows(cpx* __restrict__ Psi, const cpx* __restrict__ Tk, size_t e_batch_stride, int psi_full,
                 const cpx* __restrict__ tw)
 {
     pdl_prologue();
-    using C = typename MultiplyRowsCfg<N>::type;
+    using C = RowCfg<N>;
     extern __shared__ cpx smem[];
     constexpr int E = C::E;
     constexpr int lo_end = Band<N>::lo_end, hi_start = Band<N>::hi_start;
     const int line = threadIdx.x / C::T, theta = threadIdx.x % C::T;
-    const RowSync<N, C> sync(line);
+    const RowSync<N> sync(line);
     const size_t row = (size_t)blockIdx.x * C::RPB + line;
     const cpx* e = Tk + (size_t)blockIdx.y * e_batch_stride + row * N;
     cpx* p = Psi + ((size_t)blockIdx.y * N + row) * N;
@@ -1028,26 +986,20 @@ template <int NN>
 void launch_multiply_rows_n(const SweepGeom& g, cpx* Psi, const cpx* E, size_t e_batch_stride,
                           int batch, bool psi_full, cudaStream_t st)
 {
-    using C = typename MultiplyRowsCfg<NN>::type;
-    if constexpr (row_split_supported<NN>()) {
-        if (row_split_enabled()) {
-            using S = SplitRowCfg<NN>;
-            const size_t smem = S::SMEM_FFT + (size_t)S::RPB * NN * sizeof(cpx);
-            FDES_ALLOW_SMEM((k_multiply_rows_split<NN>), smem);
-            Band<NN>::check(g);
-            launch_pdl(k_multiply_rows_split<NN>, dim3(NN / S::RPB, batch), dim3(S::THREADS), smem, st, Psi, E, e_batch_stride,
-                       psi_full ? 1 : 0, g.tw);
-            FDES_LAUNCH_CHECK();
-            return;
-        }
-    }
-    const size_t smem = C::SMEM + (size_t)C::RPB * NN * sizeof(cpx);
-    FDES_ALLOW_SMEM((k_multiply_rows<NN>), smem);
-    dim3 grid(NN / C::RPB, batch);
     Band<NN>::check(g);
-    // the table of this kernel's points-per-thread follows the common one (make_twiddles_n)
-    const cpx* tw = g.tw + (C::E != LineCfg<NN>::E ? twiddle_table_elems<NN, LineCfg<NN>::E>() : 0);
-    launch_pdl(k_multiply_rows<NN>, dim3(grid), dim3(C::THREADS), smem, st, Psi, E, e_batch_stride, psi_full ? 1 : 0, tw);
+    if constexpr (NN == 2048) {
+        using S = SplitRowCfg<NN>;
+        const size_t smem = S::SMEM_FFT + (size_t)S::RPB * NN * sizeof(cpx);
+        FDES_ALLOW_SMEM((k_multiply_rows_split<NN>), smem);
+        launch_pdl(k_multiply_rows_split<NN>, dim3(NN / S::RPB, batch), dim3(S::THREADS), smem, st, Psi, E, e_batch_stride,
+                   psi_full ? 1 : 0, g.tw);
+    } else {
+        using C = RowCfg<NN>;
+        const size_t smem = C::SMEM + (size_t)C::RPB * NN * sizeof(cpx);
+        FDES_ALLOW_SMEM((k_multiply_rows<NN>), smem);
+        dim3 grid(NN / C::RPB, batch);
+        launch_pdl(k_multiply_rows<NN>, dim3(grid), dim3(C::THREADS), smem, st, Psi, E, e_batch_stride, psi_full ? 1 : 0, g.tw);
+    }
     FDES_LAUNCH_CHECK();
 }
 
@@ -1089,7 +1041,7 @@ k_propagate_cols_tma(const __grid_constant__ CUtensorMap map, const __grid_const
     constexpr int Q = N / 2 + 1;
     constexpr int E = C::E;
     ColPipe<N> pipe(pipe_smem, tw);
-    const TileOrder ord(tiles_x, ntiles);
+    const TileOrder ord(tiles_x);
     const int ky0 = pipe.ky0();                 // x[m] <-> ky = ky0 + m*T
     int t = blockIdx.x;
     if (t >= ntiles) return;
@@ -1129,46 +1081,37 @@ template <int NN>
 void launch_propagate_cols_n(const SweepGeom& g, cpx* Psi, const cpx* Pq, int batch, cudaStream_t st)
 {
     if constexpr (pipe_supported<NN>()) {
-        if (pipe_enabled()) {
-            using P = PipeCfg<NN>;
-            FDES_ALLOW_SMEM((k_propagate_cols_tma<NN>), P::SMEM);
-            const int tiles_x = band_cols(g) / P::CW, ntiles = tiles_x * batch;
-            CUtensorMap map;
-            tile_map(&map, Psi, NN, batch, P::CW, P::BR);
-            launch_pdl(k_propagate_cols_tma<NN>, dim3(pipe_grid(ntiles)), dim3(P::THREADS), P::SMEM, st, map, map, 1, 1.f, Pq,
-                                                                                  (const cpx*)nullptr, g.lo_end, g.hi_start, tiles_x, ntiles, g.tw);
-            FDES_LAUNCH_CHECK();
-            return;
-        }
+        using P = PipeCfg<NN>;
+        FDES_ALLOW_SMEM((k_propagate_cols_tma<NN>), P::SMEM);
+        const int tiles_x = band_cols(g) / P::CW, ntiles = tiles_x * batch;
+        CUtensorMap map;
+        tile_map(&map, Psi, NN, batch, P::CW, P::BR);
+        launch_pdl(k_propagate_cols_tma<NN>, dim3(pipe_grid(ntiles)), dim3(P::THREADS), P::SMEM, st, map, map, 1, 1.f, Pq,
+                                                                              (const cpx*)nullptr, g.lo_end, g.hi_start, tiles_x, ntiles, g.tw);
+    } else {
+        using C = ColCfg<NN>;
+        FDES_ALLOW_SMEM((k_propagate_cols<NN>), C::SMEM);
+        dim3 grid(band_cols(g) / C::CW, batch);
+        launch_pdl(k_propagate_cols<NN>, dim3(grid), dim3(C::THREADS), C::SMEM, st, Psi, Pq, g.lo_end, g.hi_start, g.tw);
     }
-    using C = ColCfg<NN>;
-    FDES_ALLOW_SMEM((k_propagate_cols<NN>), C::SMEM);
-    dim3 grid(band_cols(g) / C::CW, batch);
-    launch_pdl(k_propagate_cols<NN>, dim3(grid), dim3(C::THREADS), C::SMEM, st, Psi, Pq, g.lo_end, g.hi_start, g.tw);
     FDES_LAUNCH_CHECK();
 }
 
 // S6 reading the band columns of another image stack (launch_propagate_cols_from, kernels.cuh): pipelined kernels only
 template <int NN>
-bool launch_propagate_cols_from_n(const SweepGeom& g, cpx* Psi, const cpx* src, int src_img_stride, int src_images, const cpx* Pq,
+void launch_propagate_cols_from_n(const SweepGeom& g, cpx* Psi, const cpx* src, int src_img_stride, int src_images, const cpx* Pq,
                                   int batch, bool times_n, const cpx* lens, cudaStream_t st)
 {
-    if constexpr (pipe_supported<NN>()) {
-        if (pipe_enabled()) {
-            using P = PipeCfg<NN>;
-            FDES_ALLOW_SMEM((k_propagate_cols_tma<NN>), P::SMEM);
-            const int tiles_x = band_cols(g) / P::CW, ntiles = tiles_x * batch;
-            CUtensorMap map_in, map_out;
-            tile_map(&map_in, src, NN, src_images, P::CW, P::BR);
-            tile_map(&map_out, Psi, NN, batch, P::CW, P::BR);
-            // times_n: S5 with psi = 1 returns FFT_row(IFFT_row(D)) = N * D (unnormalised transforms): the same factor here
-            launch_pdl(k_propagate_cols_tma<NN>, dim3(pipe_grid(ntiles)), dim3(P::THREADS), P::SMEM, st, map_in, map_out, src_img_stride,
-                       times_n ? (float)NN : 1.f, Pq, lens, g.lo_end, g.hi_start, tiles_x, ntiles, g.tw);
-            FDES_LAUNCH_CHECK();
-            return true;
-        }
-    }
-    return false;
+    using P = PipeCfg<NN>;
+    FDES_ALLOW_SMEM((k_propagate_cols_tma<NN>), P::SMEM);
+    const int tiles_x = band_cols(g) / P::CW, ntiles = tiles_x * batch;
+    CUtensorMap map_in, map_out;
+    tile_map(&map_in, src, NN, src_images, P::CW, P::BR);
+    tile_map(&map_out, Psi, NN, batch, P::CW, P::BR);
+    // times_n: S5 with psi = 1 returns FFT_row(IFFT_row(D)) = N * D (unnormalised transforms): the same factor here
+    launch_pdl(k_propagate_cols_tma<NN>, dim3(pipe_grid(ntiles)), dim3(P::THREADS), P::SMEM, st, map_in, map_out, src_img_stride,
+               times_n ? (float)NN : 1.f, Pq, lens, g.lo_end, g.hi_start, tiles_x, ntiles, g.tw);
+    FDES_LAUNCH_CHECK();
 }
 
 // =============================================================================================
@@ -1403,7 +1346,7 @@ k_ctf_cols_tma(const __grid_constant__ CUtensorMap map_in, const __grid_constant
     extern __shared__ __align__(1024) unsigned char pipe_smem[];
     constexpr int E = C::E;
     ColPipe<N> pipe(pipe_smem, tw);
-    const TileOrder ord(tiles_x, ntiles);
+    const TileOrder ord(tiles_x);
     const int ky0 = pipe.ky0();                 // x[m] <-> ky = ky0 + m*T
     int t = blockIdx.x;
     if (t >= ntiles) return;
@@ -1433,7 +1376,7 @@ void launch_cols_fft_n(const SweepGeom& g, const cpx* in, void* out, int dir, Co
                      const void* table, float scale, int batch, cudaStream_t st)
 {
     if constexpr (pipe_supported<NN>()) {
-        if (op == COL_MUL_CPX_INV && pipe_enabled() && g.lo_end < g.hi_start) {
+        if (op == COL_MUL_CPX_INV && g.lo_end < g.hi_start) {
             using P = PipeCfg<NN>;
             FDES_ALLOW_SMEM((k_ctf_cols_tma<NN>), P::SMEM);
             const int tiles_x = band_cols(g) / P::CW, ntiles = tiles_x * batch;
@@ -1622,20 +1565,23 @@ void append_twiddles(std::vector<cpx>& tw)
     }
     if ((int)(tw.size() - before) != twiddle_table_elems<N, E>()) throw std::runtime_error("twiddle table size mismatch");
 }
-// The tables a SweepGeom::tw of size N points to: the one of LineCfg<N>::E, followed by the table of S5's own
-// points-per-thread where that differs (MultiplyRowsCfg).
+// The table a SweepGeom::tw of size N points to: the one of LineCfg<N>::E.
 template <int N>
 std::vector<cpx> make_twiddles_n(int = 0)
 {
     std::vector<cpx> tw;
     append_twiddles<N, LineCfg<N>::E>(tw);
-    if constexpr (MultiplyRowsCfg<N>::type::E != LineCfg<N>::E) append_twiddles<N, MultiplyRowsCfg<N>::type::E>(tw);
     if (tw.empty()) tw.push_back(make_float2(1.f, 0.f));
     return tw;
 }
 
+// S6 from another image stack exists where the column sweeps are pipelined
 template <int N>
-bool sweeps_pipelined_n() { return pipe_supported<N>() && pipe_enabled(); }
+constexpr decltype(SweepVTable::propagate_cols_from) propagate_cols_from_entry()
+{
+    if constexpr (pipe_supported<N>()) return &launch_propagate_cols_from_n<N>;
+    else return nullptr;
+}
 
 // the launchers of one grid size, collected for the run-time dispatch in sweeps.cu
 template <int N>
@@ -1647,7 +1593,7 @@ const SweepVTable* make_sweep_vtable()
         &launch_bandlimit_cols_n<N>, &launch_multiply_rows_n<N>, &launch_propagate_cols_n<N>,
         &launch_rows_fft_n<N>, &launch_rows_fft_sum_n<N>, &launch_cols_fft_n<N>,
         &launch_probe_cols_n<N>, &detector_tiles_n<N>, &launch_detector_cols_n<N>,
-        &make_twiddles_n<N>, &launch_propagate_cols_from_n<N>, &sweeps_pipelined_n<N>,
+        &make_twiddles_n<N>, propagate_cols_from_entry<N>(), pipe_supported<N>(),
     };
     return &vt;
 }

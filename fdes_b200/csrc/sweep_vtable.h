@@ -32,9 +32,9 @@ struct SweepVTable {
     int (*detector_tiles)(const SweepGeom&);
     void (*detector_cols)(const SweepGeom&, const cpx*, float*, float*, const DetectorRings&, float, float, float, int, cudaStream_t);
     std::vector<cpx> (*make_twiddles)(int N);
-    // optional (may be null): S6 reading another image stack, see launch_propagate_cols_from
-    bool (*propagate_cols_from)(const SweepGeom&, cpx*, const cpx*, int, int, const cpx*, int, bool, const cpx*, cudaStream_t);
-    bool (*pipelined)();      // optional: the column sweeps of this size run on the TMA pipeline
+    // null where pipelined is false: S6 reading another image stack, see launch_propagate_cols_from
+    void (*propagate_cols_from)(const SweepGeom&, cpx*, const cpx*, int, int, const cpx*, int, bool, const cpx*, cudaStream_t);
+    bool pipelined;           // the column sweeps of this size run on the TMA pipeline
 };
 
 // any other even size: mixed-radix line transforms in shared memory with run-time N (generic_sweeps.cu)

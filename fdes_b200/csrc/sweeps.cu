@@ -35,7 +35,7 @@ std::vector<cpx> make_twiddles(int N) { return vt(N).make_twiddles(N); }
 int rows_per_block(int N) { return vt(N).rows_per_block; }
 int cols_per_block(int N) { return vt(N).cols_per_block; }
 int line_points(int N) { return vt(N).line_points; }
-bool sweeps_pipelined(int N) { const SweepVTable& t = vt(N); return t.pipelined && t.pipelined(); }
+bool sweeps_pipelined(int N) { return vt(N).pipelined; }
 
 void launch_density_rows(const SweepGeom& g, cpx* A, const int* rowptr, const int* rec_col, const float* rec_w,
                          int slice, int slice2, int nZ, int batch, size_t rec_stride, size_t rowptr_stride, cudaStream_t st,
@@ -65,11 +65,13 @@ void launch_propagate_cols(const SweepGeom& g, cpx* Psi, const cpx* Pq, int batc
 {
     vt(g.N).propagate_cols(g, Psi, Pq, batch, st);
 }
-bool launch_propagate_cols_from(const SweepGeom& g, cpx* out, const cpx* src, int src_img_stride, int src_images, const cpx* Pq,
+void launch_propagate_cols_from(const SweepGeom& g, cpx* out, const cpx* src, int src_img_stride, int src_images, const cpx* Pq,
                                 int batch, bool times_n, const cpx* lens, cudaStream_t st)
 {
     const SweepVTable& t = vt(g.N);
-    return t.propagate_cols_from && t.propagate_cols_from(g, out, src, src_img_stride, src_images, Pq, batch, times_n, lens, st);
+    if (!t.propagate_cols_from)
+        throw std::runtime_error("grid size " + std::to_string(g.N) + ": S6 from another image stack needs the pipelined column sweeps");
+    t.propagate_cols_from(g, out, src, src_img_stride, src_images, Pq, batch, times_n, lens, st);
 }
 void launch_rows_fft(const SweepGeom& g, const void* in, void* out, int dir, RowEpilogue epi, const RowOpts& o, int batch,
                      cudaStream_t st)
