@@ -73,6 +73,9 @@ def load_library() -> ctypes.CDLL:
     lib.fdes_b200_fft2d.argtypes = [c_f, ctypes.c_int, ctypes.c_int, ctypes.c_int]
     lib.fdes_b200_sort_records.argtypes = [ctypes.POINTER(ctypes.c_uint), c_i, c_f, ctypes.c_int, ctypes.c_int,
                                            c_i, ctypes.c_int]
+    lib.fdes_b200_sweep_test.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_int, c_i, ctypes.c_int, c_f, ctypes.c_int,
+                                         ctypes.POINTER(c_f), ctypes.POINTER(ctypes.c_longlong), ctypes.c_int,
+                                         ctypes.c_int]
     lib.FDES.restype = None
     lib.FDES.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_char_p, ctypes.c_char_p, ctypes.c_char_p, c_f,
                          ctypes.c_int, c_f]
@@ -320,6 +323,40 @@ def fft2d(a: np.ndarray, direction: int = -1, gpu_index: int = 0) -> np.ndarray:
     if lib.fdes_b200_fft2d(_fp(out.view(np.float32)), n, direction, gpu_index) != 0:
         raise FdesError(lib.fdes_b200_last_error().decode())
     return out
+
+
+# operations of fdes_b200_sweep_test (include/fdes_b200.h)
+SWEEP_GEOM, SWEEP_DENSITY, SWEEP_POTENTIAL, SWEEP_TRANSMIT, SWEEP_BANDLIMIT, SWEEP_MULTIPLY, SWEEP_PROPAGATE, \
+    SWEEP_PROPAGATE_FROM, SWEEP_COLS_FFT, SWEEP_ROWS_FFT_SUM = range(10)
+# ColOp and RowEpilogue values (fdes_b200/csrc/kernels.cuh)
+COL_PLAIN, COL_MUL_CPX_INV, COL_MUL_REAL_INV, COL_DP_ACCUM = range(4)
+ROW_ACCUM, ROW_INTENS_ACCUM = 1, 2
+
+
+def sweep_test(op: int, n: int, batch: int, bufs, iargs=(), fargs=(), gpu_index: int = 0) -> None:
+    """One sweep launcher run once on host arrays (fdes_b200_sweep_test).  `bufs` are C-contiguous
+    complex64 / float32 / int32 arrays, uploaded, and overwritten in place with what the device holds
+    after the sweep."""
+    lib = load_library()
+    for b in bufs:
+        assert b.flags.c_contiguous and b.dtype in (np.complex64, np.float32, np.int32), b.dtype
+    ia = np.ascontiguousarray(list(iargs) or [0], np.int32)
+    fa = np.ascontiguousarray(list(fargs) or [0.0], np.float32)
+    ptrs = (ctypes.POINTER(ctypes.c_float) * max(len(bufs), 1))(
+        *[b.ctypes.data_as(ctypes.POINTER(ctypes.c_float)) for b in bufs])
+    sizes = (ctypes.c_longlong * max(len(bufs), 1))(*[b.nbytes // 4 for b in bufs])
+    rc = lib.fdes_b200_sweep_test(op, n, batch, _ip(ia), len(iargs), _fp(fa), len(fargs), ptrs, sizes, len(bufs),
+                                  gpu_index)
+    if rc != 0:
+        raise FdesError(lib.fdes_b200_last_error().decode())
+
+
+def sweep_geom(n: int) -> dict:
+    """The geometry the sweeps of an n x n grid run with (host only): band columns [0, lo_end) and
+    [hi_start, n), points per thread of a line (0: generic sweeps), pipelined column sweeps."""
+    out = np.zeros(5, np.int32)
+    sweep_test(SWEEP_GEOM, n, 1, [out])
+    return dict(zip(["n", "lo_end", "hi_start", "line_points", "pipelined"], map(int, out)))
 
 
 def sort_records(keys: np.ndarray, cols: np.ndarray, w: np.ndarray, nkeys: int, gpu_index: int = 0):

@@ -14,6 +14,7 @@
 #include <algorithm>
 #include <string>
 #include <chrono>
+#include <climits>
 #include <thread>
 #include <exception>
 
@@ -445,6 +446,210 @@ int fdes_b200_sort_records(unsigned int* keys, int* cols, float* w, int n, int n
     ck(cudaMemcpy(rowptr, rp, ((size_t)nkeys + 1) * 4, cudaMemcpyDeviceToHost), "cudaMemcpy");
     cudaFree(sb.keys); cudaFree(sb.keys_tmp); cudaFree(sb.cols); cudaFree(sb.cols_tmp);
     cudaFree(sb.w); cudaFree(sb.w_tmp); cudaFree(sb.hist); cudaFree(rp);
+    return 0;
+    API_CATCH(-1)
+}
+
+}  // extern "C"
+
+namespace {
+
+// device allocations and the stream of one call, released on every path out of it
+struct DeviceAllocs {
+    std::vector<void*> p;
+    cudaStream_t st = nullptr;
+    ~DeviceAllocs()
+    {
+        if (st) { cudaStreamSynchronize(st); cudaStreamDestroy(st); }
+        for (void* q : p) cudaFree(q);
+    }
+    void* get(size_t bytes)
+    {
+        void* q = nullptr;
+        ck(cudaMalloc(&q, std::max<size_t>(bytes, 4)), "cudaMalloc");
+        p.push_back(q);
+        return q;
+    }
+};
+
+// the deposit records of S1 / S2 as the engine lays them out: per configuration nkeys + 1 row pointers,
+// then the row masks (launch_row_masks) where the size has them
+struct RecordRows {
+    int* dev = nullptr;
+    size_t stride = 0;
+    int mask_off = 0;
+};
+RecordRows upload_row_pointers(DeviceAllocs& da, const int* rp_host, int nconf, int nkeys, int N, int rec_stride,
+                               cudaStream_t st)
+{
+    for (int c = 0; c < nconf; c++) {
+        const int* rp = rp_host + (size_t)c * (nkeys + 1);
+        if (rp[0] < 0 || rp[nkeys] > rec_stride) throw std::runtime_error("sweep test: row pointers outside the records");
+        for (int k = 0; k < nkeys; k++)
+            if (rp[k + 1] < rp[k]) throw std::runtime_error("sweep test: row pointers must not decrease");
+    }
+    const int E = line_points(N);
+    RecordRows r;
+    r.stride = (size_t)nkeys + 1 + (E > 0 ? (size_t)(nkeys / N) * (N / E) : 0);
+    r.mask_off = E > 0 ? nkeys + 1 : 0;
+    r.dev = static_cast<int*>(da.get((size_t)nconf * r.stride * sizeof(int)));
+    for (int c = 0; c < nconf; c++)
+        ck(cudaMemcpyAsync(r.dev + (size_t)c * r.stride, rp_host + (size_t)c * (nkeys + 1), ((size_t)nkeys + 1) * sizeof(int),
+                           cudaMemcpyHostToDevice, st), "cudaMemcpyAsync");
+    if (E > 0) launch_row_masks(r.dev, r.stride, nkeys, N, E, nconf, st);
+    return r;
+}
+
+}  // namespace
+
+extern "C" {
+
+int fdes_b200_sweep_test(int op, int N, int batch, const int* iargs, int n_iargs, const float* fargs, int n_fargs,
+                         float** bufs, const long long* buf_elems, int nbufs, int gpu_index)
+{
+    API_TRY
+    auto ia = [&](int i) {
+        if (i >= n_iargs) throw std::runtime_error("sweep test: too few integer arguments");
+        return iargs[i];
+    };
+    auto fa = [&](int i) {
+        if (i >= n_fargs) throw std::runtime_error("sweep test: too few float arguments");
+        return fargs[i];
+    };
+    auto need = [&](int i, size_t words) {
+        if (i >= nbufs || !bufs[i] || buf_elems[i] < (long long)words)
+            throw std::runtime_error("sweep test: buffer " + std::to_string(i) + " needs " + std::to_string(words) + " words");
+    };
+    if (!fft_size_supported(N)) throw std::runtime_error("unsupported FFT size");
+    if (op == FDES_B200_SWEEP_GEOM) {
+        need(0, 5);
+        const SweepGeom g = make_sweep_geom(N, nullptr, 0);
+        int* o = reinterpret_cast<int*>(bufs[0]);
+        o[0] = g.N; o[1] = g.lo_end; o[2] = g.hi_start; o[3] = line_points(N); o[4] = sweeps_pipelined(N) ? 1 : 0;
+        return 0;
+    }
+    if (batch < 1) throw std::runtime_error("sweep test: batch must be >= 1");
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) throw std::runtime_error("no CUDA device");
+    ck(cudaSetDevice(gpu_index), "cudaSetDevice");
+    const size_t NN = (size_t)N * N, IMG = 2 * NN, Q = (size_t)(N / 2 + 1);
+    for (int i = 0; i < nbufs; i++)
+        if (buf_elems[i] < 0 || (buf_elems[i] > 0 && !bufs[i])) throw std::runtime_error("sweep test: bad buffer");
+
+    DeviceAllocs da;
+    // the sweeps run as in the engine: on a non-blocking stream, launched with programmatic serialisation; every
+    // copy of this call is queued on the same stream, so the row masks and the sweep see the uploaded data
+    ck(cudaStreamCreateWithFlags(&da.st, cudaStreamNonBlocking), "cudaStreamCreate");
+    const cudaStream_t st = da.st;
+    const std::vector<cpx> twh = make_twiddles(N);
+    cpx* tw = static_cast<cpx*>(da.get(twh.size() * sizeof(cpx)));
+    ck(cudaMemcpyAsync(tw, twh.data(), twh.size() * sizeof(cpx), cudaMemcpyHostToDevice, st), "cudaMemcpyAsync");
+    SweepGeom g = make_sweep_geom(N, tw, 0);
+    // row pointers of S1 / S2 (buffer rp_buf) go up in the engine's layout, not word for word
+    int rp_buf = -1, nconf = 0, nkeys = 0;
+    RecordRows rows;
+    if (op == FDES_B200_SWEEP_DENSITY || op == FDES_B200_SWEEP_POTENTIAL) {
+        const int slice = ia(0), slice2 = ia(1), nZ = ia(2), nslices = ia(3), cfg_stride = ia(4), cfg_off2 = ia(5);
+        nconf = ia(6);
+        const int rec_stride = op == FDES_B200_SWEEP_DENSITY ? ia(7) : INT_MAX;
+        if (nZ < 1 || nslices < 1 || slice < 0 || slice >= nslices || slice2 >= nslices || cfg_stride < 1 || cfg_off2 < 0)
+            throw std::runtime_error("sweep test: bad slice / species / configuration arguments");
+        if ((long long)(batch - 1) * cfg_stride + cfg_off2 >= nconf) throw std::runtime_error("sweep test: too few configurations");
+        if ((long long)nslices * nZ * N >= (1LL << 31) - 2) throw std::runtime_error("sweep test: too many row keys");
+        nkeys = nslices * nZ * N;
+        rp_buf = op == FDES_B200_SWEEP_DENSITY ? 1 : 3;
+        need(rp_buf, (size_t)nconf * (nkeys + 1));
+        if (op == FDES_B200_SWEEP_DENSITY) {
+            need(2, (size_t)nconf * rec_stride); need(3, (size_t)nconf * rec_stride);
+            const int* cols = reinterpret_cast<const int*>(bufs[2]);
+            for (size_t i = 0; i < (size_t)nconf * rec_stride; i++)
+                if (cols[i] < 0 || cols[i] >= N) throw std::runtime_error("sweep test: record column outside the grid");
+        }
+        rows = upload_row_pointers(da, reinterpret_cast<const int*>(bufs[rp_buf]), nconf, nkeys, N,
+                                   op == FDES_B200_SWEEP_DENSITY ? rec_stride : INT_MAX, st);
+        g.mask_off = rows.mask_off;
+    }
+    std::vector<float*> d(nbufs, nullptr);
+    for (int i = 0; i < nbufs; i++) {
+        if (i == rp_buf || buf_elems[i] == 0) continue;
+        d[i] = static_cast<float*>(da.get((size_t)buf_elems[i] * 4));
+        ck(cudaMemcpyAsync(d[i], bufs[i], (size_t)buf_elems[i] * 4, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync");
+    }
+    auto c = [&](int i) { return reinterpret_cast<cpx*>(d[i]); };
+
+    switch (op) {
+        case FDES_B200_SWEEP_DENSITY: {
+            const int nZ = ia(2);
+            need(0, (size_t)batch * nZ * IMG);
+            launch_density_rows(g, c(0), rows.dev, reinterpret_cast<const int*>(d[2]), d[3], ia(0), ia(1), nZ, batch,
+                                (size_t)ia(7), rows.stride, st, ia(4), ia(5));
+        } break;
+        case FDES_B200_SWEEP_POTENTIAL: {
+            const int nZ = ia(2);
+            need(0, (size_t)batch * IMG); need(1, (size_t)batch * nZ * IMG); need(2, (size_t)nZ * Q * Q);
+            launch_potential_cols(g, c(0), c(1), d[2], rows.dev, ia(0), ia(1), nZ, batch, rows.stride, st, ia(4), ia(5));
+        } break;
+        case FDES_B200_SWEEP_TRANSMIT: {
+            const int npair = ia(0);
+            if (npair < 1 || npair > 2) throw std::runtime_error("sweep test: npair must be 1 or 2");
+            need(0, (size_t)batch * IMG); need(1, 2 * (size_t)batch * IMG);
+            launch_transmit_rows(g, c(0), c(1), npair, fa(0), batch, st);
+        } break;
+        case FDES_B200_SWEEP_BANDLIMIT: {
+            const int npair = ia(0);
+            if (npair < 0 || npair > 2) throw std::runtime_error("sweep test: npair must be 0, 1 or 2");
+            need(0, (size_t)(npair ? 2 * batch : batch) * IMG);
+            launch_bandlimit_cols(g, c(0), batch, npair, st);
+        } break;
+        case FDES_B200_SWEEP_MULTIPLY: {
+            const int es = ia(0);
+            if (es < 0) throw std::runtime_error("sweep test: negative image stride");
+            need(0, (size_t)batch * IMG); need(1, ((size_t)(batch - 1) * es + 1) * IMG);
+            launch_multiply_rows(g, c(0), c(1), (size_t)es * NN, batch, ia(1) != 0, st);
+        } break;
+        case FDES_B200_SWEEP_PROPAGATE:
+            need(0, (size_t)batch * IMG); need(1, 2 * Q * Q);
+            launch_propagate_cols(g, c(0), c(1), batch, st);
+            break;
+        case FDES_B200_SWEEP_PROPAGATE_FROM: {
+            const int stride = ia(0), images = ia(1);
+            if (stride < 1 || (long long)(batch - 1) * stride >= images) throw std::runtime_error("sweep test: bad source stack");
+            need(0, (size_t)batch * IMG); need(1, (size_t)images * IMG); need(2, 2 * Q * Q);
+            const bool lens = nbufs > 3 && buf_elems[3] > 0;
+            if (lens) need(3, IMG);
+            launch_propagate_cols_from(g, c(0), c(1), stride, images, c(2), batch, ia(2) != 0, lens ? c(3) : nullptr, st);
+        } break;
+        case FDES_B200_SWEEP_COLS_FFT: {
+            const int colop = ia(0);
+            if (colop < COL_PLAIN || colop > COL_DP_ACCUM) throw std::runtime_error("sweep test: unknown column operation");
+            need(0, (size_t)batch * IMG);
+            need(1, (size_t)batch * (colop == COL_DP_ACCUM ? NN : IMG));
+            if (colop == COL_MUL_CPX_INV) need(2, IMG);
+            if (colop == COL_MUL_REAL_INV) need(2, NN);
+            launch_cols_fft(g, c(0), d[1], ia(1), (ColOp)colop, nbufs > 2 ? d[2] : nullptr, fa(0), batch, st);
+        } break;
+        case FDES_B200_SWEEP_ROWS_FFT_SUM: {
+            const int epi = ia(0);
+            if (epi != ROW_ACCUM && epi != ROW_INTENS_ACCUM) throw std::runtime_error("sweep test: ROW_ACCUM or ROW_INTENS_ACCUM");
+            need(0, (size_t)batch * IMG); need(1, epi == ROW_ACCUM ? IMG : NN);
+            RowOpts ro;
+            ro.scale = fa(0);
+            ro.band_only_in = ia(1) != 0;
+            launch_rows_fft_sum(g, c(0), d[1], +1, (RowEpilogue)epi, ro, batch, st);
+        } break;
+        default: throw std::runtime_error("sweep test: unknown op " + std::to_string(op));
+    }
+    ck(cudaStreamSynchronize(st), "sweep kernels");
+    for (int i = 0; i < nbufs; i++) {
+        if (i == rp_buf) {
+            for (int cf = 0; cf < nconf; cf++)
+                ck(cudaMemcpyAsync(bufs[i] + (size_t)cf * (nkeys + 1), rows.dev + (size_t)cf * rows.stride,
+                                   ((size_t)nkeys + 1) * sizeof(int), cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync");
+        } else if (buf_elems[i] > 0) {
+            ck(cudaMemcpyAsync(bufs[i], d[i], (size_t)buf_elems[i] * 4, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync");
+        }
+    }
+    ck(cudaStreamSynchronize(st), "downloads");
     return 0;
     API_CATCH(-1)
 }

@@ -321,24 +321,13 @@ void Engine::setup_tables()
     // pass twiddle tables (double precision on the host)
     CK(cudaMemcpyAsync(tw_, tw_host_.data(), tw_host_.size() * sizeof(cpx), cudaMemcpyHostToDevice, st_));
 
-    // 2/3 band limit: largest |i1| kept on the axis by zeroHighFreq's float test
-    int kb = 0;
-    const float mind = (float)N_;
-    while (kb + 1 <= N_ / 2 && !(((float)((kb + 1) * (kb + 1)) * 9.f / (mind * mind)) > 1.f)) kb++;
-    g_.N = N_;
-    g_.tw = tw_;
-    g_.mask_off = mask_E_ > 0 ? nkeys_ + 1 : 0;
+    // band columns of the 2/3 limit; the row masks follow the nkeys + 1 row pointers of a configuration
+    g_ = make_sweep_geom(N_, tw_, mask_E_ > 0 ? nkeys_ + 1 : 0);
     {
         const char* e = getenv("FDES_B200_NO_FIRST_SLICE_SHORTCUT");     // A/B switch
         plane_first_slice_ = p_.mode != 2 && !p_.doBeamTilt && sweeps_pipelined(N_) && !(e && e[0] == '1');
         fuse_ctf_ = p_.mode == 0 && sweeps_pipelined(N_) && !(e && e[0] == '1');
     }
-    g_.lo_end = ((kb + 1 + 31) / 32) * 32;
-    g_.hi_start = ((N_ - kb) / 32) * 32;
-    if (g_.lo_end >= g_.hi_start) { g_.lo_end = N_; g_.hi_start = N_; }
-    // sizes without a register-resident instantiation run on the generic sweeps, which transform
-    // every column (the band limit is applied by the mask alone)
-    if (!fft_size_is_fast(N_)) { g_.lo_end = N_; g_.hi_start = N_; }
 
     launch_propagator_table(Pq_, N_, p_.d1, p_.d2, p_.d3, p_.lambda, p_.cst_pi, st_);
     const size_t Q = (size_t)(N_ / 2 + 1);

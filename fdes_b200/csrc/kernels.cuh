@@ -22,6 +22,10 @@ struct SweepGeom {
 };
 // host copy of the twiddle tables a SweepGeom of size N must point to (on the device)
 std::vector<cpx> make_twiddles(int N);
+// the geometry every sweep of size N expects: band columns of the 2/3 limit where the register-resident
+// sweeps run (the compiled bounds Band<N> of sweep_kernels.cuh check against these), every column
+// (lo_end = hi_start = N) on the generic sweeps; throws for an unsupported N
+SweepGeom make_sweep_geom(int N, const cpx* tw, int mask_off);
 
 bool fft_size_supported(int N);
 bool fft_size_is_fast(int N);   // register-resident kernels (else the generic run-time-N sweeps)

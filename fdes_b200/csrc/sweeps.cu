@@ -32,6 +32,21 @@ static const SweepVTable& vt(int N)
 bool fft_size_supported(int N) { return find_vtable(N) != nullptr; }
 bool fft_size_is_fast(int N) { return find_fast_vtable(N) != nullptr; }
 std::vector<cpx> make_twiddles(int N) { return vt(N).make_twiddles(N); }
+SweepGeom make_sweep_geom(int N, const cpx* tw, int mask_off)
+{
+    vt(N);
+    SweepGeom g{N, N, N, tw, mask_off};
+    // the generic sweeps transform every column (the band limit is applied by the mask alone)
+    if (!fft_size_is_fast(N)) return g;
+    // 2/3 band limit: largest |i1| kept on the axis by zeroHighFreq's float test, bounds rounded outwards
+    // to multiples of 32; no column skipped when the two ranges meet
+    int kb = 0;
+    const float mind = (float)N;
+    while (kb + 1 <= N / 2 && !(((float)((kb + 1) * (kb + 1)) * 9.f / (mind * mind)) > 1.f)) kb++;
+    const int lo_end = ((kb + 1 + 31) / 32) * 32, hi_start = ((N - kb) / 32) * 32;
+    if (lo_end < hi_start) { g.lo_end = lo_end; g.hi_start = hi_start; }
+    return g;
+}
 int rows_per_block(int N) { return vt(N).rows_per_block; }
 int cols_per_block(int N) { return vt(N).cols_per_block; }
 int line_points(int N) { return vt(N).line_points; }

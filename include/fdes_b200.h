@@ -175,6 +175,41 @@ int fdes_b200_fft2d(float* data_host, int N, int dir, int gpu_index);
  * keys [n] (values < nkeys are valid), cols [n], w [n] sorted in place; rowptr [nkeys+1]. */
 int fdes_b200_sort_records(unsigned int* keys, int* cols, float* w, int n, int nkeys, int* rowptr,
                            int gpu_index);
+/* One sweep of the slice loop, launched once on host arrays (test hook for per-sweep models).
+ * bufs[i] holds buf_elems[i] 32-bit words (float, int where noted; a complex image is N*N interleaved
+ * float pairs).  Every buffer is uploaded, the sweep runs on the N x N grid with the geometry the
+ * engine uses (band columns, row masks of the deposit records), and every buffer is downloaded again,
+ * so that what a sweep must not write still holds what the caller put there.  -1 on failure (also
+ * when a buffer is too small for the arguments, or the size has no such sweep).  `batch` images:
+ *   op                        iargs                                         fargs   bufs
+ *   FDES_B200_SWEEP_GEOM      -                                             -       int[5] out: N lo_end hi_start
+ *                                                                                   line_points pipelined (no device)
+ *   FDES_B200_SWEEP_DENSITY   slice slice2 nZ nslices cfg_stride cfg_off2   -       A [batch*nZ] out, rowptr (int,
+ *     (S1)                    nconf rec_stride                                      [nconf][nslices*nZ*N + 1]),
+ *                                                                                   col (int), w [nconf][rec_stride]
+ *   FDES_B200_SWEEP_POTENTIAL slice slice2 nZ nslices cfg_stride cfg_off2   -       B [batch] out, A [batch*nZ],
+ *     (S2)                    nconf                                                 Gq [nZ][(N/2+1)^2], rowptr (int)
+ *   FDES_B200_SWEEP_TRANSMIT  npair                                         imPot   W [batch], D [2*batch] out
+ *   FDES_B200_SWEEP_BANDLIMIT npair                                         -       W [npair ? 2*batch : batch] in/out
+ *   FDES_B200_SWEEP_MULTIPLY  e_stride (images) psi_full                    -       Psi [batch] in/out, E
+ *   FDES_B200_SWEEP_PROPAGATE -                                             -       Psi [batch] in/out, Pq [(N/2+1)^2]
+ *   FDES_B200_SWEEP_PROPAGATE_FROM src_img_stride src_images times_n        -       out [batch], src [src_images],
+ *                                                                                   Pq, lens [N*N] or 0 words (none)
+ *   FDES_B200_SWEEP_COLS_FFT  ColOp dir                                     scale   in [batch], out [batch]
+ *                                                                                   (float for the DP), table
+ *   FDES_B200_SWEEP_ROWS_FFT_SUM RowEpilogue band_only_in                   scale   in [batch], out (inverse) */
+#define FDES_B200_SWEEP_GEOM 0
+#define FDES_B200_SWEEP_DENSITY 1
+#define FDES_B200_SWEEP_POTENTIAL 2
+#define FDES_B200_SWEEP_TRANSMIT 3
+#define FDES_B200_SWEEP_BANDLIMIT 4
+#define FDES_B200_SWEEP_MULTIPLY 5
+#define FDES_B200_SWEEP_PROPAGATE 6
+#define FDES_B200_SWEEP_PROPAGATE_FROM 7
+#define FDES_B200_SWEEP_COLS_FFT 8
+#define FDES_B200_SWEEP_ROWS_FFT_SUM 9
+int fdes_b200_sweep_test(int op, int N, int batch, const int* iargs, int n_iargs, const float* fargs, int n_fargs,
+                         float** bufs, const long long* buf_elems, int nbufs, int gpu_index);
 
 #ifdef __cplusplus
 }

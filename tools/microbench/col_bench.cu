@@ -62,9 +62,7 @@ void run_dbg(int batch, int reps)
     auto twh = make_twiddles_n<N>();
     CK(cudaMalloc(&tw, twh.size() * sizeof(cpx)));
     CK(cudaMemcpy(tw, twh.data(), twh.size() * sizeof(cpx), cudaMemcpyHostToDevice));
-    int kb = 0; const float mind = (float)N;
-    while (kb + 1 <= N / 2 && !(((float)((kb + 1) * (kb + 1)) * 9.f / (mind * mind)) > 1.f)) kb++;
-    SweepGeom g{N, ((kb + 1 + 31) / 32) * 32, ((N - kb) / 32) * 32, tw};
+    SweepGeom g{N, Band<N>::lo_end, Band<N>::hi_start, tw};
     using Pc = PipeCfg<N>;
     CK(cudaFuncSetAttribute(k_dbg<N, DBG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Pc::SMEM));
     const int bc = band_cols(g), tiles_x = bc / Pc::CW, ntiles = tiles_x * batch;
@@ -103,10 +101,8 @@ void run(int batch, int reps)
     CK(cudaMemcpy(P, ph.data(), Q * Q * sizeof(cpx), cudaMemcpyHostToDevice));
     CK(cudaMemcpy(d0, h.data(), total * sizeof(cpx), cudaMemcpyHostToDevice));
     CK(cudaMemcpy(d1, h.data(), total * sizeof(cpx), cudaMemcpyHostToDevice));
-    // 2/3 band limit bounds as in Engine::setup_tables
-    int kb = 0; const float mind = (float)N;
-    while (kb + 1 <= N / 2 && !(((float)((kb + 1) * (kb + 1)) * 9.f / (mind * mind)) > 1.f)) kb++;
-    SweepGeom g{N, ((kb + 1 + 31) / 32) * 32, ((N - kb) / 32) * 32, tw};
+    // 2/3 band limit bounds as in make_sweep_geom (sweeps.cu)
+    SweepGeom g{N, Band<N>::lo_end, Band<N>::hi_start, tw};
     using C = ColCfg<N>;
     using Pc = PipeCfg<N>;
     CK(cudaFuncSetAttribute(k_propagate_cols<N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM));
