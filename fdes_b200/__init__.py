@@ -327,10 +327,10 @@ def fft2d(a: np.ndarray, direction: int = -1, gpu_index: int = 0) -> np.ndarray:
 
 # operations of fdes_b200_sweep_test (include/fdes_b200.h)
 SWEEP_GEOM, SWEEP_DENSITY, SWEEP_POTENTIAL, SWEEP_TRANSMIT, SWEEP_BANDLIMIT, SWEEP_MULTIPLY, SWEEP_PROPAGATE, \
-    SWEEP_PROPAGATE_FROM, SWEEP_COLS_FFT, SWEEP_ROWS_FFT_SUM = range(10)
+    SWEEP_PROPAGATE_FROM, SWEEP_COLS_FFT, SWEEP_ROWS_FFT_SUM, SWEEP_ROWS_FFT, SWEEP_PROBE, SWEEP_DETECTOR = range(13)
 # ColOp and RowEpilogue values (fdes_b200/csrc/kernels.cuh)
 COL_PLAIN, COL_MUL_CPX_INV, COL_MUL_REAL_INV, COL_DP_ACCUM = range(4)
-ROW_ACCUM, ROW_INTENS_ACCUM = 1, 2
+ROW_STORE, ROW_ACCUM, ROW_INTENS_ACCUM, ROW_STORE_SHIFT, ROW_CROP_REAL = range(5)
 
 
 def sweep_test(op: int, n: int, batch: int, bufs, iargs=(), fargs=(), gpu_index: int = 0) -> None:

@@ -621,12 +621,15 @@ int fdes_b200_sweep_test(int op, int N, int batch, const int* iargs, int n_iargs
         } break;
         case FDES_B200_SWEEP_COLS_FFT: {
             const int colop = ia(0);
+            const bool in_place = n_iargs > 2 && ia(2) != 0;
             if (colop < COL_PLAIN || colop > COL_DP_ACCUM) throw std::runtime_error("sweep test: unknown column operation");
+            if (in_place && colop != COL_PLAIN && colop != COL_MUL_REAL_INV)
+                throw std::runtime_error("sweep test: in place only with COL_PLAIN or COL_MUL_REAL_INV");
             need(0, (size_t)batch * IMG);
-            need(1, (size_t)batch * (colop == COL_DP_ACCUM ? NN : IMG));
+            if (!in_place) need(1, (size_t)batch * (colop == COL_DP_ACCUM ? NN : IMG));
             if (colop == COL_MUL_CPX_INV) need(2, IMG);
             if (colop == COL_MUL_REAL_INV) need(2, NN);
-            launch_cols_fft(g, c(0), d[1], ia(1), (ColOp)colop, nbufs > 2 ? d[2] : nullptr, fa(0), batch, st);
+            launch_cols_fft(g, c(0), in_place ? d[0] : d[1], ia(1), (ColOp)colop, nbufs > 2 ? d[2] : nullptr, fa(0), batch, st);
         } break;
         case FDES_B200_SWEEP_ROWS_FFT_SUM: {
             const int epi = ia(0);
@@ -636,6 +639,43 @@ int fdes_b200_sweep_test(int op, int N, int batch, const int* iargs, int n_iargs
             ro.scale = fa(0);
             ro.band_only_in = ia(1) != 0;
             launch_rows_fft_sum(g, c(0), d[1], +1, (RowEpilogue)epi, ro, batch, st);
+        } break;
+        case FDES_B200_SWEEP_ROWS_FFT: {
+            const int dir = ia(0), epi = ia(1);
+            RowOpts ro;
+            ro.scale = fa(0);
+            ro.in_is_real = ia(2) != 0;
+            ro.band_only_in = ia(3) != 0;
+            ro.band_only_out = ia(4) != 0;
+            ro.dn1 = ia(5); ro.dn2 = ia(6); ro.n1 = ia(7); ro.n2 = ia(8);
+            const bool in_place = ia(9) != 0;
+            if (dir != -1 && dir != 1) throw std::runtime_error("sweep test: dir must be -1 or +1");
+            if (epi < ROW_STORE || epi > ROW_CROP_REAL) throw std::runtime_error("sweep test: unknown row epilogue");
+            if (ro.band_only_out && epi != ROW_STORE) throw std::runtime_error("sweep test: band_only_out only with ROW_STORE");
+            if (in_place && (epi != ROW_STORE || ro.in_is_real))
+                throw std::runtime_error("sweep test: in place only with ROW_STORE and complex input");
+            if (epi == ROW_CROP_REAL && (ro.n1 < 1 || ro.n2 < 1 || ro.dn1 < 0 || ro.dn2 < 0 || ro.dn1 > N - ro.n1 || ro.dn2 > N - ro.n2))
+                throw std::runtime_error("sweep test: crop window outside the grid");
+            need(0, (size_t)batch * (ro.in_is_real ? NN : IMG));
+            if (!in_place)
+                need(1, (size_t)batch * (epi == ROW_INTENS_ACCUM ? NN : epi == ROW_CROP_REAL ? (size_t)ro.n1 * ro.n2 : IMG));
+            launch_rows_fft(g, d[0], in_place ? d[0] : d[1], dir, (RowEpilogue)epi, ro, batch, st);
+        } break;
+        case FDES_B200_SWEEP_PROBE:
+            need(0, (size_t)batch * IMG); need(1, IMG); need(2, 2 * (size_t)batch);
+            launch_probe_cols(g, c(0), c(1), d[2], batch, st);
+            break;
+        case FDES_B200_SWEEP_DETECTOR: {
+            DetectorRings rings{};
+            rings.n = ia(0);
+            if (rings.n < 1 || rings.n > MAX_DETECTORS) throw std::runtime_error("sweep test: 1.." + std::to_string(MAX_DETECTORS) + " detectors");
+            for (int r = 0; r < rings.n; r++) { rings.in2[r] = fa(3 + r); rings.out2[r] = fa(3 + rings.n + r); }
+            need(0, (size_t)batch * IMG); need(1, (size_t)batch * rings.n);
+            // a tile the detector sweep leaves unwritten reaches `out` as NaN
+            const size_t np = (size_t)batch * detector_tiles(g) * MAX_DETECTORS;
+            float* partial = static_cast<float*>(da.get(np * sizeof(float)));
+            launch_fill_f32(partial, np, std::nanf(""), st);
+            launch_detector_cols(g, c(0), partial, d[1], rings, fa(0), fa(1), fa(2), batch, st);
         } break;
         default: throw std::runtime_error("sweep test: unknown op " + std::to_string(op));
     }

@@ -422,7 +422,8 @@ __global__ void __launch_bounds__(GT) g_probe_cols(cpx* Psi, const cpx* PSI0, co
     cpx *x = gsm, *y = gsm + L * N;
     const float sx = shifts[2 * blockIdx.y], sy = shifts[2 * blockIdx.y + 1], inv = 1.f / (float)N;
     g_foreach<true>(N, L, [&](int i, int l) {
-        float t = (float)iwg(kx0 + l, N) * sx + (float)iwg(i, N) * sy;      // phase in turns
+        const float a = (float)iwg(kx0 + l, N), b = (float)iwg(i, N);
+        float t = fmaf(a, sx, -rintf(a * sx)) + fmaf(b, sy, -rintf(b * sy));   // phase in turns (see k_probe_cols)
         t -= rintf(t);
         float sn, cs;
         sincosf(-6.283185307179586f * t, &sn, &cs);

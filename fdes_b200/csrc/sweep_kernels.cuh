@@ -1421,13 +1421,15 @@ k_probe_cols(cpx* __restrict__ Psi, const cpx* __restrict__ PSI0, const float* _
     cpx x[E];
     ctx.load(x, PSI0 + kx0, KeepAll());
     const int i1 = kx > N / 2 ? kx - N : kx;
-    const float ax = (float)i1 * sx;
+    // phase in turns: the fractional part of each product is taken exactly (one rounding) before they are added,
+    // so the error stays near 1e-7 turns at any N instead of growing with |i sx|
+    const float ax = fmaf((float)i1, sx, -rintf((float)i1 * sx));
     const float inv = 1.f / (float)N;
 #pragma unroll
     for (int m = 0; m < E; m++) {
     const int ky = theta + m * C::T;
     const int i2 = ky > N / 2 ? ky - N : ky;
-    float t = ax + (float)i2 * sy;      // phase in turns
+    float t = ax + fmaf((float)i2, sy, -rintf((float)i2 * sy));
     t -= rintf(t);
     float sn, cs;
     sincos_compact(-6.283185307179586f * t, sn, cs);

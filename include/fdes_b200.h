@@ -195,9 +195,24 @@ int fdes_b200_sort_records(unsigned int* keys, int* cols, float* w, int n, int n
  *   FDES_B200_SWEEP_PROPAGATE -                                             -       Psi [batch] in/out, Pq [(N/2+1)^2]
  *   FDES_B200_SWEEP_PROPAGATE_FROM src_img_stride src_images times_n        -       out [batch], src [src_images],
  *                                                                                   Pq, lens [N*N] or 0 words (none)
- *   FDES_B200_SWEEP_COLS_FFT  ColOp dir                                     scale   in [batch], out [batch]
- *                                                                                   (float for the DP), table
- *   FDES_B200_SWEEP_ROWS_FFT_SUM RowEpilogue band_only_in                   scale   in [batch], out (inverse) */
+ *   FDES_B200_SWEEP_COLS_FFT  ColOp dir [in_place]                          scale   in [batch], out [batch]
+ *                                                                                   (float for the DP), table;
+ *                                                                                   in_place (COL_PLAIN,
+ *                                                                                   COL_MUL_REAL_INV): in is out
+ *   FDES_B200_SWEEP_ROWS_FFT_SUM RowEpilogue band_only_in                   scale   in [batch], out (inverse)
+ *   FDES_B200_SWEEP_ROWS_FFT  dir RowEpilogue in_is_real band_only_in       scale   in [batch] (float [batch][N][N]
+ *                             band_only_out dn1 dn2 n1 n2 in_place                  when in_is_real), out: [batch]
+ *                                                                                   (STORE, ACCUM, STORE_SHIFT),
+ *                                                                                   float [batch][N][N] (INTENS_ACCUM),
+ *                                                                                   float [batch][n2][n1] (CROP_REAL);
+ *                                                                                   in_place (ROW_STORE, complex
+ *                                                                                   input): in is out
+ *   FDES_B200_SWEEP_PROBE     -                                             -       Psi [batch] out, PSI0 [1],
+ *                                                                                   shifts [batch][2]
+ *   FDES_B200_SWEEP_DETECTOR  ndet (1..8)                                   d1 d2   Psi [batch], out [batch][ndet]
+ *                                                                           weight  (accumulated into); partial
+ *                                                                           in2[ndet] sums start as NaN
+ *                                                                           out2[ndet] */
 #define FDES_B200_SWEEP_GEOM 0
 #define FDES_B200_SWEEP_DENSITY 1
 #define FDES_B200_SWEEP_POTENTIAL 2
@@ -208,6 +223,9 @@ int fdes_b200_sort_records(unsigned int* keys, int* cols, float* w, int n, int n
 #define FDES_B200_SWEEP_PROPAGATE_FROM 7
 #define FDES_B200_SWEEP_COLS_FFT 8
 #define FDES_B200_SWEEP_ROWS_FFT_SUM 9
+#define FDES_B200_SWEEP_ROWS_FFT 10
+#define FDES_B200_SWEEP_PROBE 11
+#define FDES_B200_SWEEP_DETECTOR 12
 int fdes_b200_sweep_test(int op, int N, int batch, const int* iargs, int n_iargs, const float* fargs, int n_fargs,
                          float** bufs, const long long* buf_elems, int nbufs, int gpu_index);
 

@@ -1,4 +1,5 @@
-"""float64 models of the per-slice sweeps of fdes_b200 (S1..S6 and the sweeps of the image formation).
+"""float64 models of the per-slice sweeps of fdes_b200 (S1..S6 and the sweeps of the image formation
+and of the STEM scan).
 
 Written from the sweep contracts (DESIGN.md section 2, the launcher comments of
 fdes_b200/csrc/kernels.cuh), not from the kernels:
@@ -249,3 +250,88 @@ def plane_wave_rowspace(n, batch=1):
     P = np.zeros((batch, n, n), np.complex128)
     P[:, :, 0] = 1
     return P
+
+
+# ---------------------------------------------------------------------------------------------------
+# image formation and STEM: generic row / column sweeps, shifted probes, annular detectors
+# ---------------------------------------------------------------------------------------------------
+ROW_STORE, ROW_ACCUM, ROW_INTENS_ACCUM, ROW_STORE_SHIFT, ROW_CROP_REAL = range(5)
+
+
+def signed_index(n: int) -> np.ndarray:
+    """iw(k): the frequency of index k, k - N for k > N/2."""
+    k = np.arange(n)
+    return np.where(k > n // 2, k - n, k)
+
+
+def rows_fft(x, dir, epi, scale, out=None, band_in=None, band_out=None, crop=None):
+    """launch_rows_fft: v = scale * FFT_row(x) (dir -1) or scale * IFFT_row(x) (dir +1) per image, then
+    ROW_STORE v (0 outside band_out when given), ROW_ACCUM out + v, ROW_INTENS_ACCUM out + scale * |FFT(x)|^2,
+    ROW_STORE_SHIFT v at [(y + N/2) % N][(x + N/2) % N] (numpy's fftshift for either parity), ROW_CROP_REAL
+    Re v in the window crop = (dn1, dn2, n1, n2): [dn2:dn2 + n2, dn1:dn1 + n1].  x may be real (in_is_real);
+    band_in: only these columns of x are read (the others as zero)."""
+    x = np.asarray(x)
+    if band_in is not None:
+        x = np.where(band_in, x, 0)
+    f = fft_rows(x) if dir < 0 else ifft_rows(x)
+    v = scale * f
+    n = x.shape[-1]
+    if epi == ROW_STORE:
+        return v if band_out is None else np.where(band_out, v, 0)
+    if epi == ROW_ACCUM:
+        return np.asarray(out, np.complex128) + v
+    if epi == ROW_INTENS_ACCUM:
+        return np.asarray(out, np.float64) + scale * np.abs(f) ** 2
+    if epi == ROW_STORE_SHIFT:
+        return np.roll(v, (n // 2, n // 2), axis=(-2, -1))
+    dn1, dn2, n1, n2 = crop
+    return v.real[..., dn2:dn2 + n2, dn1:dn1 + n1]
+
+
+def cols_plain(x, dir, scale):
+    """COL_PLAIN: out = scale * FFT_col(x) (dir -1) or scale * IFFT_col(x) (dir +1), every column."""
+    return scale * (fft_cols(x) if dir < 0 else ifft_cols(x))
+
+
+def cols_mul_real_inv(x, table, scale):
+    """COL_MUL_REAL_INV: out = scale * IFFT_col(FFT_col(x) * tab[ky][kx]), every column."""
+    n = np.asarray(x).shape[-1]
+    return scale * ifft_cols(fft_cols(x) * np.asarray(table, np.float64).reshape(n, n))
+
+
+def probe_phase(n, sx, sy):
+    """exp(-2 pi i (iw(kx) sx + iw(ky) sy)) [ky][kx] in float64 for the float32 shift (sx, sy)."""
+    w = signed_index(n).astype(np.float64)
+    return np.exp(-2j * np.pi * (w[None, :] * float(sx) + w[:, None] * float(sy)))
+
+
+def probe_cols(PSI0, shifts, band):
+    """launch_probe_cols: Psi_b = (1/N) IFFT_col[PSI0 * exp(-2 pi i (iw(kx) sx_b + iw(ky) sy_b))] on the band
+    columns (PSI0 [ky][kx] read there only), shifts [batch][2] = (sx, sy) in units of the grid period."""
+    P = np.where(band, np.asarray(PSI0).reshape(np.asarray(PSI0).shape[-2:]), 0)
+    n = P.shape[-1]
+    return np.stack([ifft_cols(P * probe_phase(n, sx, sy)) / n for sx, sy in np.asarray(shifts).reshape(-1, 2)])
+
+
+def inv_length(n, d):
+    """fl32(1 / fl32(N d)): the reciprocal box length the detector launcher computes in float32."""
+    return np.float32(1) / (np.float32(n) * np.float32(d))
+
+
+def detector_ksq(n, inv_l1, inv_l2):
+    """|k|^2 [ky][kx] = (iw(kx) inv_l1)^2 + (iw(ky) inv_l2)^2 in float64."""
+    w = signed_index(n).astype(np.float64)
+    return (w[None, :] * float(inv_l1)) ** 2 + (w[:, None] * float(inv_l2)) ** 2
+
+
+def detector_cols(Psi, band, in2, out2, inv_l1, inv_l2, weight, out0):
+    """launch_detector_cols: out[b][d] = out0[b][d] + weight * sum |FFT_col(Psi_b)|^2 over the band columns and
+    every ky with in2[d] <= |k|^2 < out2[d]."""
+    Psi = np.asarray(Psi)
+    ksq = detector_ksq(Psi.shape[-1], inv_l1, inv_l2)
+    inten = np.abs(fft_cols(np.where(band, Psi, 0))) ** 2
+    res = np.array(out0, np.float64)
+    for d, (a, b) in enumerate(zip(in2, out2)):
+        m = band[None, :] & (ksq >= float(a)) & (ksq < float(b))
+        res[:, d] += float(weight) * (inten * m).sum(axis=(-2, -1))
+    return res

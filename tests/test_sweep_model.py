@@ -1,6 +1,6 @@
-"""CPU checks of oracle/sweep_model.py, the float64 models the per-sweep GPU tests (test_sweeps_fp64_gpu.py)
-compare the kernels with: composed S1..S6 they must reproduce the reference's phase grating and forward
-propagation (fdes_oracle, float32) to float32 rounding -- which pins the models' conventions (domains,
+"""CPU checks of oracle/sweep_model.py, the float64 models the per-sweep GPU tests (test_sweeps_fp64_gpu.py,
+test_formation_fp64_gpu.py) compare the kernels with: composed S1..S6 they must reproduce the reference's phase
+grating and forward propagation (fdes_oracle, float32) to float32 rounding -- which pins the models' conventions (domains,
 normalisations, table layouts, pair packing) to the reference's semantics."""
 import numpy as np
 import pytest
@@ -108,3 +108,38 @@ def test_library_geometry_matches_model(fb, n):
     # every column the 2/3 limit keeps anywhere is a band column
     assert band[sm.keep_mask(n).any(axis=0)].all()
     assert g["pipelined"] == (n in (512, 1024, 2048, 4096))
+
+
+@pytest.mark.parametrize("n", [64, 143])
+def test_probe_model_whole_pixel_shift_is_roll(n):
+    """A probe shifted by whole pixels (sx = p / N) is the unshifted probe rolled by p pixels: psi = IFFT_row(Psi)
+    in the (kx, y) convention Psi = FFT_row(psi) / N, and the shift moves the probe towards +x, +y."""
+    rng = np.random.default_rng(11)
+    psi0 = rng.standard_normal((n, n)) + 1j * rng.standard_normal((n, n))
+    PSI0 = sm.fft_cols(sm.fft_rows(psi0) / n)
+    band = np.ones(n, bool)
+    p1, p2 = 5, -(n // 3)
+    Psi = sm.probe_cols(PSI0, [[0.0, 0.0], [p1 / n, p2 / n]], band)
+    np.testing.assert_allclose(sm.ifft_rows(Psi[0]), psi0, atol=1e-12)
+    np.testing.assert_allclose(sm.ifft_rows(Psi[1]), np.roll(psi0, (p2, p1), axis=(0, 1)), atol=1e-12)
+
+
+def test_detector_model_everything_is_parseval():
+    """A ring covering every |k| sums N * sum |Psi|^2 over the band columns (Parseval along the columns)."""
+    rng = np.random.default_rng(12)
+    n = 128
+    Psi = rng.standard_normal((2, n, n)) + 1j * rng.standard_normal((2, n, n))
+    band = sm.band_columns(n, 32, 96)
+    out0 = np.array([[1.0, 2.0], [3.0, 4.0]])
+    res = sm.detector_cols(Psi, band, [0.0, 0.0], [np.inf, 0.0], 1.0, 1.0, 0.5, out0)
+    parseval = n * (np.abs(Psi[..., band]) ** 2).sum(axis=(-2, -1))
+    np.testing.assert_allclose(res[:, 0], out0[:, 0] + 0.5 * parseval, rtol=1e-12)
+    np.testing.assert_array_equal(res[:, 1], out0[:, 1])          # in2 == out2: empty
+
+
+@pytest.mark.parametrize("n", [143, 144])
+def test_rows_model_store_shift_is_fftshift(n):
+    rng = np.random.default_rng(13)
+    x = rng.standard_normal((2, n, n)) + 1j * rng.standard_normal((2, n, n))
+    got = sm.rows_fft(x, -1, sm.ROW_STORE_SHIFT, 0.5)
+    np.testing.assert_allclose(got, 0.5 * np.fft.fftshift(np.fft.fft(x, axis=-1), axes=(-2, -1)), rtol=1e-12, atol=1e-9)
