@@ -24,6 +24,7 @@
 #include "fft_core.cuh"
 #include <cuda.h>
 #include <cstdint>
+#include <type_traits>
 
 namespace fdes {
 
@@ -103,6 +104,8 @@ struct PipeCfg {
     static constexpr int TW_TABLE = twiddle_table_elems<N, E>();
     static constexpr bool TW_SHARED = 2 * TILE_BYTES + ((X_BYTES + 15) & ~15) + TW_TABLE * 8 + 64 <= 227 * 1024;
     static constexpr int TW_ELEMS = TW_SHARED ? TW_TABLE : 0;
+    // 1024-point columns (32 x 32): the second-pass twiddles of a thread are held in registers (TwRegs)
+    static constexpr bool TW_REGS = N == 1024;
     static constexpr int OFF_L = 0, OFF_S = TILE_BYTES, OFF_X = 2 * TILE_BYTES, OFF_TW = OFF_X + ((X_BYTES + 15) & ~15),
                          OFF_BAR = OFF_TW + TW_ELEMS * 8;
     static constexpr size_t SMEM = OFF_BAR + 64;
@@ -131,12 +134,14 @@ struct PipeSync {
 //   release(x, ...)       wait until the previous store has drained S, write own points, thread 0
 //                         starts the store
 // finish() before the kernel exits.
-// DBG (microbenchmarks only): bit 0 = no tile loads, bit 1 = no tile stores.
+// DBG (microbenchmarks only): bit 0 = no tile loads, bit 1 = no tile stores, bit 2 = pass twiddles from
+// shared memory only (no TwRegs).
 template <int N, int DBG = 0>
 struct ColPipe {
     using C = PipeCfg<N>;
     static constexpr bool SPLIT = C::SPLIT;
     static constexpr int E = C::E, T = C::T;
+    static constexpr bool TW_REGS = C::TW_REGS && !(DBG & 4);
     unsigned char* base;       // 1024-byte aligned shared memory
     uint64_t *full, *sfree;
     const cpx* tw_global_;
@@ -144,6 +149,8 @@ struct ColPipe {
     uint32_t tile_off;         // byte offset of this thread's (row theta, column line) inside a tile buffer
     uint32_t it = 0;           // tiles stored so far by this CTA
     uint32_t nload = 0;        // tiles acquired so far (several loads may feed one stored tile)
+    struct NoTwRegs {};
+    std::conditional_t<TW_REGS, TwRegs, NoTwRegs> twr;
 
     // tw: the pass twiddle tables of the line transform (global); a copy is placed in shared memory
     __device__ __forceinline__ ColPipe(unsigned char* smem_raw, const cpx* __restrict__ tw_global)
@@ -169,11 +176,13 @@ struct ColPipe {
         tw_global_ = tw_global;
         cpx* tws = reinterpret_cast<cpx*>(base + C::OFF_TW);
         for (int i = threadIdx.x; i < C::TW_ELEMS; i += C::THREADS) tws[i] = tw_global[i];
+        if constexpr (TW_REGS) twr.load(tw_global, theta);
         __syncthreads();
     }
     __device__ __forceinline__ auto tw() const
     {
-        if constexpr (C::TW_SHARED) return TwShared{smem_u32(base + C::OFF_TW)};
+        if constexpr (TW_REGS) return twr;
+        else if constexpr (C::TW_SHARED) return TwShared{smem_u32(base + C::OFF_TW)};
         else return TwGlobal{tw_global_};
     }
     __device__ __forceinline__ cpx* sm() const { return reinterpret_cast<cpx*>(base + C::OFF_X) + line * C::LSTRIDE; }

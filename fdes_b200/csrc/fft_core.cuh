@@ -407,6 +407,23 @@ struct TwShared {
         return v;
     }
 };
+// The second-pass twiddles of a 1024-point line with 32 points per thread (32 x 32) in registers.  Its only
+// table is tab[t * 32 + k], t < 32, and thread theta < 32 reads entries k = theta only: 31 values, the same
+// for every line the thread transforms.  w[t - 1] = tab[t * 32 + theta].
+struct TwRegs {
+    cpx w[31];
+    __device__ __forceinline__ void load(const cpx* __restrict__ tab, int theta)
+    {
+#pragma unroll
+        for (int t = 1; t < 32; t++) w[t - 1] = ld_nc(tab + t * 32 + theta);
+    }
+    template <int OFF>
+    __device__ __forceinline__ cpx at(int) const     // the argument is theta
+    {
+        static_assert(OFF % 32 == 0 && OFF >= 32 && OFF < 1024, "TwRegs: second pass of a 32 x 32 line only");
+        return w[OFF / 32 - 1];
+    }
+};
 
 // v[t] *= tab[i0 + t * NS] (or its conjugate for the inverse transform), t = T0 .. R-1
 template <int R, int NS, int DIR, int T0, class TW>

@@ -1,8 +1,11 @@
 // Developer microbenchmark: the register-staged column sweep S6 (k_propagate_cols) against the
 // TMA-pipelined persistent form (k_propagate_cols_tma, col_pipe.cuh) on random data; the two must
-// agree bit for bit (same arithmetic, different data movement).
+// agree bit for bit (same arithmetic, different data movement).  run_tw_ab: pass twiddles of the
+// pipelined form in registers against shared memory.
 //   nvcc -std=c++17 -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -I ../../fdes_b200/csrc col_bench.cu ../../fdes_b200/csrc/tma_map.cu -o col_bench
 #include "sweep_kernels.cuh"
+#include <algorithm>
+#include <array>
 #include <cstring>
 using namespace fdes;
 
@@ -148,9 +151,70 @@ void run(int batch, int reps)
     cudaFree(d0); cudaFree(d1); cudaFree(P); cudaFree(tw);
 }
 
+// A/B of ColPipe's pass twiddles at N: registers (TwRegs, DBG 0) against shared memory only (DBG 4), in
+// k_dbg (the S6 kernel), `rounds` alternated timings of `reps` launches each on the same random stack of
+// `batch` images; the two outputs of one launch on the same input must agree bit for bit.
+template <int N>
+void run_tw_ab(int batch, int reps, int rounds)
+{
+    const size_t NN = (size_t)N * N, total = NN * batch, Q = N / 2 + 1;
+    std::vector<cpx> h(total), ph(Q * Q);
+    srand(4321);
+    for (auto& v : h) v = make_float2(rand() / (float)RAND_MAX - 0.5f, rand() / (float)RAND_MAX - 0.5f);
+    for (size_t i = 0; i < Q * Q; i++) { const float a = 0.001f * (float)(i % 977); ph[i] = make_float2(cosf(a) / N, sinf(a) / N); }
+    cpx *da, *db, *P, *tw;
+    CK(cudaMalloc(&da, total * sizeof(cpx))); CK(cudaMalloc(&db, total * sizeof(cpx))); CK(cudaMalloc(&P, Q * Q * sizeof(cpx)));
+    auto twh = make_twiddles_n<N>();
+    CK(cudaMalloc(&tw, twh.size() * sizeof(cpx)));
+    CK(cudaMemcpy(tw, twh.data(), twh.size() * sizeof(cpx), cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(P, ph.data(), Q * Q * sizeof(cpx), cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(da, h.data(), total * sizeof(cpx), cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(db, h.data(), total * sizeof(cpx), cudaMemcpyHostToDevice));
+    using Pc = PipeCfg<N>;
+    CK(cudaFuncSetAttribute(k_dbg<N, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Pc::SMEM));
+    CK(cudaFuncSetAttribute(k_dbg<N, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Pc::SMEM));
+    SweepGeom g{N, Band<N>::lo_end, Band<N>::hi_start, tw};
+    const int tiles_x = band_cols(g) / Pc::CW, ntiles = tiles_x * batch;
+    CUtensorMap ma, mb;
+    tile_map(&ma, da, N, batch, Pc::CW, Pc::BR); tile_map(&mb, db, N, batch, Pc::CW, Pc::BR);
+    int nsm = 0; CK(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, 0));
+    const int grid = ntiles < nsm ? ntiles : nsm;
+    auto reg = [&] { k_dbg<N, 0><<<grid, Pc::THREADS, Pc::SMEM>>>(ma, P, g.lo_end, g.hi_start, tiles_x, ntiles, tw, nullptr); };
+    auto shd = [&] { k_dbg<N, 4><<<grid, Pc::THREADS, Pc::SMEM>>>(mb, P, g.lo_end, g.hi_start, tiles_x, ntiles, tw, nullptr); };
+    reg(); shd();
+    CK(cudaGetLastError()); CK(cudaDeviceSynchronize());
+    std::vector<cpx> a(total), b(total);
+    CK(cudaMemcpy(a.data(), da, total * sizeof(cpx), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(b.data(), db, total * sizeof(cpx), cudaMemcpyDeviceToHost));
+    size_t diff = 0, changed = 0;
+    for (size_t i = 0; i < total; i++) { diff += memcmp(&a[i], &b[i], sizeof(cpx)) != 0; changed += memcmp(&a[i], &h[i], sizeof(cpx)) != 0; }
+    cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1);
+    std::vector<float> t_reg, t_shd;
+    for (int r = 0; r < rounds; r++) {
+        for (int v = 0; v < 2; v++) {
+            cudaEventRecord(e0);
+            for (int k = 0; k < reps; k++) { if (v == 0) reg(); else shd(); }
+            cudaEventRecord(e1); cudaEventSynchronize(e1);
+            float ms = 0; cudaEventElapsedTime(&ms, e0, e1);
+            (v == 0 ? t_reg : t_shd).push_back(ms / reps * 1e3f);
+        }
+    }
+    CK(cudaGetLastError());
+    cudaFuncAttributes f0, f1;
+    cudaFuncGetAttributes(&f0, k_dbg<N, 0>); cudaFuncGetAttributes(&f1, k_dbg<N, 4>);
+    auto stats = [](std::vector<float> v) { std::sort(v.begin(), v.end()); return std::array<float, 3>{v.front(), v[v.size() / 2], v.back()}; };
+    const auto sr = stats(t_reg), ss = stats(t_shd);
+    printf("N=%4d batch=%2d S6 twiddles A/B, %d rounds x %d launches, us min/median/max | shared (regs=%3d): %.2f / %.2f / %.2f | "
+           "registers (regs=%3d): %.2f / %.2f / %.2f | median gain %.1f %% | differing=%zu changed=%zu of %zu\n",
+           N, batch, rounds, reps, f1.numRegs, ss[0], ss[1], ss[2], f0.numRegs, sr[0], sr[1], sr[2], 100.0 * (1.0 - sr[1] / ss[1]),
+           diff, changed, total);
+    cudaFree(da); cudaFree(db); cudaFree(P); cudaFree(tw);
+}
+
 int main(int argc, char** argv)
 {
     const int reps = 20;
+    run_tw_ab<1024>(40, 50, 7);
     run<1024>(8, reps);
     run<1024>(16, reps);
     run<2048>(8, reps);
