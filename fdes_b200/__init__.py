@@ -75,7 +75,7 @@ def load_library() -> ctypes.CDLL:
                                            c_i, ctypes.c_int]
     lib.fdes_b200_sweep_test.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_int, c_i, ctypes.c_int, c_f, ctypes.c_int,
                                          ctypes.POINTER(c_f), ctypes.POINTER(ctypes.c_longlong), ctypes.c_int,
-                                         ctypes.c_int]
+                                         ctypes.c_int, ctypes.c_int, c_i]
     lib.FDES.restype = None
     lib.FDES.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_char_p, ctypes.c_char_p, ctypes.c_char_p, c_f,
                          ctypes.c_int, c_f]
@@ -333,10 +333,11 @@ COL_PLAIN, COL_MUL_CPX_INV, COL_MUL_REAL_INV, COL_DP_ACCUM = range(4)
 ROW_STORE, ROW_ACCUM, ROW_INTENS_ACCUM, ROW_STORE_SHIFT, ROW_CROP_REAL = range(5)
 
 
-def sweep_test(op: int, n: int, batch: int, bufs, iargs=(), fargs=(), gpu_index: int = 0) -> None:
+def sweep_test(op: int, n: int, batch: int, bufs, iargs=(), fargs=(), gpu_index: int = 0, pipe_ctas: int = 0) -> int:
     """One sweep launcher run once on host arrays (fdes_b200_sweep_test).  `bufs` are C-contiguous
     complex64 / float32 / int32 arrays, uploaded, and overwritten in place with what the device holds
-    after the sweep."""
+    after the sweep.  pipe_ctas: CTAs of a pipelined column sweep (0: one per SM as in the engine, c >= 1:
+    min(c, tiles)).  Returns the grid of the pipelined launch (0: the op launched none)."""
     lib = load_library()
     for b in bufs:
         assert b.flags.c_contiguous and b.dtype in (np.complex64, np.float32, np.int32), b.dtype
@@ -345,10 +346,12 @@ def sweep_test(op: int, n: int, batch: int, bufs, iargs=(), fargs=(), gpu_index:
     ptrs = (ctypes.POINTER(ctypes.c_float) * max(len(bufs), 1))(
         *[b.ctypes.data_as(ctypes.POINTER(ctypes.c_float)) for b in bufs])
     sizes = (ctypes.c_longlong * max(len(bufs), 1))(*[b.nbytes // 4 for b in bufs])
+    grid = np.zeros(1, np.int32)
     rc = lib.fdes_b200_sweep_test(op, n, batch, _ip(ia), len(iargs), _fp(fa), len(fargs), ptrs, sizes, len(bufs),
-                                  gpu_index)
+                                  gpu_index, pipe_ctas, _ip(grid))
     if rc != 0:
         raise FdesError(lib.fdes_b200_last_error().decode())
+    return int(grid[0])
 
 
 def sweep_geom(n: int) -> dict:

@@ -500,14 +500,27 @@ RecordRows upload_row_pointers(DeviceAllocs& da, const int* rp_host, int nconf, 
     return r;
 }
 
+// CTA count of the pipelined column sweeps for the duration of one sweep test; restores the previous value on
+// every way out
+struct PipeCtasGuard {
+    int saved;
+    explicit PipeCtasGuard(int ctas) : saved(pipe_cta_cap) { pipe_cta_cap = ctas; pipe_last_grid = 0; }
+    ~PipeCtasGuard() { pipe_cta_cap = saved; }
+    PipeCtasGuard(const PipeCtasGuard&) = delete;
+    PipeCtasGuard& operator=(const PipeCtasGuard&) = delete;
+};
+
 }  // namespace
 
 extern "C" {
 
 int fdes_b200_sweep_test(int op, int N, int batch, const int* iargs, int n_iargs, const float* fargs, int n_fargs,
-                         float** bufs, const long long* buf_elems, int nbufs, int gpu_index)
+                         float** bufs, const long long* buf_elems, int nbufs, int gpu_index, int pipe_ctas,
+                         int* pipe_grid_out)
 {
     API_TRY
+    if (pipe_grid_out) *pipe_grid_out = 0;
+    if (pipe_ctas < 0) throw std::runtime_error("sweep test: pipe_ctas must be >= 0");
     auto ia = [&](int i) {
         if (i >= n_iargs) throw std::runtime_error("sweep test: too few integer arguments");
         return iargs[i];
@@ -577,6 +590,7 @@ int fdes_b200_sweep_test(int op, int N, int batch, const int* iargs, int n_iargs
     }
     auto c = [&](int i) { return reinterpret_cast<cpx*>(d[i]); };
 
+    const PipeCtasGuard pipe_schedule(pipe_ctas);
     switch (op) {
         case FDES_B200_SWEEP_DENSITY: {
             const int nZ = ia(2);
@@ -690,6 +704,7 @@ int fdes_b200_sweep_test(int op, int N, int batch, const int* iargs, int n_iargs
         }
     }
     ck(cudaStreamSynchronize(st), "downloads");
+    if (pipe_grid_out) *pipe_grid_out = pipe_last_grid;
     return 0;
     API_CATCH(-1)
 }

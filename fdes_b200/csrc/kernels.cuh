@@ -33,6 +33,12 @@ int rows_per_block(int N);
 int cols_per_block(int N);
 bool sweeps_pipelined(int N);   // column sweeps on the TMA pipeline (col_pipe.cuh): launch_propagate_cols_from works
 int line_points(int N);         // points per thread E of a line transform (0: generic sweeps, no row masks)
+// Grid of the pipelined column sweeps, per host thread (defined in sweeps.cu).  pipe_cta_cap 0 (the default, never
+// changed by the engine): one persistent CTA per SM; c >= 1: min(c, tiles) CTAs, any number of tiles per CTA -- the
+// sweep test hook sets it to run the same sweep under other tile schedules.  pipe_last_grid: the grid of the
+// thread's last pipelined launch.
+extern thread_local int pipe_cta_cap;
+extern thread_local int pipe_last_grid;
 
 // ---- per-slice sweeps (S1..S6, see DESIGN.md) -------------------------------------------
 // The potential sweeps S1..S3 work on slice PAIRS: the densities of slice and slice2 travel as the

@@ -221,15 +221,19 @@ constexpr bool pipe_supported() { return N == 512 || N == 1024 || N == 2048 || N
 // were fixed they are 21 % / 35 % faster: tools/microbench/col_bench.cu, profiles/r2_v4_col_bench.txt)
 static int pipe_grid(int ntiles)
 {
-    static std::atomic<int> sms[64];
-    int dev = 0;
-    FDES_CUDA_CHECK(cudaGetDevice(&dev));
-    int n = sms[dev & 63].load();
+    int n = pipe_cta_cap;               // (kernels.cuh) 0 unless a test asks for another tile schedule
     if (n == 0) {
-        FDES_CUDA_CHECK(cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev));
-        sms[dev & 63].store(n);
+        static std::atomic<int> sms[64];
+        int dev = 0;
+        FDES_CUDA_CHECK(cudaGetDevice(&dev));
+        n = sms[dev & 63].load();
+        if (n == 0) {
+            FDES_CUDA_CHECK(cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev));
+            sms[dev & 63].store(n);
+        }
     }
-    return ntiles < n ? ntiles : n;     // one persistent CTA per SM
+    pipe_last_grid = ntiles < n ? ntiles : n;     // one persistent CTA per SM
+    return pipe_last_grid;
 }
 
 // The reference multiplies complex fields with a 3-multiplication form (multiplyElementwise,

@@ -8,6 +8,10 @@
 
 namespace fdes {
 
+// read by pipe_grid (sweep_kernels.cuh), which every size's translation unit compiles
+thread_local int pipe_cta_cap = 0;
+thread_local int pipe_last_grid = 0;
+
 static const SweepVTable* find_fast_vtable(int N)
 {
     switch (N) {

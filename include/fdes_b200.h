@@ -180,7 +180,12 @@ int fdes_b200_sort_records(unsigned int* keys, int* cols, float* w, int n, int n
  * float pairs).  Every buffer is uploaded, the sweep runs on the N x N grid with the geometry the
  * engine uses (band columns, row masks of the deposit records), and every buffer is downloaded again,
  * so that what a sweep must not write still holds what the caller put there.  -1 on failure (also
- * when a buffer is too small for the arguments, or the size has no such sweep).  `batch` images:
+ * when a buffer is too small for the arguments, or the size has no such sweep).
+ * pipe_ctas: CTAs of the pipelined column sweeps (persistent CTAs that walk tiles t, t + grid, ...):
+ * 0 = as in the engine, one per SM; c >= 1 = min(c, tiles), so that c >= tiles gives every CTA exactly
+ * one tile and small c many tiles per CTA (the output must not depend on it); negative: -1.
+ * *pipe_grid_out (may be NULL) receives the grid of the pipelined launch, 0 when the op launched none.
+ * `batch` images:
  *   op                        iargs                                         fargs   bufs
  *   FDES_B200_SWEEP_GEOM      -                                             -       int[5] out: N lo_end hi_start
  *                                                                                   line_points pipelined (no device)
@@ -227,7 +232,8 @@ int fdes_b200_sort_records(unsigned int* keys, int* cols, float* w, int n, int n
 #define FDES_B200_SWEEP_PROBE 11
 #define FDES_B200_SWEEP_DETECTOR 12
 int fdes_b200_sweep_test(int op, int N, int batch, const int* iargs, int n_iargs, const float* fargs, int n_fargs,
-                         float** bufs, const long long* buf_elems, int nbufs, int gpu_index);
+                         float** bufs, const long long* buf_elems, int nbufs, int gpu_index, int pipe_ctas,
+                         int* pipe_grid_out);
 
 #ifdef __cplusplus
 }

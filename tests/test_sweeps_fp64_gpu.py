@@ -16,8 +16,8 @@ Checks: (a) per line (row of a row sweep, column of a column sweep) ||err||_2 <=
 global rel-L2 bound; (b) sentinels survive, no NaN reaches an output, written columns outside the band are
 exactly zero; (c) image b of a batch is bitwise the image run alone; (d) two launches agree bitwise.
 
-Setting FDES_SWEEP_ERRORS=<file.json> records the errors of a run per op and size (the bounds below were set from
-such a run).
+Setting FDES_SWEEP_ERRORS=<file.json> records the errors of a run per op and size (the bounds TAU / GLOB of
+sweep_cases.py were set from such a run).
 """
 import json
 import os
@@ -26,36 +26,16 @@ import numpy as np
 import pytest
 
 import sweep_model as sm
+import sweep_cases
+from sweep_cases import (FROM_VARIANTS, NCONF, NSL, PIPELINED, SENT, band_of, check_lines, confs_of, crand, nz_of,
+                         random_pq, record, records, run, same_bits, stack_with_nan)
 
 pytestmark = pytest.mark.gpu
 
 FAST = [64, 128, 256, 512, 1024, 2048, 4096, 320, 800, 1000]
 GENERIC = [96, 250, 600, 1022, 143]
 SIZES = FAST + GENERIC
-PIPELINED = [512, 1024, 2048, 4096]
 B_ODD, B_EVEN = 3, 2
-SENT = np.complex64(complex(1234.5, -777.25))
-
-# Bounds of the per-line metric ||err_line|| / (rms(ref) sqrt(L)) and of the global rel-L2 per op, about three times
-# the largest value over all fifteen sizes measured on an NVIDIA B200 (1000 W power limit); the run of this file
-# there took 5.3 min.  op: (measured line, at size; measured global, at size) -> bounds in TAU / GLOB
-MEASURED = {
-    "S1": (2.7e-6, 2048, 1.7e-7, 1022),         # lines with few deposits carry a small share of rms(ref)
-    "S2": (2.3e-7, 143, 1.8e-7, 4096),
-    "S3": (9.3e-7, 143, 6.3e-7, 143),
-    "S4": (2.9e-7, 143, 1.8e-7, 4096),
-    "S5": (3.0e-7, 143, 2.4e-7, 2048),
-    "S6": (2.5e-7, 143, 1.9e-7, 4096),
-    "S6 from": (2.2e-7, 1024, 1.9e-7, 4096),
-    "CTF": (2.3e-7, 143, 1.9e-7, 4096),
-    "DP accum": (3.2e-8, 96, 2.7e-8, 320),
-    "rows sum": (1.6e-7, 143, 1.1e-7, 4096),
-}
-TAU = {"S1": 8e-6, "S2": 7e-7, "S3": 3e-6, "S4": 9e-7, "S5": 9e-7, "S6": 8e-7, "S6 from": 7e-7, "CTF": 7e-7,
-       "DP accum": 1e-7, "rows sum": 5e-7}
-GLOB = {"S1": 5e-7, "S2": 5e-7, "S3": 2e-6, "S4": 5e-7, "S5": 7e-7, "S6": 6e-7, "S6 from": 6e-7, "CTF": 6e-7,
-        "DP accum": 8e-8, "rows sum": 3.5e-7}
-_ERRORS = {}        # this run's errors (FDES_SWEEP_ERRORS)
 
 
 @pytest.fixture(scope="module", autouse=True)
@@ -64,13 +44,7 @@ def _record_errors():
     path = os.environ.get("FDES_SWEEP_ERRORS")
     if path:
         with open(path, "w") as f:
-            json.dump(_ERRORS, f, indent=1, sort_keys=True)
-
-
-def record(op, n, **vals):
-    d = _ERRORS.setdefault(op, {}).setdefault(str(n), {})
-    for k, v in vals.items():
-        d[k] = max(float(v), d.get(k, 0.0))
+            json.dump(sweep_cases.ERRORS, f, indent=1, sort_keys=True)
 
 
 @pytest.fixture(scope="module")
@@ -79,129 +53,12 @@ def fbm():
     return fdes_b200
 
 
-_GEOM = {}
-
-
-def geom(fb, n):
-    if n not in _GEOM:
-        _GEOM[n] = fb.sweep_geom(n)
-    return _GEOM[n]
-
-
-def band_of(fb, n):
-    g = geom(fb, n)
-    return sm.band_columns(n, g["lo_end"], g["hi_start"])
-
-
-def crand(rng, shape):
-    return (rng.standard_normal(shape) + 1j * rng.standard_normal(shape)).astype(np.complex64)
-
-
-def check_lines(op, n, out, ref, cols=None, rows_axis=True, line_mask=None):
-    """(a): per-line and global error of out against ref over the columns `cols` (all if None); lines are rows
-    (rows_axis) or columns.  line_mask [..., N] restricts the lines compared (rows of S1)."""
-    out = np.asarray(out)
-    ref = np.asarray(ref)
-    if cols is not None:
-        out, ref = out[..., cols], ref[..., cols]
-    assert not np.isnan(out).any(), f"{op} {n}: NaN in the output"
-    err = out.astype(np.complex128) - ref
-    if line_mask is not None:
-        err, refm = err[line_mask], ref[line_mask]
-    else:
-        refm = ref
-    rms = np.sqrt(np.mean(np.abs(refm) ** 2))
-    if rows_axis:
-        per, L = np.linalg.norm(err, axis=-1), err.shape[-1]
-    else:
-        per, L = np.linalg.norm(err, axis=-2), err.shape[-2]
-    line = float(per.max() / (rms * np.sqrt(L)))
-    glob = float(np.linalg.norm(err) / np.linalg.norm(refm))
-    record(op, n, line=line, glob=glob)
-    assert line <= TAU[op], f"{op} {n}: per-line error {line:.3e}"
-    assert glob <= GLOB[op], f"{op} {n}: global rel-L2 {glob:.3e}"
-
-
-def run(fb, op, n, batch, bufs, iargs=(), fargs=()):
-    """Launch on copies; returns the buffers after the sweep."""
-    cp = [np.ascontiguousarray(b).copy() for b in bufs]
-    fb.sweep_test(op, n, batch, cp, iargs, fargs)
-    return cp
-
-
-def same_bits(a, b):
-    return np.array_equal(np.ascontiguousarray(a).view(np.uint32), np.ascontiguousarray(b).view(np.uint32))
-
-
-def nz_of(n):
-    return 2 if n >= 4096 else 4
-
-
-# ---------------------------------------------------------------------------------------------------
-# deposit records (S1 / S2)
-# ---------------------------------------------------------------------------------------------------
-NSL = 3
-NCONF = 6
-# species present per slice (configuration 1 has no deposit at all).  The pair (0, 1): species 0 in both, 1 only
-# in the second slice, 2 in neither, 3 only in the first.  Slice 2 alone or paired with itself: species 0 (and 3),
-# 1 and 2 absent -- so with the two species of 4096 both edges remain: 1 only in the second slice of the pair,
-# 1 absent from slice 2.
-PRESENT = {0: {0, 3}, 1: {0, 1}, 2: {0, 3}}
-
-
-def make_records(n, nz, seed):
-    rng = np.random.default_rng(seed)
-    special = sorted({r for r in (0, 1, 3, 4, 7, 8, 31, 32, 63, 64, n // 2 - 1, n // 2, n - 2, n - 1) if 0 <= r < n})
-    per = []
-    for c in range(NCONF):
-        keys, cols, ws = [], [], []
-        if c != 1:
-            for s in range(NSL):
-                for z in range(nz):
-                    if z not in PRESENT[s]:
-                        continue
-                    rows = set(special) | set(rng.choice(n, max(n // 16, 1), replace=False).tolist())
-                    for r in sorted(rows):
-                        k = int(rng.integers(1, 4))
-                        keys += [(s * nz + z) * n + r] * k
-                        cols += rng.integers(0, n, k).tolist()
-                        ws += (rng.random(k) + 0.1).tolist()
-                    keys += [(s * nz + z) * n + n // 2] * 40          # many records on one pixel
-                    cols += [min(5, n - 1)] * 40
-                    ws += rng.random(40).tolist()
-        per.append((np.array(keys, np.int64), np.array(cols, np.int32), np.array(ws, np.float32)))
-    rec_stride = max(len(k) for k, _, _ in per)
-    nkeys = NSL * nz * n
-    rowptr = np.zeros((NCONF, nkeys + 1), np.int32)
-    cols = np.zeros((NCONF, rec_stride), np.int32)
-    w = np.zeros((NCONF, rec_stride), np.float32)
-    for c, (k, cc, ww) in enumerate(per):
-        o = np.argsort(k, kind="stable")
-        rowptr[c] = np.searchsorted(k[o], np.arange(nkeys + 1))
-        cols[c, :len(k)] = cc[o]
-        w[c, :len(k)] = ww[o]
-    return rowptr, cols, w
-
-
-_RECORDS = {}
-
-
-def records(n):
-    if n not in _RECORDS:
-        _RECORDS[n] = make_records(n, nz_of(n), 1000 + n)
-    return _RECORDS[n]
-
-
 # (slice, slice2, cfg_stride, cfg_off2, batches)
 PAIRINGS = {
     "pair": (0, 1, 1, 0, (1, B_ODD)),
     "single": (2, -1, 1, 0, (1, B_ODD)),
     "configs": (2, 2, 2, 1, (B_EVEN, B_ODD)),
 }
-
-
-def confs_of(b, cs, off):
-    return [b * cs] if off == 0 else [b * cs, b * cs + off]
 
 
 @pytest.mark.parametrize("pairing", list(PAIRINGS))
@@ -370,14 +227,6 @@ MIXED_TAU = 24.0        # measured on the B200: 8.0 (2048)
 # ---------------------------------------------------------------------------------------------------
 # S4
 # ---------------------------------------------------------------------------------------------------
-def stack_with_nan(rng, n, images, entries, band):
-    W = np.full((images, n, n), np.nan + 1j * np.nan, np.complex64)
-    for e in entries:
-        W[e] = crand(rng, (n, n))
-        W[e][:, ~band] = np.nan
-    return W
-
-
 @pytest.mark.parametrize("npair", [0, 1, 2])
 @pytest.mark.parametrize("n", SIZES)
 def test_bandlimit_cols(fbm, n, npair):
@@ -429,11 +278,6 @@ def test_multiply_rows(fbm, n, e_stride, psi_full):
 # ---------------------------------------------------------------------------------------------------
 # S6 and the sweeps reading another stack
 # ---------------------------------------------------------------------------------------------------
-def random_pq(rng, n):
-    Q = n // 2 + 1
-    return crand(rng, Q * Q) / np.float32(n)
-
-
 @pytest.mark.parametrize("n", SIZES)
 def test_propagate_cols(fbm, n):
     rng = np.random.default_rng(6000 + n)
@@ -448,14 +292,6 @@ def test_propagate_cols(fbm, n):
     b = B_ODD - 1
     assert same_bits(run(fbm, fbm.SWEEP_PROPAGATE, n, 1, [Psi[b:b + 1], Pq])[0][0], out[b])
     assert same_bits(run(fbm, fbm.SWEEP_PROPAGATE, n, B_ODD, [Psi, Pq])[0], out)
-
-
-FROM_VARIANTS = {          # (src_img_stride, times_n, lens): first slice of a pair / of the odd pairing, the CTF
-    "pair_first": (2, True, False),
-    "odd_first": (1, True, False),
-    "ctf_last": (1, False, True),
-    "single_slice": (2, True, True),
-}
 
 
 @pytest.mark.parametrize("variant", list(FROM_VARIANTS))
