@@ -68,6 +68,10 @@ def load_library() -> ctypes.CDLL:
     lib.fdes_b200_bench_configs.restype = ctypes.c_double
     lib.fdes_b200_stem_scan.argtypes = [vp, ctypes.c_int, ctypes.c_int, c_f, ctypes.c_int, c_f, c_f]
     lib.fdes_b200_stem_scan.restype = ctypes.c_double
+    lib.fdes_b200_stem_scan_4d.argtypes = [vp, ctypes.c_int, ctypes.c_int, c_f, ctypes.c_int, ctypes.c_int, ctypes.c_int, c_f,
+                                           ctypes.c_int, c_f, c_f]
+    lib.fdes_b200_stem_scan_4d.restype = ctypes.c_double
+    lib.fdes_b200_stem_4d_side.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_int]
     lib.fdes_b200_time_sweeps.argtypes = [vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, c_f]
     lib.fdes_b200_get_counters.argtypes = [vp, ctypes.POINTER(ctypes.c_longlong), ctypes.c_int]
     lib.fdes_b200_fft2d.argtypes = [c_f, ctypes.c_int, ctypes.c_int, ctypes.c_int]
@@ -166,6 +170,16 @@ def write_emd(input_path, emd_path, image=None, potential=None, exitwave=None):
                                  ptr(potential, np.complex64), nslices, ptr(exitwave, np.complex64))
     if rc != 0:
         raise FdesError(lib.fdes_b200_last_error().decode())
+
+
+def stem_4d_side(n: int, window: int = 0, bin: int = 1) -> int:
+    """Host-only: side of the 4D-STEM patterns (Q / bin) on an n x n grid; window 0 is the smallest centred window
+    that holds the band limit.  Raises FdesError with the reason when window / bin are not admissible."""
+    lib = load_library()
+    side = lib.fdes_b200_stem_4d_side(int(n), int(window), int(bin))
+    if side < 0:
+        raise FdesError(lib.fdes_b200_last_error().decode())
+    return side
 
 
 def parse_gpu_list(spec, first: int = 0):
@@ -307,6 +321,31 @@ class Simulation:
             raise FdesError(self._lib.fdes_b200_last_error().decode())
         return out, float(ms)
 
+    def stem_scan_4d(self, positions: np.ndarray, window: int = 0, bin: int = 1, detectors_mrad=None, k: int = 0,
+                     probes_per_pass: int = 0, out: Optional[np.ndarray] = None):
+        """4D-STEM scan (mode 2 .cnf): the diffraction pattern of every probe, fftshifted, cropped to the centred
+        window of side `window` (0: the smallest that holds the band limit) and binned bin x bin
+        (fdes_b200_stem_scan_4d).  positions [n, 2] as for stem_scan; detectors_mrad [ndet, 2] (optional) adds the
+        annular signals of the same pass, bitwise those of stem_scan.  out: a caller-owned float32 C-contiguous
+        array [n, side, side] (e.g. an np.memmap, so that a scan larger than the RAM streams to disk).
+        Returns (patterns [n, side, side], signals [n, ndet] or None, device ms)."""
+        pos = np.ascontiguousarray(positions, np.float32).reshape(-1, 2)
+        side = stem_4d_side(self.m1, window, bin)
+        shape = (pos.shape[0], side, side)
+        if out is None:
+            out = np.zeros(shape, np.float32)
+        elif out.dtype != np.float32 or not out.flags.c_contiguous or out.shape != shape or not out.flags.writeable:
+            raise FdesError(f"out must be a writeable C-contiguous float32 array of shape {shape}")
+        det = None if detectors_mrad is None else np.ascontiguousarray(detectors_mrad, np.float32).reshape(-1, 2)
+        ndet = 0 if det is None else det.shape[0]
+        sig = np.zeros((pos.shape[0], ndet), np.float32) if ndet else None
+        ms = self._lib.fdes_b200_stem_scan_4d(self._h, k, pos.shape[0], _fp(pos), window, bin, ndet,
+                                              _fp(det) if ndet else None, probes_per_pass, _fp(out),
+                                              _fp(sig) if ndet else None)
+        if ms < 0:
+            raise FdesError(self._lib.fdes_b200_last_error().decode())
+        return out, sig, float(ms)
+
     def time_sweeps(self, k: int = 0, batch: int = 0, reps: int = 20):
         """Average launch duration [ms] of the six per-slice sweeps S1..S6."""
         ms = np.zeros(6, np.float32)
@@ -328,6 +367,7 @@ def fft2d(a: np.ndarray, direction: int = -1, gpu_index: int = 0) -> np.ndarray:
 # operations of fdes_b200_sweep_test (include/fdes_b200.h)
 SWEEP_GEOM, SWEEP_DENSITY, SWEEP_POTENTIAL, SWEEP_TRANSMIT, SWEEP_BANDLIMIT, SWEEP_MULTIPLY, SWEEP_PROPAGATE, \
     SWEEP_PROPAGATE_FROM, SWEEP_COLS_FFT, SWEEP_ROWS_FFT_SUM, SWEEP_ROWS_FFT, SWEEP_PROBE, SWEEP_DETECTOR = range(13)
+SWEEP_DETECTOR4D = 13
 # ColOp and RowEpilogue values (fdes_b200/csrc/kernels.cuh)
 COL_PLAIN, COL_MUL_CPX_INV, COL_MUL_REAL_INV, COL_DP_ACCUM = range(4)
 ROW_STORE, ROW_ACCUM, ROW_INTENS_ACCUM, ROW_STORE_SHIFT, ROW_CROP_REAL = range(5)

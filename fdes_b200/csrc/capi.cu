@@ -368,6 +368,70 @@ double fdes_b200_stem_scan(fdes_b200_sim* sim, int k, int nprobes, const float* 
     API_CATCH(-1.0)
 }
 
+int fdes_b200_stem_4d_side(int N, int window, int bin)
+{
+    API_TRY
+    return stem4d_window(N, window, bin) / bin;
+    API_CATCH(-1)
+}
+
+double fdes_b200_stem_scan_4d(fdes_b200_sim* sim, int k, int nprobes, const float* xy_host, int window, int bin, int ndet,
+                              const float* det_mrad_host, int probes_per_pass, float* patterns_host, float* det_out_host)
+{
+    API_TRY
+    if (!patterns_host || (ndet > 0 && !det_out_host)) throw std::runtime_error("4D-STEM output array is NULL");
+    const int n = (int)sim->engs.size();
+    if (n > 1 && nprobes > 0) {
+        const int side = stem4d_window(sim->eng->grid(), window, bin) / bin;
+        const size_t SS = (size_t)side * side;
+        std::vector<double> ms(n, 0.0);
+        if (sim->shard == SHARD_CONFIGS) {
+            // every device computes each pass with its share of the frozen-phonon configurations (weights 1/count
+            // inside); the passes are summed here in device order, so that the host holds one pass per device
+            if (probes_per_pass < 0) throw std::runtime_error("probes_per_pass must be >= 0 (0: automatic)");
+            int ppp = probes_per_pass > 0 ? std::min(probes_per_pass, nprobes) : nprobes;
+            if (probes_per_pass == 0)
+                for (auto& e : sim->engs) ppp = std::min(ppp, e->stem_4d_probes_per_pass(nprobes, window, bin));
+            std::vector<std::vector<float>> part(n), dpart(n);
+            for (int p0 = 0; p0 < nprobes; p0 += ppp) {
+                const int np = std::min(ppp, nprobes - p0);
+                parallel_for(n, [&](int r) {
+                    part[r].resize((size_t)np * SS);
+                    dpart[r].resize((size_t)np * ndet);
+                    double t = 0.0;
+                    sim->engs[r]->stem_scan_4d(k, np, xy_host + 2 * (size_t)p0, window, bin, ndet, det_mrad_host, np, part[r].data(),
+                                               dpart[r].data(), &t);
+                    ms[r] += t;
+                });
+                for (size_t i = 0; i < (size_t)np * SS; i++) {
+                    float s = part[0][i];
+                    for (int r = 1; r < n; r++) s += part[r][i];
+                    patterns_host[(size_t)p0 * SS + i] = s;
+                }
+                for (size_t i = 0; i < (size_t)np * ndet; i++) {
+                    float s = dpart[0][i];
+                    for (int r = 1; r < n; r++) s += dpart[r][i];
+                    det_out_host[(size_t)p0 * ndet + i] = s;
+                }
+            }
+        } else {
+            // replicas: contiguous ranges of the raster per device, written in place
+            parallel_for(n, [&](int r) {
+                const int i0 = (int)((long long)nprobes * r / n), i1 = (int)((long long)nprobes * (r + 1) / n);
+                if (i1 > i0)
+                    sim->engs[r]->stem_scan_4d(k, i1 - i0, xy_host + 2 * (size_t)i0, window, bin, ndet, det_mrad_host, probes_per_pass,
+                                               patterns_host + (size_t)i0 * SS, det_out_host ? det_out_host + (size_t)i0 * ndet : nullptr,
+                                               &ms[r]);
+            });
+        }
+        return *std::max_element(ms.begin(), ms.end());
+    }
+    double ms = 0.0;
+    sim->eng->stem_scan_4d(k, nprobes, xy_host, window, bin, ndet, det_mrad_host, probes_per_pass, patterns_host, det_out_host, &ms);
+    return ms;
+    API_CATCH(-1.0)
+}
+
 int fdes_b200_time_sweeps(fdes_b200_sim* sim, int k, int batch, int reps, float* ms6)
 {
     API_TRY
@@ -690,6 +754,24 @@ int fdes_b200_sweep_test(int op, int N, int batch, const int* iargs, int n_iargs
             float* partial = static_cast<float*>(da.get(np * sizeof(float)));
             launch_fill_f32(partial, np, std::nanf(""), st);
             launch_detector_cols(g, c(0), partial, d[1], rings, fa(0), fa(1), fa(2), batch, st);
+        } break;
+        case FDES_B200_SWEEP_DETECTOR4D: {
+            const int Q = ia(0), bin = ia(1);
+            if (Q < 1) throw std::runtime_error("sweep test: window must be >= 1");
+            stem4d_window(N, Q, bin);
+            const size_t S = (size_t)(Q / bin);
+            need(0, (size_t)batch * IMG); need(1, (size_t)batch * S * S);
+            // scratch: NaN in the band columns (the sweep must write each of their window pixels before the bins are
+            // summed), 0 in the others (the engine zeroes them once per scan)
+            std::vector<float> h((size_t)batch * Q * Q);
+            for (size_t i = 0; i < h.size(); i++) {
+                const int kx = (int)((i % Q) + (N - Q) / 2 + N - N / 2) % N;
+                h[i] = (kx < g.lo_end || kx >= g.hi_start) ? std::nanf("") : 0.f;
+            }
+            float* scratch = static_cast<float*>(da.get(h.size() * sizeof(float)));
+            ck(cudaMemcpyAsync(scratch, h.data(), h.size() * sizeof(float), cudaMemcpyHostToDevice, st), "cudaMemcpyAsync");
+            launch_detector4d_cols(g, c(0), scratch, d[1], Q, bin, fa(0), batch, st);
+            ck(cudaStreamSynchronize(st), "sweep kernels");     // h goes out of scope
         } break;
         default: throw std::runtime_error("sweep test: unknown op " + std::to_string(op));
     }

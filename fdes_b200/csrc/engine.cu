@@ -858,16 +858,14 @@ double Engine::bench_configs(int k, int configs)
 // then advance in batches through S5/S6 only, and annular detectors integrate the diffraction
 // intensity |FFT2 psi|^2 / N^2 (diffractionPattern, src/crystalMaker.cu:700-718).
 // ---------------------------------------------------------------------------------------------
-void Engine::stem_scan(int k, int nprobes, const float* xy_host, int ndet, const float* det_mrad_host,
-                       float* out_host, double* loop_ms)
+// Checks shared by the scans; the annular detectors as |k|^2 bounds
+DetectorRings Engine::stem_rings(int k, int nprobes, int ndet, const float* det_mrad_host, int min_det) const
 {
-    DeviceGuard guard(opt_.gpu_index);
     if (p_.mode != 2) throw std::runtime_error("STEM scan needs mode 2 (convergent probe)");
     if (k < 0 || k >= p_.n3) throw std::runtime_error("measurement index out of range");
     if (nprobes <= 0) throw std::runtime_error("no probe positions");
-    if (ndet <= 0 || ndet > MAX_DETECTORS) throw std::runtime_error("1..8 detectors supported");
+    if (ndet < min_det || ndet > MAX_DETECTORS) throw std::runtime_error(std::to_string(min_det) + "..8 detectors supported");
     if (p_.doBeamTilt) throw std::runtime_error("STEM scan with beam tilt is not supported");
-    const size_t NN = (size_t)N_ * N_;
     DetectorRings rings{};
     rings.n = ndet;
     for (int d = 0; d < ndet; d++) {
@@ -876,6 +874,68 @@ void Engine::stem_scan(int k, int nprobes, const float* xy_host, int ndet, const
         rings.in2[d] = a * a;
         rings.out2[d] = b * b;
     }
+    return rings;
+}
+
+// probe shifts -> shifts (device), zeroed detector sums, incident probe of index k and its column spectrum PSI0 in
+// scratch_; returns after the device has taken the host data
+void Engine::stem_prepare(int k, int nprobes, const float* xy_host, float* shifts, float* det_out, size_t det_elems)
+{
+    std::vector<float> sh(2 * (size_t)nprobes);
+    for (int i = 0; i < nprobes; i++) {
+        sh[2 * i] = xy_host[2 * i] / ((float)N_ * p_.d1);
+        sh[2 * i + 1] = xy_host[2 * i + 1] / ((float)N_ * p_.d2);
+    }
+    CK(cudaMemcpyAsync(shifts, sh.data(), sh.size() * sizeof(float), cudaMemcpyHostToDevice, st_));
+    launch_fill_f32(det_out, det_elems, 0.f, st_);
+    CK(cudaMemcpyAsync(xyzK_, xyzTO_, 3 * (size_t)nAt_ * sizeof(float), cudaMemcpyDeviceToDevice, st_));
+    tilt(xyzK_, p_.tiltspec[2 * k], p_.tiltspec[2 * k + 1], 0.f);
+    make_incident(k);
+    // spectrum of the centred probe: PSI0 = FFT_col(psi_in) (scratch_ is free after make_incident)
+    launch_cols_fft(g_, psi_in_, scratch_, -1, COL_PLAIN, nullptr, 1.f, 1, st_);
+    CK(cudaStreamSynchronize(st_));    // sh goes out of scope
+}
+
+// transmission stack of configuration (k, j): the same displacements whenever it is built (rng_target_ re-seeds the
+// streams when they are past it)
+void Engine::stem_transmission(int k, int j, cpx* tstack)
+{
+    const size_t NN = (size_t)N_ * N_;
+    rng_target_ = (long long)k * count_ + j;
+    prepare_batch(1, xyzK_);
+    for (int s = 0; s < p_.m3; s += 2) {
+        const int npair = std::min(2, p_.m3 - s);
+        const int s2 = npair > 1 ? s + 1 : -1;
+        launch_density_rows(g_, A_, rs_[act_].rowptr, rs_[act_].cols, rs_[act_].w, s, s2, nZ_, 1, rec_stride_, rp_stride_, st_);
+        launch_potential_cols(g_, W_, A_, Gq_, rs_[act_].rowptr, s, s2, nZ_, 1, rp_stride_, st_);
+        launch_transmit_rows(g_, W_, tstack + (size_t)s * NN, npair, p_.imPot, 1, st_);
+        launch_bandlimit_cols(g_, tstack + (size_t)s * NN, 1, npair, st_);
+    }
+    // (keeping t in real space instead, to save the per-probe inverse row transform of S5,
+    // measured SLOWER on B200: 8.3k vs 9.5k probes/s at 512^2 -- the transform hides the
+    // latency of the wave loads)
+    tm_.kernel_launches += 4LL * ((p_.m3 + 1) / 2);
+}
+
+// nb probes at shifts through every slice of tstack: exit waves in Psi_
+void Engine::stem_probes(const float* shifts, int nb, const cpx* tstack)
+{
+    const size_t NN = (size_t)N_ * N_;
+    launch_probe_cols(g_, Psi_, scratch_, shifts, nb, st_);
+    for (int s = 0; s < p_.m3; s++) {
+        launch_multiply_rows(g_, Psi_, tstack + (size_t)s * NN, 0, nb, false, st_);
+        launch_propagate_cols(g_, Psi_, Pq_, nb, st_);
+    }
+    tm_.kernel_launches += 1 + 2LL * p_.m3;
+    tm_.slices_executed += (long long)p_.m3 * nb;
+}
+
+void Engine::stem_scan(int k, int nprobes, const float* xy_host, int ndet, const float* det_mrad_host,
+                       float* out_host, double* loop_ms)
+{
+    DeviceGuard guard(opt_.gpu_index);
+    const DetectorRings rings = stem_rings(k, nprobes, ndet, det_mrad_host, 1);
+    const size_t NN = (size_t)N_ * N_;
     // device scratch of this call: transmission stack, probe shifts, detector sums
     const int tiles = detector_tiles(g_);
     cpx* tstack = nullptr; float *shifts = nullptr, *out = nullptr, *partial = nullptr;
@@ -887,51 +947,183 @@ void Engine::stem_scan(int k, int nprobes, const float* xy_host, int ndet, const
     void* block = pool_acquire(plan.total(), opt_.gpu_index);
     plan.assign(block);
     try {
-        std::vector<float> sh(2 * (size_t)nprobes);
-        for (int i = 0; i < nprobes; i++) {
-            sh[2 * i] = xy_host[2 * i] / ((float)N_ * p_.d1);
-            sh[2 * i + 1] = xy_host[2 * i + 1] / ((float)N_ * p_.d2);
-        }
-        CK(cudaMemcpyAsync(shifts, sh.data(), sh.size() * sizeof(float), cudaMemcpyHostToDevice, st_));
-        launch_fill_f32(out, (size_t)nprobes * ndet, 0.f, st_);
-        CK(cudaMemcpyAsync(xyzK_, xyzTO_, 3 * (size_t)nAt_ * sizeof(float), cudaMemcpyDeviceToDevice, st_));
-        tilt(xyzK_, p_.tiltspec[2 * k], p_.tiltspec[2 * k + 1], 0.f);
-        make_incident(k);
-        // spectrum of the centred probe: PSI0 = FFT_col(psi_in) (scratch_ is free after make_incident)
-        launch_cols_fft(g_, psi_in_, scratch_, -1, COL_PLAIN, nullptr, 1.f, 1, st_);
-        CK(cudaStreamSynchronize(st_));    // sh goes out of scope below
+        stem_prepare(k, nprobes, xy_host, shifts, out, (size_t)nprobes * ndet);
         CK(cudaEventRecord(ev0_, st_));
         const float weight = 1.f / (float)count_;
         for (int j = j0_; j < j1_; j++) {
-            rng_target_ = (long long)k * count_ + j;
-            prepare_batch(1, xyzK_);
-            for (int s = 0; s < p_.m3; s += 2) {   // transmission stack of this configuration
-                const int npair = std::min(2, p_.m3 - s);
-                const int s2 = npair > 1 ? s + 1 : -1;
-                launch_density_rows(g_, A_, rs_[act_].rowptr, rs_[act_].cols, rs_[act_].w, s, s2, nZ_, 1, rec_stride_, rp_stride_, st_);
-                launch_potential_cols(g_, W_, A_, Gq_, rs_[act_].rowptr, s, s2, nZ_, 1, rp_stride_, st_);
-                launch_transmit_rows(g_, W_, tstack + (size_t)s * NN, npair, p_.imPot, 1, st_);
-                launch_bandlimit_cols(g_, tstack + (size_t)s * NN, 1, npair, st_);
-            }
-            // (keeping t in real space instead, to save the per-probe inverse row transform of S5,
-            // measured SLOWER on B200: 8.3k vs 9.5k probes/s at 512^2 -- the transform hides the
-            // latency of the wave loads)
-            tm_.kernel_launches += 4LL * ((p_.m3 + 1) / 2);
+            stem_transmission(k, j, tstack);
             for (int i0 = 0; i0 < nprobes; i0 += B_) {
                 const int nb = std::min(B_, nprobes - i0);
-                launch_probe_cols(g_, Psi_, scratch_, shifts + 2 * (size_t)i0, nb, st_);
-                for (int s = 0; s < p_.m3; s++) {
-                    launch_multiply_rows(g_, Psi_, tstack + (size_t)s * NN, 0, nb, false, st_);
-                    launch_propagate_cols(g_, Psi_, Pq_, nb, st_);
-                }
+                stem_probes(shifts + 2 * (size_t)i0, nb, tstack);
                 launch_detector_cols(g_, Psi_, partial, out + (size_t)i0 * ndet, rings, p_.d1, p_.d2, weight, nb, st_);
-                tm_.kernel_launches += 3 + 2LL * p_.m3;
-                tm_.slices_executed += (long long)p_.m3 * nb;
+                tm_.kernel_launches += 2;
             }
         }
         CK(cudaEventRecord(ev1_, st_));
         CK(cudaMemcpyAsync(out_host, out, (size_t)nprobes * ndet * sizeof(float), cudaMemcpyDeviceToHost, st_));
         CK(cudaStreamSynchronize(st_));
+        if (loop_ms) { float ms = 0.f; CK(cudaEventElapsedTime(&ms, ev0_, ev1_)); *loop_ms = ms; }
+    } catch (...) {
+        cudaStreamSynchronize(st_);
+        pool_release(block);
+        throw;
+    }
+    pool_release(block);
+}
+
+// ---------------------------------------------------------------------------------------------
+// 4D-STEM: the diffraction pattern of every probe, fftshifted, cropped to a centred window of Q x Q pixels and
+// binned bin x bin.  A whole data set does not fit the device (256^2 probes x 342^2 pixels x 4 B = 30 GB at 512^2),
+// so the raster runs in passes of probes_per_pass probes; a pass rebuilds the transmission stack of every
+// configuration (S1..S4 are a small share of a pass: one stack per configuration against m3 x (S5, S6) per probe).
+// Finished passes go to the host from the other of two device pass buffers while the next pass computes: in chunks
+// through two pinned buffers on two copy streams, each chunk copied on to its place in the caller's array by a
+// host function of its stream.
+// ---------------------------------------------------------------------------------------------
+int stem4d_window(int N, int window, int bin)
+{
+    if (N < 1) throw std::runtime_error("grid size must be positive");
+    if (bin < 1) throw std::runtime_error("4D-STEM bin must be >= 1");
+    if (window < 0) throw std::runtime_error("4D-STEM window must be >= 0 (0: the band limit)");
+    if (window == 0) {
+        // kb: the largest |i| the band limit keeps on an axis (zeroHighFreq's float test, src/multisliceSimulation.cu:225-250;
+        // the same loop as make_sweep_geom).  Window pixel q holds frequency q - Q/2: an even Q covers [-Q/2, Q/2 - 1],
+        // an odd Q [-(Q-1)/2, (Q-1)/2].
+        int kb = 0;
+        const float mind = (float)N;
+        while (kb + 1 <= N / 2 && !(((float)((kb + 1) * (kb + 1)) * 9.f / (mind * mind)) > 1.f)) kb++;
+        int Q = 2 * kb + 1 + (N % 2 == 0 ? 1 : 0);
+        while (Q <= N && Q % bin != 0) Q += 2;
+        if (Q > N)
+            throw std::runtime_error("4D-STEM: no window of N's parity (N = " + std::to_string(N) + ") that is a multiple of bin " +
+                                     std::to_string(bin) + " holds the band limit");
+        return Q;
+    }
+    if (window > N) throw std::runtime_error("4D-STEM window " + std::to_string(window) + " larger than the grid (" + std::to_string(N) + ")");
+    if ((N - window) % 2 != 0)
+        throw std::runtime_error("4D-STEM window " + std::to_string(window) + " must have the parity of the grid size " + std::to_string(N) +
+                                 " (a whole-pixel centred crop)");
+    if (window % bin != 0)
+        throw std::runtime_error("4D-STEM window " + std::to_string(window) + " is not a multiple of bin " + std::to_string(bin));
+    return window;
+}
+
+int Engine::stem_4d_probes_per_pass(int nprobes, int window, int bin)
+{
+    DeviceGuard guard(opt_.gpu_index);
+    const int S = stem4d_window(N_, window, bin) / bin;
+    size_t fr = 0, tot = 0;
+    CK(cudaMemGetInfo(&fr, &tot));
+    // the two pass buffers: at most about a quarter of the free memory
+    const size_t per_probe = 2 * (size_t)S * S * sizeof(float);
+    return (int)std::max<size_t>(1, std::min<size_t>((size_t)std::max(nprobes, 1), fr / 4 / per_probe));
+}
+
+namespace {
+struct HostCopy { float* dst; const float* src; size_t bytes; };
+void CUDART_CB host_copy(void* p)
+{
+    const HostCopy* c = static_cast<const HostCopy*>(p);
+    memcpy(c->dst, c->src, c->bytes);
+}
+// copy streams, events and pinned chunks of one 4D scan; the destructor waits for every copy
+struct PassCopies {
+    static constexpr size_t CHUNK = (size_t)64 << 20;    // bytes per pinned buffer
+    cudaStream_t st[2] = {nullptr, nullptr};
+    cudaEvent_t done[2] = {nullptr, nullptr}, copied[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};
+    float* pin[2] = {nullptr, nullptr};
+    PassCopies()
+    {
+        for (int i = 0; i < 2; i++) {
+            CK(cudaStreamCreateWithFlags(&st[i], cudaStreamNonBlocking));
+            CK(cudaEventCreateWithFlags(&done[i], cudaEventDisableTiming));
+            for (int q = 0; q < 2; q++) CK(cudaEventCreateWithFlags(&copied[i][q], cudaEventDisableTiming));
+            CK(cudaHostAlloc(reinterpret_cast<void**>(&pin[i]), CHUNK, cudaHostAllocDefault));
+        }
+    }
+    ~PassCopies()
+    {
+        for (int i = 0; i < 2; i++) {
+            if (st[i]) { cudaStreamSynchronize(st[i]); cudaStreamDestroy(st[i]); }
+            if (done[i]) cudaEventDestroy(done[i]);
+            for (int q = 0; q < 2; q++) if (copied[i][q]) cudaEventDestroy(copied[i][q]);
+            if (pin[i]) cudaFreeHost(pin[i]);
+        }
+    }
+    PassCopies(const PassCopies&) = delete;
+    PassCopies& operator=(const PassCopies&) = delete;
+};
+}  // namespace
+
+void Engine::stem_scan_4d(int k, int nprobes, const float* xy_host, int window, int bin, int ndet, const float* det_mrad_host,
+                          int probes_per_pass, float* out_pattern_host, float* out_det_host, double* loop_ms)
+{
+    DeviceGuard guard(opt_.gpu_index);
+    const DetectorRings rings = stem_rings(k, nprobes, ndet, det_mrad_host, 0);
+    const int Q = stem4d_window(N_, window, bin);
+    const size_t NN = (size_t)N_ * N_, QQ = (size_t)Q * Q, SS = (size_t)(Q / bin) * (Q / bin);
+    if (probes_per_pass < 0) throw std::runtime_error("probes_per_pass must be >= 0 (0: automatic)");
+    if (!out_pattern_host || (ndet > 0 && !out_det_host)) throw std::runtime_error("4D-STEM output array is NULL");
+    const int ppp = std::min(nprobes, probes_per_pass > 0 ? probes_per_pass : stem_4d_probes_per_pass(nprobes, window, bin));
+    const int tiles = detector_tiles(g_);
+    cpx* tstack = nullptr;
+    float *shifts = nullptr, *det = nullptr, *partial = nullptr, *scratch4d = nullptr, *pass[2] = {nullptr, nullptr};
+    ArenaPlan plan;
+    plan.add(tstack, ((size_t)p_.m3 + 1) * NN);
+    plan.add(shifts, 2 * (size_t)nprobes);
+    plan.add(det, (size_t)nprobes * ndet);
+    plan.add(partial, (size_t)B_ * tiles * MAX_DETECTORS);
+    plan.add(scratch4d, (size_t)B_ * QQ);
+    for (float*& p : pass) plan.add(p, (size_t)ppp * SS);
+    void* block = pool_acquire(plan.total(), opt_.gpu_index);
+    plan.assign(block);
+    const int npass = (nprobes + ppp - 1) / ppp;
+    const size_t chunk = PassCopies::CHUNK / sizeof(float);
+    std::vector<HostCopy> jobs;      // read by the host functions: no reallocation while they are queued
+    jobs.reserve((size_t)npass * (((size_t)ppp * SS + chunk - 1) / chunk));
+    try {
+        PassCopies pc;
+        stem_prepare(k, nprobes, xy_host, shifts, det, (size_t)nprobes * ndet);
+        // the pixels outside the band columns are never written by the 4D sweep
+        launch_fill_f32(scratch4d, (size_t)B_ * QQ, 0.f, st_);
+        CK(cudaEventRecord(ev0_, st_));
+        const float weight = 1.f / (float)count_;
+        size_t c = 0;
+        for (int pi = 0; pi < npass; pi++) {
+            const int s = pi & 1, p0 = pi * ppp, np = std::min(ppp, nprobes - p0);
+            if (pi >= 2)      // pass buffer s still on its way to the host (pass pi - 2)
+                for (int q = 0; q < 2; q++) CK(cudaStreamWaitEvent(st_, pc.copied[s][q], 0));
+            launch_fill_f32(pass[s], (size_t)np * SS, 0.f, st_);
+            tm_.kernel_launches += 1;
+            for (int j = j0_; j < j1_; j++) {
+                stem_transmission(k, j, tstack);
+                for (int i0 = 0; i0 < np; i0 += B_) {
+                    const int nb = std::min(B_, np - i0);
+                    stem_probes(shifts + 2 * (size_t)(p0 + i0), nb, tstack);
+                    launch_detector4d_cols(g_, Psi_, scratch4d, pass[s] + (size_t)i0 * SS, Q, bin, weight, nb, st_);
+                    tm_.kernel_launches += 2;
+                    if (ndet > 0) {
+                        launch_detector_cols(g_, Psi_, partial, det + (size_t)(p0 + i0) * ndet, rings, p_.d1, p_.d2, weight, nb, st_);
+                        tm_.kernel_launches += 2;
+                    }
+                }
+            }
+            CK(cudaEventRecord(pc.done[s], st_));
+            for (int q = 0; q < 2; q++) CK(cudaStreamWaitEvent(pc.st[q], pc.done[s], 0));
+            const size_t total = (size_t)np * SS;
+            for (size_t off = 0; off < total; off += chunk, c++) {
+                const int q = (int)(c & 1);
+                const size_t n = std::min(chunk, total - off);
+                CK(cudaMemcpyAsync(pc.pin[q], pass[s] + off, n * sizeof(float), cudaMemcpyDeviceToHost, pc.st[q]));
+                jobs.push_back({out_pattern_host + (size_t)p0 * SS + off, pc.pin[q], n * sizeof(float)});
+                CK(cudaLaunchHostFunc(pc.st[q], host_copy, &jobs.back()));
+            }
+            for (int q = 0; q < 2; q++) CK(cudaEventRecord(pc.copied[s][q], pc.st[q]));
+        }
+        CK(cudaEventRecord(ev1_, st_));
+        if (ndet > 0) CK(cudaMemcpyAsync(out_det_host, det, (size_t)nprobes * ndet * sizeof(float), cudaMemcpyDeviceToHost, st_));
+        CK(cudaStreamSynchronize(st_));
+        for (int q = 0; q < 2; q++) CK(cudaStreamSynchronize(pc.st[q]));
         if (loop_ms) { float ms = 0.f; CK(cudaEventElapsedTime(&ms, ev0_, ev1_)); *loop_ms = ms; }
     } catch (...) {
         cudaStreamSynchronize(st_);

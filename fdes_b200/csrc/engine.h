@@ -78,6 +78,16 @@ public:
     // with weight 1/count.  loop_ms (may be null): CUDA-event time of the scan.
     void stem_scan(int k, int nprobes, const float* xy_host, int ndet, const float* det_mrad_host,
                    float* out_host, double* loop_ms);
+    // 4D-STEM scan: out_pattern_host [nprobes][Q/bin][Q/bin] = the diffraction intensity of every probe, fftshifted,
+    // cropped to the centred window Q = stem4d_window(N, window, bin) and binned bin x bin, averaged like stem_scan;
+    // with ndet > 0 also the annular signals out_det_host [nprobes][ndet], bitwise those of stem_scan.  The raster
+    // runs in passes of probes_per_pass probes (0: stem_4d_probes_per_pass), the copy of a finished pass to the
+    // host overlapping the next pass.  loop_ms: CUDA-event time of the device loop.
+    void stem_scan_4d(int k, int nprobes, const float* xy_host, int window, int bin, int ndet, const float* det_mrad_host,
+                      int probes_per_pass, float* out_pattern_host, float* out_det_host, double* loop_ms);
+    // automatic pass size: the two device pass buffers take at most about a quarter of the free device memory,
+    // and never more than the whole raster
+    int stem_4d_probes_per_pass(int nprobes, int window, int bin);
     // average launch duration [ms] of each of the six sweeps on a prepared batch of nb configs
     void time_sweeps(int k, int nb, int reps, float* ms6);
     int batch() const { return B_; }
@@ -100,6 +110,11 @@ private:
     void run_slices_plain(int nb);
     void accumulate_outputs(int k, int nb);
     void tilt(float* xyz_dev, float t0, float t1, float t2);
+    // pieces of the STEM scans (engine.cu)
+    DetectorRings stem_rings(int k, int nprobes, int ndet, const float* det_mrad_host, int min_det) const;
+    void stem_prepare(int k, int nprobes, const float* xy_host, float* shifts, float* det_out, size_t det_elems);
+    void stem_transmission(int k, int j, cpx* tstack);
+    void stem_probes(const float* shifts, int nb, const cpx* tstack);
 
     Params p_;
     EngineOptions opt_;
@@ -151,5 +166,10 @@ private:
 
 // frees the device blocks cached between simulations (idle ones)
 void release_device_cache();
+
+// Side Q of the 4D-STEM window on an N x N grid (host only; throws with the reason when not admissible):
+// window > 0 is taken as is when 1 <= window <= N, window = N (mod 2) and bin divides it; window = 0 is the smallest
+// such Q that holds every frequency the 2/3 band limit keeps.
+int stem4d_window(int N, int window, int bin);
 
 }  // namespace fdes

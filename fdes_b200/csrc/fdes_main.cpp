@@ -6,7 +6,10 @@
 #include "../../include/fdes_b200.h"
 #include "params.h"
 #include "emd.h"
+#include <fcntl.h>
 #include <getopt.h>
+#include <sys/mman.h>
+#include <unistd.h>
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>
@@ -20,6 +23,8 @@ int main(int argc, char** argv)
     std::string input = "dataFDES.cnf", image = "Measurements.bin", emd = "results.emd";
     int gpu_index = 0, print_level = 0;
     bool stem_scan = false;
+    std::string stem_4d;
+    int stem_4d_bin = 1;
     std::string gpus_spec;
     static struct option opts[] = {{"gpu_index", required_argument, 0, 0},
                                    {"input_name", required_argument, 0, 0},
@@ -30,6 +35,8 @@ int main(int argc, char** argv)
                                    {"version", no_argument, 0, 0},
                                    {"stem_scan", no_argument, 0, 0},   // extension, see below
                                    {"gpus", required_argument, 0, 0},  // extension: shard the run over several GPUs
+                                   {"stem_4d", required_argument, 0, 0},       // extension: 4D-STEM data set of --stem_scan
+                                   {"stem_4d_bin", required_argument, 0, 0},
                                    {NULL, 0, 0, 0}};
     while (true) {
         int idx = 0;
@@ -60,10 +67,16 @@ int main(int argc, char** argv)
                         "  [ --gpus        extension: <count> (gpu_index, gpu_index + 1, ...) or a list i,j,... -- frozen-phonon\n"
                         "                  configurations, tilt/defocus series or STEM probes are sharded over these GPUs ]\n"
                         "  [ --stem_scan   extension: run the probe scan a `mode: STEM` .qsc describes (scan_* and\n"
-                        "                  detector: keys); image_name receives float32 [detector][x][y] ]\n");
+                        "                  detector: keys); image_name receives float32 [detector][x][y] ]\n"
+                        "  [ --stem_4d     extension, with --stem_scan: <path> receives the diffraction pattern of every probe\n"
+                        "                  of the same scan, raw float32 [x][y][qy][qx]: fftshifted, cropped to the smallest\n"
+                        "                  centred window that holds the band limit, binned; image_name as without it ]\n"
+                        "  [ --stem_4d_bin <b>: pattern pixels summed b x b (default 1) ]\n");
                 return EXIT_FAILURE;
             case 7: stem_scan = true; break;
             case 8: gpus_spec = optarg; break;
+            case 9: stem_4d = optarg; break;
+            case 10: stem_4d_bin = atoi(optarg); break;
             case 6: fprintf(stderr, " \n FDES (fdes_b200) Version : %1.1f  \n", fdes_b200_version() / 100.0); return EXIT_FAILURE;
         }
     }
@@ -91,6 +104,7 @@ int main(int argc, char** argv)
     const char* spec = !gpus_spec.empty() ? gpus_spec.c_str() : getenv("FDES_B200_GPUS");
     std::vector<int> gpus((size_t)std::max(1, fdes_b200_parse_gpu_list(spec, gpu_index, nullptr, 0)));
     fdes_b200_parse_gpu_list(spec, gpu_index, gpus.data(), (int)gpus.size());
+    if (!stem_4d.empty() && !stem_scan) { fprintf(stderr, " \n --stem_4d needs --stem_scan \n"); return EXIT_FAILURE; }
     if (stem_scan) {
         // Extension (FDES has no STEM mode): the raster and detectors of a QSTEM `mode: STEM` file, keys the
         // reference parses and drops (src/rwQsc.cu:444-466, 698-735), drive the batched probe scan.
@@ -105,7 +119,31 @@ int main(int argc, char** argv)
         fdes_b200_qsc_scan(input.c_str(), nxy, xy.data(), np, det.data(), ndet);
         fdes_b200_sim* sim = fdes_b200_open_multi(input.c_str(), nullptr, 0, gpus.data(), (int)gpus.size(), 37, 0);   // 37 probes per launch: whole waves of 148 SMs at 512^2
         if (!sim) { fprintf(stderr, " \n fdes_b200: %s \n", fdes_b200_last_error()); return EXIT_FAILURE; }
-        const double ms = fdes_b200_stem_scan(sim, 0, np, xy.data(), ndet, det.data(), sig.data());
+        double ms = 0.0;
+        if (stem_4d.empty()) {
+            ms = fdes_b200_stem_scan(sim, 0, np, xy.data(), ndet, det.data(), sig.data());
+        } else {
+            // the data set goes straight into the mapped output file: [x][y][qy][qx], probe i = x * ny + y
+            int dims[10];
+            fdes_b200_get_dims(sim, dims);
+            const int side = fdes_b200_stem_4d_side(dims[3], 0, stem_4d_bin);
+            if (side < 0) { fprintf(stderr, " \n fdes_b200: --stem_4d_bin: %s \n", fdes_b200_last_error()); return EXIT_FAILURE; }
+            const size_t bytes = (size_t)np * side * side * sizeof(float);
+            const int fd = open(stem_4d.c_str(), O_RDWR | O_CREAT | O_TRUNC, 0644);
+            void* map = MAP_FAILED;
+            if (fd >= 0 && ftruncate(fd, (off_t)bytes) == 0) map = mmap(nullptr, bytes, PROT_READ | PROT_WRITE, MAP_SHARED, fd, 0);
+            if (map == MAP_FAILED) {
+                fprintf(stderr, " \n fdes_b200: cannot write %s \n", stem_4d.c_str());
+                return EXIT_FAILURE;
+            }
+            ms = fdes_b200_stem_scan_4d(sim, 0, np, xy.data(), 0, stem_4d_bin, ndet, det.data(), 0, static_cast<float*>(map), sig.data());
+            const bool synced = msync(map, bytes, MS_SYNC) == 0;
+            munmap(map, bytes);
+            if (close(fd) != 0 || !synced) {
+                fprintf(stderr, " \n fdes_b200: cannot write %s \n", stem_4d.c_str());
+                return EXIT_FAILURE;
+            }
+        }
         if (ms < 0) { fprintf(stderr, " \n fdes_b200: %s \n", fdes_b200_last_error()); return EXIT_FAILURE; }
         for (int i = 0; i < np; i++)
             for (int d = 0; d < ndet; d++) out[(size_t)d * np + i] = sig[(size_t)i * ndet + d];   // [probe][det] -> [det][x][y]

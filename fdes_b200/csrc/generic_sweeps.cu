@@ -468,6 +468,26 @@ __global__ void __launch_bounds__(GT) g_detector_cols(const cpx* Psi, float* par
         __syncthreads();
     }
 }
+// 4D-STEM (see k_detector4d_cols): the window pixels of the L columns, stored from the line buffers row by row
+__global__ void __launch_bounds__(GT) g_detector4d_cols(const cpx* Psi, float* scratch, int Q, int L, GPlan pl, const cpx* W)
+{
+    extern __shared__ cpx gsm[];
+    const int N = pl.N, kx0 = blockIdx.x * L, o = (N - Q) / 2;
+    bool any = false;
+    for (int l = 0; l < L; l++) any |= (unsigned)((kx0 + l + N / 2) % N - o) < (unsigned)Q;
+    if (!any) return;                              // CTA-uniform
+    cpx *x = gsm, *y = gsm + L * N;
+    const cpx* tile = Psi + (size_t)blockIdx.y * N * N + kx0;
+    g_foreach<true>(N, L, [&](int i, int l) { x[l * N + i] = tile[gaddr<true>(i, l, N)]; });
+    __syncthreads();
+    g_fft(x, y, pl, L, W, -1);
+    float* out = scratch + (size_t)blockIdx.y * Q * Q;
+    g_foreach<true>(N, L, [&](int i, int l) {
+        const int qx = (kx0 + l + N / 2) % N - o, qy = (i + N / 2) % N - o;
+        const cpx v = x[l * N + i];
+        if ((unsigned)qx < (unsigned)Q && (unsigned)qy < (unsigned)Q) out[(size_t)qy * Q + qx] = v.x * v.x + v.y * v.y;
+    });
+}
 __global__ void g_detector_finish(const float* partial, float* out, int ntiles, int ndet, int batch, float weight)
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -619,6 +639,18 @@ void gen_detector_cols(const SweepGeom& g, const cpx* Psi, float* partial, float
     g_detector_finish<<<(n + 127) / 128, 128, 0, st>>>(partial, out, tiles, rings.n, batch, weight);
     GEN_LAUNCHED();
 }
+void gen_detector4d_cols(const SweepGeom& g, const cpx* Psi, float* scratch, float* out, int Q, int bin, float weight, int batch,
+                         cudaStream_t st)
+{
+    check_geom(g);
+    const int L = col_width(g.N, 2);
+    const size_t sm = 2 * (size_t)L * g.N * sizeof(cpx);
+    allow(g_detector4d_cols, sm);
+    g_detector4d_cols<<<dim3(g.N / L, batch), GT, sm, st>>>(Psi, scratch, Q, L, make_plan(g.N), g.tw);
+    GEN_LAUNCHED();
+    launch_detector4d_finish(scratch, out, Q, bin, weight, batch, st);
+    GEN_LAUNCHED();
+}
 // W[k] = exp(-2 pi i k / N), exact on the axes: N float32 pairs, followed by the same N values as double
 // pairs (2 cpx slots each) for the long direct DFTs of g_fft
 std::vector<cpx> gen_twiddles(int N)
@@ -651,7 +683,7 @@ const SweepVTable* generic_sweep_vtable()
 {
     static const SweepVTable vt = {0, 1, 1, 0, &gen_density_rows, &gen_potential_cols, &gen_transmit_rows, &gen_bandlimit_cols, &gen_multiply_rows,
                                    &gen_propagate_cols, &gen_rows_fft, &gen_rows_fft_sum, &gen_cols_fft, &gen_probe_cols, &gen_detector_tiles,
-                                   &gen_detector_cols, &gen_twiddles, nullptr, false};
+                                   &gen_detector_cols, &gen_detector4d_cols, &gen_twiddles, nullptr, false};
     return &vt;
 }
 

@@ -89,6 +89,14 @@ void launch_probe_cols(const SweepGeom& g, cpx* Psi, const cpx* PSI0, const floa
 int detector_tiles(const SweepGeom& g);
 void launch_detector_cols(const SweepGeom& g, const cpx* Psi, float* partial, float* out, const DetectorRings& rings,
                           float d1, float d2, float weight, int batch, cudaStream_t st);
+// 4D-STEM: out[b][y][x] += weight * (sum of the bin x bin pixels (y, x) of the diffraction intensity of Psi[b],
+// fftshifted and cropped to the centred window [o, o + Q)^2, o = (N - Q) / 2); out is [batch][Q/bin][Q/bin].
+// scratch: [batch][Q][Q] floats, zero in the columns outside the band (the sweep writes the band columns only).
+// Q = N (mod 2), bin divides Q, 1 <= Q <= N (stem4d_window, engine.h).
+void launch_detector4d_cols(const SweepGeom& g, const cpx* Psi, float* scratch, float* out, int Q, int bin, float weight,
+                            int batch, cudaStream_t st);
+// the finish of launch_detector4d_cols: the bins of scratch summed in a fixed order (row by row) onto out
+void launch_detector4d_finish(const float* scratch, float* out, int Q, int bin, float weight, int batch, cudaStream_t st);
 
 // ---- generic sweeps used outside the slice loop ------------------------------------------
 enum RowEpilogue {

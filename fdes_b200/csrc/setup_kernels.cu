@@ -193,6 +193,27 @@ static int grid_for(size_t n) { size_t g = (n + 255) / 256; return (int)(g > 148
 void launch_fill_cpx(cpx* p, size_t n, cpx v, cudaStream_t st) { k_fill_cpx<<<grid_for(n), 256, 0, st>>>(p, n, v); }
 void launch_fill_f32(float* p, size_t n, float v, cudaStream_t st) { k_fill_f32<<<grid_for(n), 256, 0, st>>>(p, n, v); }
 
+// out[b][y][x] += weight * sum of scratch[b][y*bin + r][x*bin + c], r outer, c inner: bins straddle the CTAs of the
+// detector sweep, so they are summed here, one thread per output pixel, without atomics
+__global__ void k_detector4d_finish(const float* __restrict__ scratch, float* __restrict__ out, int Q, int bin, float weight,
+                                    size_t n)
+{
+    const int S = Q / bin;
+    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+        const int x = (int)(i % S), y = (int)((i / S) % S);
+        const float* src = scratch + (i / ((size_t)S * S)) * Q * Q + (size_t)y * bin * Q + (size_t)x * bin;
+        float s = 0.f;
+        for (int r = 0; r < bin; r++)
+            for (int c = 0; c < bin; c++) s += src[(size_t)r * Q + c];
+        out[i] += weight * s;
+    }
+}
+void launch_detector4d_finish(const float* scratch, float* out, int Q, int bin, float weight, int batch, cudaStream_t st)
+{
+    const size_t n = (size_t)batch * (Q / bin) * (Q / bin);
+    k_detector4d_finish<<<grid_for(n), 256, 0, st>>>(scratch, out, Q, bin, weight, n);
+}
+
 __global__ void k_plane_wave_rowspace(cpx* Psi, int N, size_t n)
 {
     for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)

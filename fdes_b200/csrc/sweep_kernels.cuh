@@ -1539,6 +1539,56 @@ void launch_detector_cols_n(const SweepGeom& g, const cpx* Psi, float* partial, 
     FDES_LAUNCH_CHECK();
 }
 
+// 4D-STEM: scratch[b][qy][qx] = |FFT_col(Psi_b)|^2 at the window pixel (qy, qx) of the fftshifted pattern, for the
+// band columns inside the window [o, o + Q)^2, o = (N - Q) / 2 (the other pixels are not written).  A thread holds
+// rows ky = theta + m*T of one column; the CTA's [N][CW] intensities go through shared memory, so that each
+// window row is stored as CW consecutive floats.
+template <int N>
+__global__ void __launch_bounds__(ColCfg<N>::THREADS, ColCfg<N>::MIN_CTAS)
+k_detector4d_cols(const cpx* __restrict__ Psi, float* __restrict__ scratch, int Q, int lo_end, int hi_start,
+                  const cpx* __restrict__ tw)
+{
+    using C = ColCfg<N>;
+    extern __shared__ cpx smem[];
+    constexpr int E = C::E, CWP = C::CW + 1;     // odd row stride: the T rows of a column hit distinct banks
+    const int o = (N - Q) / 2;
+    const int kx0 = band_col0(blockIdx.x * C::CW, lo_end, hi_start);
+    bool any = false;
+    for (int l = 0; l < C::CW; l++) any |= (unsigned)((kx0 + l + N / 2) % N - o) < (unsigned)Q;
+    if (!any) return;                              // no column of this tile inside the window (CTA-uniform)
+    const ColCtx<N> ctx(smem);
+    const int theta = ctx.theta;
+    cpx x[E];
+    ctx.load(x, Psi + (size_t)blockIdx.y * N * N + kx0, KeepAll());
+    fft_line<N, E, -1>(x, ctx.sm, theta, tw, ctx);
+    __syncthreads();
+    float* st = reinterpret_cast<float*>(smem);
+#pragma unroll
+    for (int m = 0; m < E; m++) st[(theta + m * C::T) * CWP + ctx.line] = x[m].x * x[m].x + x[m].y * x[m].y;
+    __syncthreads();
+    float* out = scratch + (size_t)blockIdx.y * Q * Q;
+    for (int w = threadIdx.x; w < Q * C::CW; w += C::THREADS) {
+        const int qy = w / C::CW, l = w % C::CW;
+        const int qx = (kx0 + l + N / 2) % N - o;
+        const int ky = (qy + o + N - N / 2) % N;  // inverse of the shift (ky + N/2) % N
+        if ((unsigned)qx < (unsigned)Q) out[(size_t)qy * Q + qx] = st[ky * CWP + l];
+    }
+}
+
+template <int NN>
+void launch_detector4d_cols_n(const SweepGeom& g, const cpx* Psi, float* scratch, float* out, int Q, int bin, float weight,
+                              int batch, cudaStream_t st)
+{
+    using C = ColCfg<NN>;
+    static_assert((size_t)NN * (C::CW + 1) * sizeof(float) <= C::SMEM, "intensity tile must fit the line buffers");
+    FDES_ALLOW_SMEM((k_detector4d_cols<NN>), C::SMEM);
+    dim3 grid(band_cols(g) / C::CW, batch);
+    k_detector4d_cols<NN><<<grid, C::THREADS, C::SMEM, st>>>(Psi, scratch, Q, g.lo_end, g.hi_start, g.tw);
+    FDES_LAUNCH_CHECK();
+    launch_detector4d_finish(scratch, out, Q, bin, weight, batch, st);
+    FDES_LAUNCH_CHECK();
+}
+
 // ---------------------------------------------------------------------------------------------
 // twiddle tables (layout: fft_core.cuh) and geometry queries
 // ---------------------------------------------------------------------------------------------
@@ -1598,7 +1648,7 @@ const SweepVTable* make_sweep_vtable()
         &launch_density_rows_n<N>, &launch_potential_cols_n<N>, &launch_transmit_rows_n<N>,
         &launch_bandlimit_cols_n<N>, &launch_multiply_rows_n<N>, &launch_propagate_cols_n<N>,
         &launch_rows_fft_n<N>, &launch_rows_fft_sum_n<N>, &launch_cols_fft_n<N>,
-        &launch_probe_cols_n<N>, &detector_tiles_n<N>, &launch_detector_cols_n<N>,
+        &launch_probe_cols_n<N>, &detector_tiles_n<N>, &launch_detector_cols_n<N>, &launch_detector4d_cols_n<N>,
         &make_twiddles_n<N>, propagate_cols_from_entry<N>(), pipe_supported<N>(),
     };
     return &vt;

@@ -31,6 +31,7 @@ struct SweepVTable {
     void (*probe_cols)(const SweepGeom&, cpx*, const cpx*, const float*, int, cudaStream_t);
     int (*detector_tiles)(const SweepGeom&);
     void (*detector_cols)(const SweepGeom&, const cpx*, float*, float*, const DetectorRings&, float, float, float, int, cudaStream_t);
+    void (*detector4d_cols)(const SweepGeom&, const cpx*, float*, float*, int, int, float, int, cudaStream_t);
     std::vector<cpx> (*make_twiddles)(int N);
     // null where pipelined is false: S6 reading another image stack, see launch_propagate_cols_from
     void (*propagate_cols_from)(const SweepGeom&, cpx*, const cpx*, int, int, const cpx*, int, bool, const cpx*, cudaStream_t);

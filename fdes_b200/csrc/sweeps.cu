@@ -117,5 +117,13 @@ void launch_detector_cols(const SweepGeom& g, const cpx* Psi, float* partial, fl
 {
     vt(g.N).detector_cols(g, Psi, partial, out, rings, d1, d2, weight, batch, st);
 }
+void launch_detector4d_cols(const SweepGeom& g, const cpx* Psi, float* scratch, float* out, int Q, int bin, float weight,
+                            int batch, cudaStream_t st)
+{
+    if (Q < 1 || Q > g.N || (Q - g.N) % 2 != 0 || bin < 1 || Q % bin != 0)
+        throw std::runtime_error("4D-STEM window " + std::to_string(Q) + " / bin " + std::to_string(bin) + " not admissible at N = " +
+                                 std::to_string(g.N));
+    vt(g.N).detector4d_cols(g, Psi, scratch, out, Q, bin, weight, batch, st);
+}
 
 }  // namespace fdes

@@ -136,6 +136,28 @@ int fdes_b200_potential(fdes_b200_sim* sim, float* out_host);
 double fdes_b200_stem_scan(fdes_b200_sim* sim, int k, int nprobes, const float* xy_host, int ndet,
                            const float* det_mrad_host, float* out_host);
 
+/* 4D-STEM scan (extension): the diffraction pattern of every probe position instead of ring sums.  Positions,
+ * units and frame as fdes_b200_stem_scan.  Pattern p is I_p = |FFT2 psi_p|^2 / N^2 (diffractionPattern,
+ * src/crystalMaker.cu:700-718) averaged over the frozen-phonon configurations with weight 1/count, in the
+ * reference's fftshift frame (out[(i + N/2) mod N] = in[i]), cropped to the centred window [o, o + Q)^2 with
+ * o = (N - Q) / 2 and binned bin x bin by summation: patterns_host [nprobes][Q/bin][Q/bin] float32, qx fastest;
+ * window pixel (qy, qx) holds the frequency (qx - Q/2, qy - Q/2) (integer division), the zero frequency sits at
+ * [Q/2][Q/2] before binning.  window: Q, with Q = N (mod 2), bin dividing Q and 1 <= Q <= N; 0 = the smallest such Q
+ * that holds every frequency the 2/3 band limit keeps (nothing of the pattern is lost, an empty specimen sums to
+ * n1*n2).  fdes_b200_stem_4d_side gives Q/bin.
+ * ndet (0..8) annular detectors as in fdes_b200_stem_scan run in the same pass: det_out_host [nprobes][ndet],
+ * bitwise the signals fdes_b200_stem_scan returns (NULL allowed when ndet = 0).
+ * The raster runs in passes of probes_per_pass probes (0 = automatic: the two device pass buffers take at most
+ * about a quarter of the free device memory); a finished pass is copied to patterns_host while the next one
+ * computes.  Results do not depend on the pass size, the batch size or the number of GPUs the probes are dealt
+ * out to; with frozen-phonon configurations sharded over GPUs the passes of the devices are summed on the host in
+ * device order.  Returns the CUDA-event milliseconds of the device loop (negative on failure). */
+double fdes_b200_stem_scan_4d(fdes_b200_sim* sim, int k, int nprobes, const float* xy_host, int window, int bin, int ndet,
+                              const float* det_mrad_host, int probes_per_pass, float* patterns_host, float* det_out_host);
+/* Host-only (no CUDA call): the side Q/bin of the 4D-STEM patterns on an N x N grid for window / bin as
+ * fdes_b200_stem_scan_4d takes them, -1 with the reason in fdes_b200_last_error() when they are not admissible. */
+int fdes_b200_stem_4d_side(int N, int window, int bin);
+
 /* Host-only: the scan raster and detectors a QSTEM `mode: STEM` .qsc describes -- the keys readQsc
  * parses (scan_x_start/stop/pixels, scan_y_*, src/rwQsc.cu:444-466; `detector: inner outer name ..`
  * [mrad], :698-735) but FDES never uses -- in the form fdes_b200_stem_scan takes: nxy[2] = pixels in
@@ -217,7 +239,11 @@ int fdes_b200_sort_records(unsigned int* keys, int* cols, float* w, int n, int n
  *   FDES_B200_SWEEP_DETECTOR  ndet (1..8)                                   d1 d2   Psi [batch], out [batch][ndet]
  *                                                                           weight  (accumulated into); partial
  *                                                                           in2[ndet] sums start as NaN
- *                                                                           out2[ndet] */
+ *                                                                           out2[ndet]
+ *   FDES_B200_SWEEP_DETECTOR4D Q bin                                        weight  Psi [batch], out [batch][Q/bin]
+ *                                                                                   [Q/bin] (accumulated into); the
+ *                                                                                   [batch][Q][Q] scratch starts as
+ *                                                                                   NaN in the band columns */
 #define FDES_B200_SWEEP_GEOM 0
 #define FDES_B200_SWEEP_DENSITY 1
 #define FDES_B200_SWEEP_POTENTIAL 2
@@ -231,6 +257,7 @@ int fdes_b200_sort_records(unsigned int* keys, int* cols, float* w, int n, int n
 #define FDES_B200_SWEEP_ROWS_FFT 10
 #define FDES_B200_SWEEP_PROBE 11
 #define FDES_B200_SWEEP_DETECTOR 12
+#define FDES_B200_SWEEP_DETECTOR4D 13
 int fdes_b200_sweep_test(int op, int N, int batch, const int* iargs, int n_iargs, const float* fargs, int n_fargs,
                          float** bufs, const long long* buf_elems, int nbufs, int gpu_index, int pipe_ctas,
                          int* pipe_grid_out);
