@@ -23,7 +23,7 @@ __global__ void k_rot(float* xyz, int nAt, int axA, int axB, float c, float s)
 }
 void launch_rot(float* xyz, int nAt, int axA, int axB, float c, float s, cudaStream_t st)
 {
-    k_rot<<<(nAt + 255) / 256, 256, 0, st>>>(xyz, nAt, axA, axB, c, s);
+    launch(k_rot, (nAt + 255) / 256, 256, 0, st, xyz, nAt, axA, axB, c, s);
 }
 
 size_t rng_state_bytes() { return sizeof(curandState); }
@@ -35,7 +35,7 @@ __global__ void k_rng_init(curandState* state, int n, unsigned long long seed)
 }
 void launch_rng_init(void* states, int n, unsigned long long seed, cudaStream_t st)
 {
-    k_rng_init<<<(n + 127) / 128, 128, 0, st>>>(static_cast<curandState*>(states), n, seed);
+    launch(k_rng_init, (n + 127) / 128, 128, 0, st, static_cast<curandState*>(states), n, seed);
 }
 
 // atomJitter_d, src/crystalMaker.cu:37-48 (out-of-place so the equilibrium copy stays intact).
@@ -61,8 +61,8 @@ __global__ void k_atom_jitter(float* __restrict__ out, const float* __restrict__
 void launch_atom_jitter(float* xyz_out, const float* xyz_in, const float* dwf, int nAt,
                         void* states, long long burn, int nconf, cudaStream_t st)
 {
-    k_atom_jitter<<<(3 * nAt + 127) / 128, 128, 0, st>>>(xyz_out, xyz_in, dwf, nAt,
-                                                        static_cast<curandState*>(states), burn, nconf);
+    launch(k_atom_jitter, (3 * nAt + 127) / 128, 128, 0, st, xyz_out, xyz_in, dwf, nAt, static_cast<curandState*>(states), burn,
+           nconf);
 }
 
 // ascombeNoise_d, src/crystalMaker.cu:50-70: Poisson noise via the Anscombe transform
@@ -84,7 +84,7 @@ __global__ void k_anscombe_noise(cpx* f, size_t n, float dose, curandState* stat
 }
 void launch_anscombe_noise(cpx* f, size_t n, float dose, void* states, cudaStream_t st)
 {
-    k_anscombe_noise<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(f, n, dose, static_cast<curandState*>(states));
+    launch(k_anscombe_noise, (unsigned)((n + 127) / 128), 128, 0, st, f, n, dose, static_cast<curandState*>(states));
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -146,7 +146,7 @@ void launch_bin_atoms(const float* xyz, const int* zidx, const float* occ, int n
                       const BinGeom& bg, uint32_t* keys, int* cols, float* w, int* bins_out,
                       int nconf, cudaStream_t st)
 {
-    k_bin_atoms<<<dim3((nAt + 255) / 256, nconf), 256, 0, st>>>(xyz, zidx, occ, nAt, bg, keys, cols, w, bins_out);
+    launch(k_bin_atoms, dim3((nAt + 255) / 256, nconf), 256, 0, st, xyz, zidx, occ, nAt, bg, keys, cols, w, bins_out);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -253,9 +253,9 @@ void launch_radix_sort(const SortBuffers& sb, int n, int key_bits, int nconf, cu
     if (passes == 0) passes = 2;
     for (int p = 0; p < passes; p++) {
         const int shift = 8 * p;
-        k_sort_hist<<<dim3(nb, nconf), SORT_THREADS, 0, st>>>(ki, n, shift, sb.hist, nb);
-        k_sort_scan<<<dim3(1, nconf), 1024, 0, st>>>(sb.hist, 256 * nb);
-        k_sort_scatter<<<dim3(nb, nconf), SORT_THREADS, 0, st>>>(ki, ci, wi, ko, co, wo, n, shift, sb.hist, nb);
+        launch(k_sort_hist, dim3(nb, nconf), SORT_THREADS, 0, st, ki, n, shift, sb.hist, nb);
+        launch(k_sort_scan, dim3(1, nconf), 1024, 0, st, sb.hist, 256 * nb);
+        launch(k_sort_scatter, dim3(nb, nconf), SORT_THREADS, 0, st, ki, ci, wi, ko, co, wo, n, shift, sb.hist, nb);
         uint32_t* tk = ki; ki = ko; ko = tk;
         int* tc = ci; ci = co; co = tc;
         float* tw2 = wi; wi = wo; wo = tw2;
@@ -279,7 +279,7 @@ __global__ void k_row_pointers(const uint32_t* __restrict__ keys, int n, int* __
 void launch_row_pointers(const uint32_t* keys_sorted, int n, int* rowptr, int nkeys, int nconf, cudaStream_t st, size_t rp_stride)
 {
     if (rp_stride == 0) rp_stride = (size_t)nkeys + 1;
-    k_row_pointers<<<dim3((nkeys + 1 + 255) / 256, nconf), 256, 0, st>>>(keys_sorted, n, rowptr, nkeys, rp_stride);
+    launch(k_row_pointers, dim3((nkeys + 1 + 255) / 256, nconf), 256, 0, st, keys_sorted, n, rowptr, nkeys, rp_stride);
 }
 
 // one thread per mask word (kernels.cuh: launch_row_masks)
@@ -301,7 +301,7 @@ __global__ void k_row_masks(int* __restrict__ rowptr, size_t rp_stride, int nkey
 void launch_row_masks(int* rowptr, size_t rp_stride, int nkeys, int N, int E, int nconf, cudaStream_t st)
 {
     const int nwords = (nkeys / N) * (N / E);
-    k_row_masks<<<dim3((nwords + 255) / 256, nconf), 256, 0, st>>>(rowptr, rp_stride, nkeys, N, E);
+    launch(k_row_masks, dim3((nwords + 255) / 256, nconf), 256, 0, st, rowptr, rp_stride, nkeys, N, E);
 }
 
 }  // namespace fdes

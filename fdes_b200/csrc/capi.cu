@@ -451,31 +451,26 @@ int fdes_b200_get_counters(fdes_b200_sim* sim, long long* c, int reset)
     API_CATCH(-1)
 }
 
-static void ck(cudaError_t e, const char* what)
-{
-    if (e != cudaSuccess) throw std::runtime_error(std::string(what) + ": " + cudaGetErrorString(e));
-}
-
 int fdes_b200_fft2d(float* data_host, int N, int dir, int gpu_index)
 {
     API_TRY
     if (!fft_size_supported(N)) throw std::runtime_error("unsupported FFT size");
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) throw std::runtime_error("no CUDA device");
-    ck(cudaSetDevice(gpu_index), "cudaSetDevice");
+    CK(cudaSetDevice(gpu_index));
     const size_t NN = (size_t)N * N;
     cpx *d = nullptr, *tw = nullptr;
-    ck(cudaMalloc(&d, NN * sizeof(cpx)), "cudaMalloc");
+    CK(cudaMalloc(&d, NN * sizeof(cpx)));
     const std::vector<cpx> h = make_twiddles(N);
-    ck(cudaMalloc(&tw, h.size() * sizeof(cpx)), "cudaMalloc");
-    ck(cudaMemcpy(tw, h.data(), h.size() * sizeof(cpx), cudaMemcpyHostToDevice), "cudaMemcpy");
-    ck(cudaMemcpy(d, data_host, NN * sizeof(cpx), cudaMemcpyHostToDevice), "cudaMemcpy");
+    CK(cudaMalloc(&tw, h.size() * sizeof(cpx)));
+    CK(cudaMemcpy(tw, h.data(), h.size() * sizeof(cpx), cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(d, data_host, NN * sizeof(cpx), cudaMemcpyHostToDevice));
     SweepGeom g{N, N, N, tw};
     RowOpts ro;
     launch_rows_fft(g, d, d, dir, ROW_STORE, ro, 1, 0);
     launch_cols_fft(g, d, d, dir, COL_PLAIN, nullptr, 1.f, 1, 0);
-    ck(cudaDeviceSynchronize(), "fft2d kernels");
-    ck(cudaMemcpy(data_host, d, NN * sizeof(cpx), cudaMemcpyDeviceToHost), "cudaMemcpy");
+    CK(cudaDeviceSynchronize());
+    CK(cudaMemcpy(data_host, d, NN * sizeof(cpx), cudaMemcpyDeviceToHost));
     cudaFree(d); cudaFree(tw);
     return 0;
     API_CATCH(-1)
@@ -487,27 +482,27 @@ int fdes_b200_sort_records(unsigned int* keys, int* cols, float* w, int n, int n
     API_TRY
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) throw std::runtime_error("no CUDA device");
-    ck(cudaSetDevice(gpu_index), "cudaSetDevice");
+    CK(cudaSetDevice(gpu_index));
     SortBuffers sb{};
     int* rp = nullptr;
     const size_t nn = (size_t)std::max(n, 1);
-    ck(cudaMalloc(&sb.keys, nn * 4), "cudaMalloc"); ck(cudaMalloc(&sb.keys_tmp, nn * 4), "cudaMalloc");
-    ck(cudaMalloc(&sb.cols, nn * 4), "cudaMalloc"); ck(cudaMalloc(&sb.cols_tmp, nn * 4), "cudaMalloc");
-    ck(cudaMalloc(&sb.w, nn * 4), "cudaMalloc"); ck(cudaMalloc(&sb.w_tmp, nn * 4), "cudaMalloc");
-    ck(cudaMalloc(&sb.hist, 256 * (size_t)sort_num_blocks(n) * 4), "cudaMalloc");
-    ck(cudaMalloc(&rp, ((size_t)nkeys + 1) * 4), "cudaMalloc");
-    ck(cudaMemcpy(sb.keys, keys, (size_t)n * 4, cudaMemcpyHostToDevice), "cudaMemcpy");
-    ck(cudaMemcpy(sb.cols, cols, (size_t)n * 4, cudaMemcpyHostToDevice), "cudaMemcpy");
-    ck(cudaMemcpy(sb.w, w, (size_t)n * 4, cudaMemcpyHostToDevice), "cudaMemcpy");
+    CK(cudaMalloc(&sb.keys, nn * 4)); CK(cudaMalloc(&sb.keys_tmp, nn * 4));
+    CK(cudaMalloc(&sb.cols, nn * 4)); CK(cudaMalloc(&sb.cols_tmp, nn * 4));
+    CK(cudaMalloc(&sb.w, nn * 4)); CK(cudaMalloc(&sb.w_tmp, nn * 4));
+    CK(cudaMalloc(&sb.hist, 256 * (size_t)sort_num_blocks(n) * 4));
+    CK(cudaMalloc(&rp, ((size_t)nkeys + 1) * 4));
+    CK(cudaMemcpy(sb.keys, keys, (size_t)n * 4, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(sb.cols, cols, (size_t)n * 4, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(sb.w, w, (size_t)n * 4, cudaMemcpyHostToDevice));
     int bits = 0;
     while ((1LL << bits) <= (long long)nkeys) bits++;
     launch_radix_sort(sb, n, bits, 1, 0);
     launch_row_pointers(sb.keys, n, rp, nkeys, 1, 0);
-    ck(cudaDeviceSynchronize(), "sort kernels");
-    ck(cudaMemcpy(keys, sb.keys, (size_t)n * 4, cudaMemcpyDeviceToHost), "cudaMemcpy");
-    ck(cudaMemcpy(cols, sb.cols, (size_t)n * 4, cudaMemcpyDeviceToHost), "cudaMemcpy");
-    ck(cudaMemcpy(w, sb.w, (size_t)n * 4, cudaMemcpyDeviceToHost), "cudaMemcpy");
-    ck(cudaMemcpy(rowptr, rp, ((size_t)nkeys + 1) * 4, cudaMemcpyDeviceToHost), "cudaMemcpy");
+    CK(cudaDeviceSynchronize());
+    CK(cudaMemcpy(keys, sb.keys, (size_t)n * 4, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(cols, sb.cols, (size_t)n * 4, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(w, sb.w, (size_t)n * 4, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(rowptr, rp, ((size_t)nkeys + 1) * 4, cudaMemcpyDeviceToHost));
     cudaFree(sb.keys); cudaFree(sb.keys_tmp); cudaFree(sb.cols); cudaFree(sb.cols_tmp);
     cudaFree(sb.w); cudaFree(sb.w_tmp); cudaFree(sb.hist); cudaFree(rp);
     return 0;
@@ -530,7 +525,7 @@ struct DeviceAllocs {
     void* get(size_t bytes)
     {
         void* q = nullptr;
-        ck(cudaMalloc(&q, std::max<size_t>(bytes, 4)), "cudaMalloc");
+        CK(cudaMalloc(&q, std::max<size_t>(bytes, 4)));
         p.push_back(q);
         return q;
     }
@@ -558,8 +553,8 @@ RecordRows upload_row_pointers(DeviceAllocs& da, const int* rp_host, int nconf, 
     r.mask_off = E > 0 ? nkeys + 1 : 0;
     r.dev = static_cast<int*>(da.get((size_t)nconf * r.stride * sizeof(int)));
     for (int c = 0; c < nconf; c++)
-        ck(cudaMemcpyAsync(r.dev + (size_t)c * r.stride, rp_host + (size_t)c * (nkeys + 1), ((size_t)nkeys + 1) * sizeof(int),
-                           cudaMemcpyHostToDevice, st), "cudaMemcpyAsync");
+        CK(cudaMemcpyAsync(r.dev + (size_t)c * r.stride, rp_host + (size_t)c * (nkeys + 1), ((size_t)nkeys + 1) * sizeof(int),
+                           cudaMemcpyHostToDevice, st));
     if (E > 0) launch_row_masks(r.dev, r.stride, nkeys, N, E, nconf, st);
     return r;
 }
@@ -608,7 +603,7 @@ int fdes_b200_sweep_test(int op, int N, int batch, const int* iargs, int n_iargs
     if (batch < 1) throw std::runtime_error("sweep test: batch must be >= 1");
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) throw std::runtime_error("no CUDA device");
-    ck(cudaSetDevice(gpu_index), "cudaSetDevice");
+    CK(cudaSetDevice(gpu_index));
     const size_t NN = (size_t)N * N, IMG = 2 * NN, Q = (size_t)(N / 2 + 1);
     for (int i = 0; i < nbufs; i++)
         if (buf_elems[i] < 0 || (buf_elems[i] > 0 && !bufs[i])) throw std::runtime_error("sweep test: bad buffer");
@@ -616,11 +611,11 @@ int fdes_b200_sweep_test(int op, int N, int batch, const int* iargs, int n_iargs
     DeviceAllocs da;
     // the sweeps run as in the engine: on a non-blocking stream, launched with programmatic serialisation; every
     // copy of this call is queued on the same stream, so the row masks and the sweep see the uploaded data
-    ck(cudaStreamCreateWithFlags(&da.st, cudaStreamNonBlocking), "cudaStreamCreate");
+    CK(cudaStreamCreateWithFlags(&da.st, cudaStreamNonBlocking));
     const cudaStream_t st = da.st;
     const std::vector<cpx> twh = make_twiddles(N);
     cpx* tw = static_cast<cpx*>(da.get(twh.size() * sizeof(cpx)));
-    ck(cudaMemcpyAsync(tw, twh.data(), twh.size() * sizeof(cpx), cudaMemcpyHostToDevice, st), "cudaMemcpyAsync");
+    CK(cudaMemcpyAsync(tw, twh.data(), twh.size() * sizeof(cpx), cudaMemcpyHostToDevice, st));
     SweepGeom g = make_sweep_geom(N, tw, 0);
     // row pointers of S1 / S2 (buffer rp_buf) go up in the engine's layout, not word for word
     int rp_buf = -1, nconf = 0, nkeys = 0;
@@ -650,7 +645,7 @@ int fdes_b200_sweep_test(int op, int N, int batch, const int* iargs, int n_iargs
     for (int i = 0; i < nbufs; i++) {
         if (i == rp_buf || buf_elems[i] == 0) continue;
         d[i] = static_cast<float*>(da.get((size_t)buf_elems[i] * 4));
-        ck(cudaMemcpyAsync(d[i], bufs[i], (size_t)buf_elems[i] * 4, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync");
+        CK(cudaMemcpyAsync(d[i], bufs[i], (size_t)buf_elems[i] * 4, cudaMemcpyHostToDevice, st));
     }
     auto c = [&](int i) { return reinterpret_cast<cpx*>(d[i]); };
 
@@ -769,23 +764,23 @@ int fdes_b200_sweep_test(int op, int N, int batch, const int* iargs, int n_iargs
                 h[i] = (kx < g.lo_end || kx >= g.hi_start) ? std::nanf("") : 0.f;
             }
             float* scratch = static_cast<float*>(da.get(h.size() * sizeof(float)));
-            ck(cudaMemcpyAsync(scratch, h.data(), h.size() * sizeof(float), cudaMemcpyHostToDevice, st), "cudaMemcpyAsync");
+            CK(cudaMemcpyAsync(scratch, h.data(), h.size() * sizeof(float), cudaMemcpyHostToDevice, st));
             launch_detector4d_cols(g, c(0), scratch, d[1], Q, bin, fa(0), batch, st);
-            ck(cudaStreamSynchronize(st), "sweep kernels");     // h goes out of scope
+            CK(cudaStreamSynchronize(st));     // h goes out of scope
         } break;
         default: throw std::runtime_error("sweep test: unknown op " + std::to_string(op));
     }
-    ck(cudaStreamSynchronize(st), "sweep kernels");
+    CK(cudaStreamSynchronize(st));
     for (int i = 0; i < nbufs; i++) {
         if (i == rp_buf) {
             for (int cf = 0; cf < nconf; cf++)
-                ck(cudaMemcpyAsync(bufs[i] + (size_t)cf * (nkeys + 1), rows.dev + (size_t)cf * rows.stride,
-                                   ((size_t)nkeys + 1) * sizeof(int), cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync");
+                CK(cudaMemcpyAsync(bufs[i] + (size_t)cf * (nkeys + 1), rows.dev + (size_t)cf * rows.stride,
+                                   ((size_t)nkeys + 1) * sizeof(int), cudaMemcpyDeviceToHost, st));
         } else if (buf_elems[i] > 0) {
-            ck(cudaMemcpyAsync(bufs[i], d[i], (size_t)buf_elems[i] * 4, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync");
+            CK(cudaMemcpyAsync(bufs[i], d[i], (size_t)buf_elems[i] * 4, cudaMemcpyDeviceToHost, st));
         }
     }
-    ck(cudaStreamSynchronize(st), "downloads");
+    CK(cudaStreamSynchronize(st));
     if (pipe_grid_out) *pipe_grid_out = pipe_last_grid;
     return 0;
     API_CATCH(-1)

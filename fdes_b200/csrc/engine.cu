@@ -39,17 +39,9 @@ static const KirklandRow kKirkland[103] = {
 #include "kirkland_table.inc"
 };
 
-#define CK(x)                                                                                    \
-    do {                                                                                         \
-        cudaError_t e_ = (x);                                                                    \
-        if (e_ != cudaSuccess)                                                                   \
-            throw std::runtime_error(std::string("CUDA error: ") + cudaGetErrorString(e_) +      \
-                                     " at " + __FILE__ + ":" + std::to_string(__LINE__));        \
-    } while (0)
-
 // Every public entry point runs on the engine's own device, whatever the caller's current device
 // is (torch switching devices, several engines of one process on different GPUs), and restores
-// the caller's device on the way out.
+// the caller's device on the way out (Engine::Call).
 namespace {
 struct DeviceGuard {
     int prev = -1;
@@ -69,6 +61,25 @@ struct DeviceGuard {
     DeviceGuard& operator=(const DeviceGuard&) = delete;
 };
 }  // namespace
+
+// The scope of a public entry point: the engine's device, and the kernels the call launched (the growth of
+// launch_tally) added to EngineTimings::kernel_launches.  A call made from inside another one
+// (stem_scan_4d -> stem_4d_probes_per_pass) is counted by the outer call.
+struct Engine::Call {
+    Engine& e;
+    DeviceGuard device;
+    const bool outer;
+    const long long tally0;
+    explicit Call(Engine& eng) : e(eng), device(eng.opt_.gpu_index), outer(!eng.in_call_), tally0(launch_tally) { e.in_call_ = true; }
+    ~Call()
+    {
+        if (!outer) return;
+        e.tm_.kernel_launches += launch_tally - tally0;
+        e.in_call_ = false;
+    }
+    Call(const Call&) = delete;
+    Call& operator=(const Call&) = delete;
+};
 
 // ---------------------------------------------------------------------------------------------
 // Device memory: every buffer of an Engine is a slice of ONE block, and blocks are cached per
@@ -171,7 +182,7 @@ Engine::Engine(const Params& pin, const Atoms& atoms, const EngineOptions& opt) 
         throw std::runtime_error("no CUDA device: fdes_b200 has no CPU fallback");
     if (opt_.gpu_index < 0 || opt_.gpu_index >= ndev)
         throw std::runtime_error("gpu index " + std::to_string(opt_.gpu_index) + " out of range (" + std::to_string(ndev) + " device(s))");
-    DeviceGuard guard(opt_.gpu_index);
+    const Call call(*this);
     try {
         init(atoms);
     } catch (...) {
@@ -277,14 +288,9 @@ void Engine::init(const Atoms& atoms)
     CK(cudaMemcpyAsync(xyzTO_, xyz0_, 3 * (size_t)nAt_ * sizeof(float), cudaMemcpyDeviceToDevice, st_));
     tilt(xyzTO_, p_.tilt_off[0], p_.tilt_off[1], p_.tilt_off[2]);
 
-    if (p_.pD > FLT_EPSILON) {
-        // Poisson-noise streams: seed 1 + n3, one per pixel (src/crystalMaker.cu:295)
-        launch_rng_init(noise_rng_, (int)NN, 1ULL + (unsigned long long)p_.n3, st_);
-        tm_.kernel_launches += 1;
-    }
-    if (p_.frPh > 0) {
-        launch_rng_init(rng_, 3 * nAt_, 1ULL, st_);   // seed 1, src/crystalMaker.cu:292
-    }
+    // Poisson-noise streams: seed 1 + n3, one per pixel (src/crystalMaker.cu:295)
+    if (p_.pD > FLT_EPSILON) launch_rng_init(noise_rng_, (int)NN, 1ULL + (unsigned long long)p_.n3, st_);
+    if (p_.frPh > 0) launch_rng_init(rng_, 3 * nAt_, 1ULL, st_);   // seed 1, src/crystalMaker.cu:292
     setup_tables();
     CK(cudaStreamSynchronize(st_));
     pt.mark("ctor: rng+tables");
@@ -341,7 +347,6 @@ void Engine::setup_tables()
         }
         launch_scattering_table(Gq_ + (size_t)z * Q * Q, N_, kr, p_.d1, p_.d2, p_.sigma, p_.cst_pi, st_);
     }
-    tm_.kernel_launches += 1 + nZ_;
 }
 
 void Engine::tilt(float* xyz, float t0, float t1, float t2)
@@ -350,6 +355,13 @@ void Engine::tilt(float* xyz, float t0, float t1, float t2)
     if (fabsf(t2) > FLT_EPSILON) launch_rot(xyz, nAt_, 0, 1, cosf(t2), -sinf(t2), st_);
     if (fabsf(t1) > FLT_EPSILON) launch_rot(xyz, nAt_, 0, 2, cosf(t1), -sinf(t1), st_);
     if (fabsf(t0) > FLT_EPSILON) launch_rot(xyz, nAt_, 1, 2, cosf(t0), -sinf(t0), st_);
+}
+
+// the specimen of measurement k in xyzK_: offset and tilt (src/crystalMaker.cu:282-283, 427-454)
+void Engine::specimen_k(int k)
+{
+    CK(cudaMemcpyAsync(xyzK_, xyzTO_, 3 * (size_t)nAt_ * sizeof(float), cudaMemcpyDeviceToDevice, st_));
+    tilt(xyzK_, p_.tiltspec[2 * k], p_.tiltspec[2 * k + 1], 0.f);
 }
 
 void Engine::set_accumulators(float* intensity_dev, cpx* exitwave_dev)
@@ -391,10 +403,8 @@ void Engine::make_incident(int k)
         const float nrm = (float)sqrt(s * (double)N_);
         const float alpha = sqrtf((float)(p_.n1 * p_.n2)) / nrm;
         launch_scale_cpx(psi_in_, NN, alpha, st_);
-        tm_.kernel_launches += 8;
     } else {
         launch_plane_wave_rowspace(psi_in_, N_, 1, st_);
-        tm_.kernel_launches += 1;
     }
     if (p_.doBeamTilt) {
         // phase ramp in real space (tiltBeam_d, :89-120)
@@ -413,7 +423,6 @@ void Engine::make_incident(int k)
             r3.scale = 1.f / (float)N_;   // row-space convention: Psi = FFT_row(psi) / N
             launch_rows_fft(g_, scratch_, psi_in_, -1, ROW_STORE, r3, 1, st_);
         }
-        tm_.kernel_launches += 5;
     }
     incident_k_ = k;
 }
@@ -434,8 +443,6 @@ void Engine::bin_and_sort(int b0, int nconf, const float* xyz_dev, int set, cuda
     launch_radix_sort(sb, nrec_, key_bits_, nconf, st);
     launch_row_pointers(keys, nrec_, r.rowptr + (size_t)b0 * rp_stride_, nkeys_, nconf, st, rp_stride_);
     if (mask_E_ > 0) launch_row_masks(r.rowptr + (size_t)b0 * rp_stride_, rp_stride_, nkeys_, N_, mask_E_, nconf, st);
-    int passes = (key_bits_ + 7) / 8; if (passes & 1) passes++; if (!passes) passes = 2;
-    tm_.kernel_launches += 2 + 3 * passes + (mask_E_ > 0 ? 1 : 0);
 }
 
 // jitter + bin + sort + row pointers for the configurations of one batch (slots 0 .. nb-1)
@@ -455,12 +462,10 @@ void Engine::prepare_batch(int nb, const float* xyz_k, int set, cudaStream_t st)
             launch_rng_init(rng_, 3 * nAt_, 1ULL, st);
             rng_pos_ = 0;
             burn = rng_target_;
-            tm_.kernel_launches += 1;
         }
         launch_atom_jitter(xyzFP, xyz_k, dwf_, nAt_, rng_, burn, nb, st);
         rng_pos_ = rng_target_ + nb;
         rng_target_ = rng_pos_;
-        tm_.kernel_launches += 1;
     } else {
         for (int b = 0; b < nb; b++)
             CK(cudaMemcpyAsync(xyzFP + (size_t)b * 3 * nAt_, xyz_k, 3 * (size_t)nAt_ * sizeof(float), cudaMemcpyDeviceToDevice, st));
@@ -537,18 +542,13 @@ void Engine::run_slices_plain(int nb)
         if (npair == 1 && nb % 2 == 0) {
             // odd slice count: the last slices of configurations 2j and 2j + 1 share one complex transform
             // through S1 / S2 / S3 (instead of nb half-empty pairs); S3 writes t of configuration b to D[b]
-            launch_density_rows(g_, A_, rs_[act_].rowptr, rs_[act_].cols, rs_[act_].w, s, s, nZ_, nb / 2, rec_stride_, rp_stride_, st_, 2, 1);
-            launch_potential_cols(g_, W_, A_, Gq_, rs_[act_].rowptr, s, s, nZ_, nb / 2, rp_stride_, st_, 2, 1);
+            potential_pair(s, s, nb / 2, 2, 1);
             launch_transmit_rows(g_, W_, D_, 2, p_.imPot, nb / 2, st_);
             launch_bandlimit_cols(g_, D_, nb, 0, st_);
             wave_step(D_, NN, s);
             break;
         }
-        const int s2 = npair > 1 ? s + 1 : -1;
-        launch_density_rows(g_, A_, rs_[act_].rowptr, rs_[act_].cols, rs_[act_].w, s, s2, nZ_, nb, rec_stride_, rp_stride_, st_);
-        launch_potential_cols(g_, W_, A_, Gq_, rs_[act_].rowptr, s, s2, nZ_, nb, rp_stride_, st_);
-        launch_transmit_rows(g_, W_, D_, npair, p_.imPot, nb, st_);
-        launch_bandlimit_cols(g_, D_, nb, npair, st_);
+        transmission_pair(s, npair, nb, D_);
         for (int p = 0; p < npair; p++) wave_step(D_ + (size_t)p * NN, 2 * NN, s + p);
     }
     if (first_full) launch_zero_outband(Psi_, N_, g_.lo_end, g_.hi_start, nb, st_);
@@ -557,26 +557,49 @@ void Engine::run_slices_plain(int nb)
 void Engine::slice_loop(int nb)
 {
     tm_.slices_executed += (long long)p_.m3 * nb;
-    tm_.kernel_launches += 4LL * ((p_.m3 + 1) / 2) + 2LL * p_.m3 - (plane_first_slice_ ? 1 : 0);   // no S5 in the first slice of a plane wave
     // a CUDA graph pays off when the sweeps are launch-bound (small grids, small batches); its
     // capture + instantiation costs about a millisecond, more than it saves on large launches
     if (!opt_.use_graph || (size_t)nb * N_ * N_ > ((size_t)1 << 21)) { run_slices_plain(nb); return; }
     cudaGraphExec_t& graph_ = this->graph_[act_];     // the captured launches carry the record pointers of a set
     int& graph_nb_ = this->graph_nb_[act_];
+    long long& graph_launches = graph_launches_[act_];
     const int key = 2 * nb + (fuse_ctf_ && !ew_ ? 1 : 0);     // what the captured launches depend on
     if (!graph_ || graph_nb_ != key) {
         if (graph_) { cudaGraphExecDestroy(graph_); graph_ = nullptr; }
         // first use of each kernel must happen outside capture (function attributes are set there)
         if (!warmed_) { run_slices_plain(nb); warmed_ = true; graph_nb_ = -1; return; }
         cudaGraph_t g = nullptr;
+        const long long tally0 = launch_tally;
         CK(cudaStreamBeginCapture(st_, cudaStreamCaptureModeThreadLocal));
         run_slices_plain(nb);
         CK(cudaStreamEndCapture(st_, &g));
+        // a capture runs nothing: its kernels count at every launch of the graph
+        graph_launches = launch_tally - tally0;
+        launch_tally = tally0;
         CK(cudaGraphInstantiate(&graph_, g, 0));
         CK(cudaGraphDestroy(g));
         graph_nb_ = key;
     }
     CK(cudaGraphLaunch(graph_, st_));
+    tm_.kernel_launches += graph_launches;
+}
+
+// S1 + S2 of a slice pair from the active record set: the potentials of `images` images in W_ (image b: slice s of
+// configuration b * cfg_stride, slice s2 of configuration b * cfg_stride + cfg_off2, kernels.cuh)
+void Engine::potential_pair(int s, int s2, int images, int cfg_stride, int cfg_off2)
+{
+    const RecordSet& r = rs_[act_];
+    launch_density_rows(g_, A_, r.rowptr, r.cols, r.w, s, s2, nZ_, images, rec_stride_, rp_stride_, st_, cfg_stride, cfg_off2);
+    launch_potential_cols(g_, W_, A_, Gq_, r.rowptr, s, s2, nZ_, images, rp_stride_, st_, cfg_stride, cfg_off2);
+}
+
+// S1..S4 of slices s, s + 1 (npair = 2) or of slice s alone (npair = 1) of nb configurations: the band-limited
+// transmission functions in the [nb][2] stack D
+void Engine::transmission_pair(int s, int npair, int nb, cpx* D)
+{
+    potential_pair(s, npair > 1 ? s + 1 : -1, nb);
+    launch_transmit_rows(g_, W_, D, npair, p_.imPot, nb, st_);
+    launch_bandlimit_cols(g_, D, nb, npair, st_);
 }
 
 // CTF table of measurement k (applyLensFunction, src/multisliceSimulation.cu:614-622), stored [kx][ky]
@@ -585,7 +608,6 @@ void Engine::ensure_lens(int k)
     if (p_.mode == 0 && lens_k_ != k) {
         launch_lens_table(lens_, N_, lens_params(p_, k, 0), 1.f, st_, /*transposed=*/true);
         lens_k_ = k;
-        tm_.kernel_launches += 1;
     }
 }
 
@@ -599,7 +621,6 @@ void Engine::accumulate_outputs(int k, int nb)
     if (ew_) {
         RowOpts ro; ro.scale = alpha; ro.band_only_in = true;
         launch_rows_fft_sum(g_, Psi_, ew_, +1, ROW_ACCUM, ro, nb, st_);
-        tm_.kernel_launches += 1;
     }
     if (p_.mode == 0) {
         // W_ is free after the slice loop: CTF-filtered waves of the whole batch
@@ -609,7 +630,6 @@ void Engine::accumulate_outputs(int k, int nb)
         if (!(fuse_ctf_ && !ew_)) launch_cols_fft(g_, Psi_, W_, -1, COL_MUL_CPX_INV, lens_, 1.f / ((float)N_), nb, st_);
         RowOpts ro; ro.scale = alpha; ro.band_only_in = true;
         launch_rows_fft_sum(g_, W_, I_, +1, ROW_INTENS_ACCUM, ro, nb, st_);
-        tm_.kernel_launches += (fuse_ctf_ && !ew_) ? 1 : 2;
         return;
     }
     for (int b = 0; b < nb; b++) {   // fixed order: deterministic phonon average
@@ -636,24 +656,21 @@ void Engine::accumulate_outputs(int k, int nb)
                     launch_rows_fft(g_, scratch_, scratch_, -1, ROW_STORE, r2, 1, st_);
                 }
                 src = scratch_;
-                tm_.kernel_launches += 4;
             }
             launch_cols_fft(g_, src, I_, -1, COL_DP_ACCUM, nullptr, scale, 1, st_);
-            tm_.kernel_launches += 1;
         }
     }
 }
 
 void Engine::run_k(int k)
 {
-    DeviceGuard guard(opt_.gpu_index);
+    const Call call(*this);
     PhaseTimer pt;
     if (k < 0 || k >= p_.n3) throw std::runtime_error("measurement index out of range");
     const size_t NN = (size_t)N_ * N_;
     launch_fill_f32(I_, NN, 0.f, st_);
     if (ew_) launch_fill_cpx(ew_, NN, make_float2(0.f, 0.f), st_);
-    CK(cudaMemcpyAsync(xyzK_, xyzTO_, 3 * (size_t)nAt_ * sizeof(float), cudaMemcpyDeviceToDevice, st_));
-    tilt(xyzK_, p_.tiltspec[2 * k], p_.tiltspec[2 * k + 1], 0.f);
+    specimen_k(k);
     make_incident(k);
     run_batches(k, j0_, j1_, true);
     pt.mark("run_k: enqueue");
@@ -666,7 +683,7 @@ void Engine::run_k(int k)
 // are added to this engine's accumulators.  All engines must have finished run_k (it synchronises).
 void Engine::reduce_from(const std::vector<Engine*>& others)
 {
-    DeviceGuard guard(opt_.gpu_index);
+    const Call call(*this);
     if (others.empty()) return;
     if ((int)others.size() > MAX_PEERS) throw std::runtime_error("too many peer engines");
     const size_t NN = (size_t)N_ * N_;
@@ -691,7 +708,6 @@ void Engine::reduce_from(const std::vector<Engine*>& others)
     if (direct) {
         launch_peer_sum(I_, si, NN, st_);
         if (ew_ && se.n) launch_peer_sum(reinterpret_cast<float*>(ew_), se, 2 * NN, st_);
-        tm_.kernel_launches += 1 + (ew_ && se.n ? 1 : 0);
     } else {
         // no peer mapping (PCIe boxes without P2P): stage each partial sum through scratch_
         for (Engine* o : others) {
@@ -704,7 +720,6 @@ void Engine::reduce_from(const std::vector<Engine*>& others)
                 CK(cudaMemcpyPeerAsync(scratch_, opt_.gpu_index, o->ew_, o->opt_.gpu_index, NN * sizeof(cpx), st_));
                 launch_peer_sum(reinterpret_cast<float*>(ew_), one, 2 * NN, st_);
             }
-            tm_.kernel_launches += 2;
         }
     }
     CK(cudaStreamSynchronize(st_));
@@ -712,7 +727,7 @@ void Engine::reduce_from(const std::vector<Engine*>& others)
 
 void Engine::finish_k(int k, float* image_host, float* exitwave_host)
 {
-    DeviceGuard guard(opt_.gpu_index);
+    const Call call(*this);
     PhaseTimer pt;
     const size_t NN = (size_t)N_ * N_;
     // addNoiseAndMtf (src/crystalMaker.cu:579-613) + copyMiddleOut
@@ -731,13 +746,11 @@ void Engine::finish_k(int k, float* image_host, float* exitwave_host)
         launch_anscombe_noise(scratch_, NN, p_.pD, noise_rng_, st_);
         launch_rows_fft(g_, scratch_, scratch_, -1, ROW_STORE, rr, 1, st_);
         dp.use_incoherence = 0;   // already applied
-        tm_.kernel_launches += 5;
     }
     launch_detector_table(det_, N_, dp, inv_nn, st_);
     launch_cols_fft(g_, scratch_, scratch_, -1, COL_MUL_REAL_INV, det_, 1.f, 1, st_);
     RowOpts rc; rc.dn1 = p_.dn1; rc.dn2 = p_.dn2; rc.n1 = p_.n1; rc.n2 = p_.n2;
     launch_rows_fft(g_, scratch_, J_, +1, ROW_CROP_REAL, rc, 1, st_);
-    tm_.kernel_launches += 4;
     if (image_host)
         CK(cudaMemcpyAsync(image_host, J_, (size_t)p_.n1 * p_.n2 * sizeof(float), cudaMemcpyDeviceToHost, st_));
     if (exitwave_host && ew_)
@@ -746,9 +759,21 @@ void Engine::finish_k(int k, float* image_host, float* exitwave_host)
     pt.mark("finish_k");
 }
 
+// the potential of slice s (records of the active set) in real space, with the absorptive factor -> V_host [m2][m1][2]
+void Engine::potential_to_host(int s, float* V_host)
+{
+    const size_t NN = (size_t)N_ * N_;
+    potential_pair(s, -1, 1);
+    RowOpts ro;
+    launch_rows_fft(g_, W_, scratch_, +1, ROW_STORE, ro, 1, st_);
+    launch_absorptive_factor(scratch_, NN, p_.imPot, st_);
+    CK(cudaMemcpyAsync(V_host, scratch_, NN * sizeof(cpx), cudaMemcpyDeviceToHost, st_));
+    CK(cudaStreamSynchronize(st_));
+}
+
 void Engine::potential_slices(float* out_host)
 {
-    DeviceGuard guard(opt_.gpu_index);
+    const Call call(*this);
     // untilted (offset only), phonon-free potential with the original slicing
     // (src/crystalMaker.cu:381-397).  NOTE: the reference leaves this buffer uninitialised when
     // no sub-slicing/phonons/tilt are active; here it is always computed.
@@ -759,16 +784,7 @@ void Engine::potential_slices(float* out_host)
     nkeys_ = m3_orig_ * nZ_ * N_;
     key_bits_ = 0; while ((1LL << key_bits_) <= nkeys_) key_bits_++;
     bin_and_sort(0, 1, xyzTO_);
-    RowOpts ro; ro.scale = 1.f;
-    for (int s = 0; s < m3_orig_; s++) {
-        launch_density_rows(g_, A_, rs_[act_].rowptr, rs_[act_].cols, rs_[act_].w, s, -1, nZ_, 1, rec_stride_, rp_stride_, st_);
-        launch_potential_cols(g_, W_, A_, Gq_, rs_[act_].rowptr, s, -1, nZ_, 1, rp_stride_, st_);
-        launch_rows_fft(g_, W_, scratch_, +1, ROW_STORE, ro, 1, st_);
-        launch_absorptive_factor(scratch_, NN, p_.imPot, st_);
-        CK(cudaMemcpyAsync(out_host + (size_t)s * 2 * NN, scratch_, NN * sizeof(cpx), cudaMemcpyDeviceToHost, st_));
-        CK(cudaStreamSynchronize(st_));
-    }
-    tm_.kernel_launches += 4LL * m3_orig_;
+    for (int s = 0; s < m3_orig_; s++) potential_to_host(s, out_host + (size_t)s * 2 * NN);
     p_ = save; nkeys_ = nkeys_save; key_bits_ = bits_save;
 }
 
@@ -777,9 +793,8 @@ void Engine::potential_slices(float* out_host)
 // ---------------------------------------------------------------------------------------------
 void Engine::next_jittered_coords(int k, float* xyz_host)
 {
-    DeviceGuard guard(opt_.gpu_index);
-    CK(cudaMemcpyAsync(xyzK_, xyzTO_, 3 * (size_t)nAt_ * sizeof(float), cudaMemcpyDeviceToDevice, st_));
-    tilt(xyzK_, p_.tiltspec[2 * k], p_.tiltspec[2 * k + 1], 0.f);
+    const Call call(*this);
+    specimen_k(k);
     if (p_.frPh > 0) { launch_atom_jitter(rs_[act_].xyzFP, xyzK_, dwf_, nAt_, rng_, 0, 1, st_); rng_pos_ += 1; rng_target_ = rng_pos_; }
     else CK(cudaMemcpyAsync(rs_[act_].xyzFP, xyzK_, 3 * (size_t)nAt_ * sizeof(float), cudaMemcpyDeviceToDevice, st_));
     CK(cudaMemcpyAsync(xyz_host, rs_[act_].xyzFP, 3 * (size_t)nAt_ * sizeof(float), cudaMemcpyDeviceToHost, st_));
@@ -788,7 +803,7 @@ void Engine::next_jittered_coords(int k, float* xyz_host)
 
 void Engine::bin_tuples(const float* xyz_host, int* bins_host)
 {
-    DeviceGuard guard(opt_.gpu_index);
+    const Call call(*this);
     CK(cudaMemcpyAsync(rs_[act_].xyzFP, xyz_host, 3 * (size_t)nAt_ * sizeof(float), cudaMemcpyHostToDevice, st_));
     BinGeom bg{N_, N_, p_.m3, nZ_, p_.d1, p_.d2, p_.d3};
     launch_bin_atoms(rs_[act_].xyzFP, zidx_, occ_, nAt_, bg, rs_[act_].keys, rs_[act_].cols, rs_[act_].w, bins_, 1, st_);
@@ -798,22 +813,15 @@ void Engine::bin_tuples(const float* xyz_host, int* bins_host)
 
 void Engine::phase_grating(const float* xyz_host, int s, float* V_host)
 {
-    DeviceGuard guard(opt_.gpu_index);
-    const size_t NN = (size_t)N_ * N_;
+    const Call call(*this);
     CK(cudaMemcpyAsync(rs_[act_].xyzFP, xyz_host, 3 * (size_t)nAt_ * sizeof(float), cudaMemcpyHostToDevice, st_));
     bin_and_sort(0, 1, rs_[act_].xyzFP);
-    launch_density_rows(g_, A_, rs_[act_].rowptr, rs_[act_].cols, rs_[act_].w, s, -1, nZ_, 1, rec_stride_, rp_stride_, st_);
-    launch_potential_cols(g_, W_, A_, Gq_, rs_[act_].rowptr, s, -1, nZ_, 1, rp_stride_, st_);
-    RowOpts ro;
-    launch_rows_fft(g_, W_, scratch_, +1, ROW_STORE, ro, 1, st_);
-    launch_absorptive_factor(scratch_, NN, p_.imPot, st_);
-    CK(cudaMemcpyAsync(V_host, scratch_, NN * sizeof(cpx), cudaMemcpyDeviceToHost, st_));
-    CK(cudaStreamSynchronize(st_));
+    potential_to_host(s, V_host);
 }
 
 void Engine::exit_wave(const float* xyz_host, int k, float* psi_host)
 {
-    DeviceGuard guard(opt_.gpu_index);
+    const Call call(*this);
     const size_t NN = (size_t)N_ * N_;
     CK(cudaMemcpyAsync(rs_[act_].xyzFP, xyz_host, 3 * (size_t)nAt_ * sizeof(float), cudaMemcpyHostToDevice, st_));
     bin_and_sort(0, 1, rs_[act_].xyzFP);
@@ -831,12 +839,11 @@ void Engine::exit_wave(const float* xyz_host, int k, float* psi_host)
 
 double Engine::bench_configs(int k, int configs)
 {
-    DeviceGuard guard(opt_.gpu_index);
+    const Call call(*this);
     const size_t NN = (size_t)N_ * N_;
     launch_fill_f32(I_, NN, 0.f, st_);
     if (ew_) launch_fill_cpx(ew_, NN, make_float2(0.f, 0.f), st_);
-    CK(cudaMemcpyAsync(xyzK_, xyzTO_, 3 * (size_t)nAt_ * sizeof(float), cudaMemcpyDeviceToDevice, st_));
-    tilt(xyzK_, p_.tiltspec[2 * k], p_.tiltspec[2 * k + 1], 0.f);
+    specimen_k(k);
     make_incident(k);
     CK(cudaStreamSynchronize(st_));
     CK(cudaEventRecord(ev0_, st_));
@@ -888,8 +895,7 @@ void Engine::stem_prepare(int k, int nprobes, const float* xy_host, float* shift
     }
     CK(cudaMemcpyAsync(shifts, sh.data(), sh.size() * sizeof(float), cudaMemcpyHostToDevice, st_));
     launch_fill_f32(det_out, det_elems, 0.f, st_);
-    CK(cudaMemcpyAsync(xyzK_, xyzTO_, 3 * (size_t)nAt_ * sizeof(float), cudaMemcpyDeviceToDevice, st_));
-    tilt(xyzK_, p_.tiltspec[2 * k], p_.tiltspec[2 * k + 1], 0.f);
+    specimen_k(k);
     make_incident(k);
     // spectrum of the centred probe: PSI0 = FFT_col(psi_in) (scratch_ is free after make_incident)
     launch_cols_fft(g_, psi_in_, scratch_, -1, COL_PLAIN, nullptr, 1.f, 1, st_);
@@ -903,18 +909,10 @@ void Engine::stem_transmission(int k, int j, cpx* tstack)
     const size_t NN = (size_t)N_ * N_;
     rng_target_ = (long long)k * count_ + j;
     prepare_batch(1, xyzK_);
-    for (int s = 0; s < p_.m3; s += 2) {
-        const int npair = std::min(2, p_.m3 - s);
-        const int s2 = npair > 1 ? s + 1 : -1;
-        launch_density_rows(g_, A_, rs_[act_].rowptr, rs_[act_].cols, rs_[act_].w, s, s2, nZ_, 1, rec_stride_, rp_stride_, st_);
-        launch_potential_cols(g_, W_, A_, Gq_, rs_[act_].rowptr, s, s2, nZ_, 1, rp_stride_, st_);
-        launch_transmit_rows(g_, W_, tstack + (size_t)s * NN, npair, p_.imPot, 1, st_);
-        launch_bandlimit_cols(g_, tstack + (size_t)s * NN, 1, npair, st_);
-    }
+    for (int s = 0; s < p_.m3; s += 2) transmission_pair(s, std::min(2, p_.m3 - s), 1, tstack + (size_t)s * NN);
     // (keeping t in real space instead, to save the per-probe inverse row transform of S5,
     // measured SLOWER on B200: 8.3k vs 9.5k probes/s at 512^2 -- the transform hides the
     // latency of the wave loads)
-    tm_.kernel_launches += 4LL * ((p_.m3 + 1) / 2);
 }
 
 // nb probes at shifts through every slice of tstack: exit waves in Psi_
@@ -926,14 +924,13 @@ void Engine::stem_probes(const float* shifts, int nb, const cpx* tstack)
         launch_multiply_rows(g_, Psi_, tstack + (size_t)s * NN, 0, nb, false, st_);
         launch_propagate_cols(g_, Psi_, Pq_, nb, st_);
     }
-    tm_.kernel_launches += 1 + 2LL * p_.m3;
     tm_.slices_executed += (long long)p_.m3 * nb;
 }
 
 void Engine::stem_scan(int k, int nprobes, const float* xy_host, int ndet, const float* det_mrad_host,
                        float* out_host, double* loop_ms)
 {
-    DeviceGuard guard(opt_.gpu_index);
+    const Call call(*this);
     const DetectorRings rings = stem_rings(k, nprobes, ndet, det_mrad_host, 1);
     const size_t NN = (size_t)N_ * N_;
     // device scratch of this call: transmission stack, probe shifts, detector sums
@@ -956,7 +953,6 @@ void Engine::stem_scan(int k, int nprobes, const float* xy_host, int ndet, const
                 const int nb = std::min(B_, nprobes - i0);
                 stem_probes(shifts + 2 * (size_t)i0, nb, tstack);
                 launch_detector_cols(g_, Psi_, partial, out + (size_t)i0 * ndet, rings, p_.d1, p_.d2, weight, nb, st_);
-                tm_.kernel_launches += 2;
             }
         }
         CK(cudaEventRecord(ev1_, st_));
@@ -1010,7 +1006,7 @@ int stem4d_window(int N, int window, int bin)
 
 int Engine::stem_4d_probes_per_pass(int nprobes, int window, int bin)
 {
-    DeviceGuard guard(opt_.gpu_index);
+    const Call call(*this);
     const int S = stem4d_window(N_, window, bin) / bin;
     size_t fr = 0, tot = 0;
     CK(cudaMemGetInfo(&fr, &tot));
@@ -1058,7 +1054,7 @@ struct PassCopies {
 void Engine::stem_scan_4d(int k, int nprobes, const float* xy_host, int window, int bin, int ndet, const float* det_mrad_host,
                           int probes_per_pass, float* out_pattern_host, float* out_det_host, double* loop_ms)
 {
-    DeviceGuard guard(opt_.gpu_index);
+    const Call call(*this);
     const DetectorRings rings = stem_rings(k, nprobes, ndet, det_mrad_host, 0);
     const int Q = stem4d_window(N_, window, bin);
     const size_t NN = (size_t)N_ * N_, QQ = (size_t)Q * Q, SS = (size_t)(Q / bin) * (Q / bin);
@@ -1094,18 +1090,14 @@ void Engine::stem_scan_4d(int k, int nprobes, const float* xy_host, int window, 
             if (pi >= 2)      // pass buffer s still on its way to the host (pass pi - 2)
                 for (int q = 0; q < 2; q++) CK(cudaStreamWaitEvent(st_, pc.copied[s][q], 0));
             launch_fill_f32(pass[s], (size_t)np * SS, 0.f, st_);
-            tm_.kernel_launches += 1;
             for (int j = j0_; j < j1_; j++) {
                 stem_transmission(k, j, tstack);
                 for (int i0 = 0; i0 < np; i0 += B_) {
                     const int nb = std::min(B_, np - i0);
                     stem_probes(shifts + 2 * (size_t)(p0 + i0), nb, tstack);
                     launch_detector4d_cols(g_, Psi_, scratch4d, pass[s] + (size_t)i0 * SS, Q, bin, weight, nb, st_);
-                    tm_.kernel_launches += 2;
-                    if (ndet > 0) {
+                    if (ndet > 0)
                         launch_detector_cols(g_, Psi_, partial, det + (size_t)(p0 + i0) * ndet, rings, p_.d1, p_.d2, weight, nb, st_);
-                        tm_.kernel_launches += 2;
-                    }
                 }
             }
             CK(cudaEventRecord(pc.done[s], st_));
@@ -1137,7 +1129,7 @@ void Engine::stem_scan_4d(int k, int nprobes, const float* xy_host, int window, 
 // bracketed by CUDA events on the engine's stream: ms6[i] = average launch duration of S(i+1).
 void Engine::time_sweeps(int k, int nb, int reps, float* ms6)
 {
-    DeviceGuard guard(opt_.gpu_index);
+    const Call call(*this);
     const size_t NN = (size_t)N_ * N_;
     nb = std::max(1, std::min(nb, B_));
     CK(cudaMemcpyAsync(xyzK_, xyzTO_, 3 * (size_t)nAt_ * sizeof(float), cudaMemcpyDeviceToDevice, st_));
@@ -1170,7 +1162,6 @@ void Engine::time_sweeps(int k, int nb, int reps, float* ms6)
         float ms = 0.f;
         CK(cudaEventElapsedTime(&ms, ev0_, ev1_));
         ms6[i] = ms / (float)reps / (i < 4 ? (float)npair : 1.f);   // per slice
-        tm_.kernel_launches += reps + 1;
     }
 }
 

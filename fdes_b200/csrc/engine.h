@@ -21,7 +21,7 @@ struct EngineTimings {
     double slice_loop_ms = 0.0;     // CUDA-event time spent in the S1..S6 loops
     double atoms_ms = 0.0;          // jitter + binning + sort + row pointers
     long long slices_executed = 0;  // (#sub-slices) x (#configurations) processed by this rank
-    long long kernel_launches = 0;  // kernels of this library launched (graph nodes included)
+    long long kernel_launches = 0;  // kernels of this library launched by the engine's calls (graph nodes at every replay)
 };
 
 // One simulation = one Params + one atom list on one GPU.
@@ -98,6 +98,7 @@ public:
     cudaStream_t stream() const { return st_; }
 
 private:
+    struct Call;                                    // scope of a public entry point (engine.cu)
     void init(const Atoms& atoms);                  // constructor body (device already selected)
     void release();                                 // stream, events, arena, graph
     void setup_tables();
@@ -110,6 +111,11 @@ private:
     void run_slices_plain(int nb);
     void accumulate_outputs(int k, int nb);
     void tilt(float* xyz_dev, float t0, float t1, float t2);
+    void specimen_k(int k);                         // xyzK_ <- the specimen of measurement k (offset and tilt)
+    // S1 + S2 (W_ <- potentials) and S1..S4 (D <- transmission functions) of a slice pair, from the active record set
+    void potential_pair(int s, int s2, int images, int cfg_stride = 1, int cfg_off2 = 0);
+    void transmission_pair(int s, int npair, int nb, cpx* D);
+    void potential_to_host(int s, float* V_host);   // real-space potential of slice s, absorptive factor applied
     // pieces of the STEM scans (engine.cu)
     DetectorRings stem_rings(int k, int nprobes, int ndet, const float* det_mrad_host, int min_det) const;
     void stem_prepare(int k, int nprobes, const float* xy_host, float* shifts, float* det_out, size_t det_elems);
@@ -160,8 +166,10 @@ private:
     int lens_k_ = -1, incident_k_ = -1;
     cudaGraphExec_t graph_[2] = {nullptr, nullptr};     // slice loop of a batch, per record set
     int graph_nb_[2] = {0, 0};
+    long long graph_launches_[2] = {0, 0};              // kernels of each graph
     bool warmed_ = false;
     EngineTimings tm_;
+    bool in_call_ = false;            // inside a public entry point (Call)
 };
 
 // frees the device blocks cached between simulations (idle ones)

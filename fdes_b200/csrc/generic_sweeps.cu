@@ -13,22 +13,12 @@
 #include "sweep_vtable.h"
 #include <algorithm>
 #include <cmath>
-#include <map>
-#include <mutex>
 #include <stdexcept>
 #include <string>
 #include <vector>
 
 namespace fdes {
 namespace {
-
-#define GEN_CHECK(x)                                                                             \
-    do {                                                                                         \
-        cudaError_t e_ = (x);                                                                    \
-        if (e_ != cudaSuccess)                                                                   \
-            throw std::runtime_error(std::string("CUDA error: ") + cudaGetErrorString(e_) +      \
-                                     " at " + __FILE__ + ":" + std::to_string(__LINE__));        \
-    } while (0)
 
 constexpr int GT = 256;          // threads per CTA
 constexpr int MAXFAC = 24;
@@ -502,8 +492,8 @@ __global__ void g_detector_finish(const float* partial, float* out, int ntiles, 
 size_t smem_limit()
 {
     int dev = 0, lim = 0;
-    GEN_CHECK(cudaGetDevice(&dev));
-    GEN_CHECK(cudaDeviceGetAttribute(&lim, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    CK(cudaGetDevice(&dev));
+    CK(cudaDeviceGetAttribute(&lim, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
     return (size_t)lim;
 }
 // columns per CTA: the widest of 4, 2, 1 that divides N and fits `bufs` line buffers
@@ -513,116 +503,76 @@ int col_width(int N, int bufs)
         if (N % L == 0 && (size_t)L * bufs * N * sizeof(cpx) <= smem_limit()) return L;
     throw std::runtime_error("grid size " + std::to_string(N) + " too large for the generic sweeps");
 }
-// Dynamic shared-memory opt-in, per kernel and per DEVICE (function attributes are per device); raised
-// only when a call needs more than what was set before, so replays inside a stream capture do not
-// touch the attribute.
-template <class K>
-void allow(K kernel, size_t bytes)
-{
-    if (bytes <= 48 * 1024) return;
-    static std::mutex mu;
-    static std::map<std::pair<const void*, int>, size_t> have;
-    int dev = 0;
-    GEN_CHECK(cudaGetDevice(&dev));
-    std::lock_guard<std::mutex> lk(mu);
-    size_t& cur = have[{reinterpret_cast<const void*>(kernel), dev}];
-    if (bytes > cur) {
-        GEN_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-        cur = bytes;
-    }
-}
 void check_geom(const SweepGeom& g)
 {
     if (g.lo_end < g.N || g.hi_start < g.N)
         throw std::runtime_error("generic sweeps expect the whole column range (lo_end = hi_start = N)");
 }
-#define GEN_LAUNCHED() GEN_CHECK(cudaGetLastError())
-
 void gen_density_rows(const SweepGeom& g, cpx* A, const int* rowptr, const int* rec_col, const float* rec_w, int slice, int slice2,
                   int nZ, int batch, size_t rec_stride, size_t rp_stride, int cfg_stride, int cfg_off2, cudaStream_t st)
 {
     const size_t sm = 2 * (size_t)g.N * sizeof(cpx);
-    allow(g_density_rows, sm);
-    g_density_rows<<<dim3(g.N, nZ, batch), GT, sm, st>>>(A, rowptr, rec_col, rec_w, slice, slice2, nZ, rec_stride, rp_stride,
-                                                        cfg_stride, cfg_off2, make_plan(g.N), g.tw);
-    GEN_LAUNCHED();
+    launch(g_density_rows, dim3(g.N, nZ, batch), GT, sm, st, A, rowptr, rec_col, rec_w, slice, slice2, nZ, rec_stride, rp_stride,
+           cfg_stride, cfg_off2, make_plan(g.N), g.tw);
 }
 void gen_potential_cols(const SweepGeom& g, cpx* B, const cpx* A, const float* Gq, const int* rowptr, int slice, int slice2, int nZ,
                     int batch, size_t rp_stride, int cfg_stride, int cfg_off2, cudaStream_t st)
 {
     const int L = col_width(g.N, 3);
     const size_t sm = 3 * (size_t)L * g.N * sizeof(cpx);
-    allow(g_potential_cols, sm);
-    g_potential_cols<<<dim3(g.N / L, batch), GT, sm, st>>>(B, A, Gq, rowptr, slice, slice2, nZ, rp_stride, cfg_stride, cfg_off2, L,
-                                                           make_plan(g.N), g.tw);
-    GEN_LAUNCHED();
+    launch(g_potential_cols, dim3(g.N / L, batch), GT, sm, st, B, A, Gq, rowptr, slice, slice2, nZ, rp_stride, cfg_stride, cfg_off2, L,
+           make_plan(g.N), g.tw);
 }
 void gen_transmit_rows(const SweepGeom& g, const cpx* Wf, cpx* D, int npair, float imPot, int batch, cudaStream_t st)
 {
     check_geom(g);
     const size_t sm = 3 * (size_t)g.N * sizeof(cpx);
-    allow(g_transmit_rows, sm);
-    g_transmit_rows<<<dim3(g.N, batch), GT, sm, st>>>(Wf, D, npair, imPot, make_plan(g.N), g.tw);
-    GEN_LAUNCHED();
+    launch(g_transmit_rows, dim3(g.N, batch), GT, sm, st, Wf, D, npair, imPot, make_plan(g.N), g.tw);
 }
 void gen_bandlimit_cols(const SweepGeom& g, cpx* Wf, int batch, int npair, cudaStream_t st)
 {
     check_geom(g);
     const int L = col_width(g.N, 2);
     const size_t sm = 2 * (size_t)L * g.N * sizeof(cpx);
-    allow(g_bandlimit_cols, sm);
-    g_bandlimit_cols<<<dim3(g.N / L, npair == 0 ? batch : batch * npair), GT, sm, st>>>(Wf, npair, L, make_plan(g.N), g.tw);
-    GEN_LAUNCHED();
+    launch(g_bandlimit_cols, dim3(g.N / L, npair == 0 ? batch : batch * npair), GT, sm, st, Wf, npair, L, make_plan(g.N), g.tw);
 }
 void gen_multiply_rows(const SweepGeom& g, cpx* Psi, const cpx* E, size_t e_batch_stride, int batch, bool, cudaStream_t st)
 {
     check_geom(g);
     const size_t sm = 3 * (size_t)g.N * sizeof(cpx);
-    allow(g_multiply_rows, sm);
-    g_multiply_rows<<<dim3(g.N, batch), GT, sm, st>>>(Psi, E, e_batch_stride, make_plan(g.N), g.tw);
-    GEN_LAUNCHED();
+    launch(g_multiply_rows, dim3(g.N, batch), GT, sm, st, Psi, E, e_batch_stride, make_plan(g.N), g.tw);
 }
 void gen_propagate_cols(const SweepGeom& g, cpx* Psi, const cpx* Pq, int batch, cudaStream_t st)
 {
     check_geom(g);
     const int L = col_width(g.N, 2);
     const size_t sm = 2 * (size_t)L * g.N * sizeof(cpx);
-    allow(g_propagate_cols, sm);
-    g_propagate_cols<<<dim3(g.N / L, batch), GT, sm, st>>>(Psi, Pq, L, make_plan(g.N), g.tw);
-    GEN_LAUNCHED();
+    launch(g_propagate_cols, dim3(g.N / L, batch), GT, sm, st, Psi, Pq, L, make_plan(g.N), g.tw);
 }
 void gen_rows_fft(const SweepGeom& g, const void* in, void* out, int dir, RowEpilogue epi, const RowOpts& o, int batch, cudaStream_t st)
 {
     const size_t sm = 2 * (size_t)g.N * sizeof(cpx);
-    allow(g_rows_fft, sm);
-    g_rows_fft<<<dim3(g.N, batch), GT, sm, st>>>(in, out, dir, (int)epi, o, make_plan(g.N), g.tw);
-    GEN_LAUNCHED();
+    launch(g_rows_fft, dim3(g.N, batch), GT, sm, st, in, out, dir, (int)epi, o, make_plan(g.N), g.tw);
 }
 void gen_rows_fft_sum(const SweepGeom& g, const cpx* in, void* out, int dir, RowEpilogue epi, const RowOpts& o, int nb, cudaStream_t st)
 {
     if (dir <= 0 || (epi != ROW_ACCUM && epi != ROW_INTENS_ACCUM))
         throw std::runtime_error("launch_rows_fft_sum supports inverse transforms with ROW_ACCUM / ROW_INTENS_ACCUM");
     const size_t sm = 3 * (size_t)g.N * sizeof(cpx);
-    allow(g_rows_fft_sum, sm);
-    g_rows_fft_sum<<<dim3(g.N), GT, sm, st>>>(in, out, (int)epi, o, nb, make_plan(g.N), g.tw);
-    GEN_LAUNCHED();
+    launch(g_rows_fft_sum, dim3(g.N), GT, sm, st, in, out, (int)epi, o, nb, make_plan(g.N), g.tw);
 }
 void gen_cols_fft(const SweepGeom& g, const cpx* in, void* out, int dir, ColOp op, const void* table, float scale, int batch, cudaStream_t st)
 {
     const int L = col_width(g.N, 2);
     const size_t sm = 2 * (size_t)L * g.N * sizeof(cpx);
-    allow(g_cols_fft, sm);
-    g_cols_fft<<<dim3(g.N / L, batch), GT, sm, st>>>(in, out, dir, (int)op, table, scale, L, make_plan(g.N), g.tw);
-    GEN_LAUNCHED();
+    launch(g_cols_fft, dim3(g.N / L, batch), GT, sm, st, in, out, dir, (int)op, table, scale, L, make_plan(g.N), g.tw);
 }
 void gen_probe_cols(const SweepGeom& g, cpx* Psi, const cpx* PSI0, const float* shifts, int batch, cudaStream_t st)
 {
     check_geom(g);
     const int L = col_width(g.N, 2);
     const size_t sm = 2 * (size_t)L * g.N * sizeof(cpx);
-    allow(g_probe_cols, sm);
-    g_probe_cols<<<dim3(g.N / L, batch), GT, sm, st>>>(Psi, PSI0, shifts, L, make_plan(g.N), g.tw);
-    GEN_LAUNCHED();
+    launch(g_probe_cols, dim3(g.N / L, batch), GT, sm, st, Psi, PSI0, shifts, L, make_plan(g.N), g.tw);
 }
 int gen_detector_tiles(const SweepGeom& g) { return g.N / col_width(g.N, 2); }
 void gen_detector_cols(const SweepGeom& g, const cpx* Psi, float* partial, float* out, const DetectorRings& rings, float d1, float d2,
@@ -631,13 +581,10 @@ void gen_detector_cols(const SweepGeom& g, const cpx* Psi, float* partial, float
     check_geom(g);
     const int L = col_width(g.N, 2), tiles = g.N / L;
     const size_t sm = std::max<size_t>(2 * (size_t)L * g.N * sizeof(cpx), GT * sizeof(float));
-    allow(g_detector_cols, sm);
-    g_detector_cols<<<dim3(tiles, batch), GT, sm, st>>>(Psi, partial, rings, 1.f / ((float)g.N * d1), 1.f / ((float)g.N * d2), L,
-                                                       make_plan(g.N), g.tw);
-    GEN_LAUNCHED();
+    launch(g_detector_cols, dim3(tiles, batch), GT, sm, st, Psi, partial, rings, 1.f / ((float)g.N * d1), 1.f / ((float)g.N * d2), L,
+           make_plan(g.N), g.tw);
     const int n = batch * rings.n;
-    g_detector_finish<<<(n + 127) / 128, 128, 0, st>>>(partial, out, tiles, rings.n, batch, weight);
-    GEN_LAUNCHED();
+    launch(g_detector_finish, (n + 127) / 128, 128, 0, st, partial, out, tiles, rings.n, batch, weight);
 }
 void gen_detector4d_cols(const SweepGeom& g, const cpx* Psi, float* scratch, float* out, int Q, int bin, float weight, int batch,
                          cudaStream_t st)
@@ -645,11 +592,8 @@ void gen_detector4d_cols(const SweepGeom& g, const cpx* Psi, float* scratch, flo
     check_geom(g);
     const int L = col_width(g.N, 2);
     const size_t sm = 2 * (size_t)L * g.N * sizeof(cpx);
-    allow(g_detector4d_cols, sm);
-    g_detector4d_cols<<<dim3(g.N / L, batch), GT, sm, st>>>(Psi, scratch, Q, L, make_plan(g.N), g.tw);
-    GEN_LAUNCHED();
+    launch(g_detector4d_cols, dim3(g.N / L, batch), GT, sm, st, Psi, scratch, Q, L, make_plan(g.N), g.tw);
     launch_detector4d_finish(scratch, out, Q, bin, weight, batch, st);
-    GEN_LAUNCHED();
 }
 // W[k] = exp(-2 pi i k / N), exact on the axes: N float32 pairs, followed by the same N values as double
 // pairs (2 cpx slots each) for the long direct DFTs of g_fft

@@ -1,6 +1,7 @@
 // fdes_b200 -- launch interface of the sm_100a multislice kernels (kernels.cu).
 // Everything here is plain device pointers + sizes; the engine (engine.cu) owns the memory.
 #pragma once
+#include "launch.cuh"
 #include <cuda_runtime.h>
 #include <cstddef>
 #include <cstdint>

@@ -45,7 +45,7 @@ void launch_scattering_table(float* Gq, int N, KirklandRow kr, float d1, float d
                              float pi, cudaStream_t st)
 {
     const int Q = N / 2 + 1, n = Q * Q;
-    k_scattering_table<<<(n + 255) / 256, 256, 0, st>>>(Gq, N, kr, d1, d2, sigma, pi);
+    launch(k_scattering_table, (n + 255) / 256, 256, 0, st, Gq, N, kr, d1, d2, sigma, pi);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -76,7 +76,7 @@ void launch_propagator_table(cpx* Pq, int N, float d1, float d2, float d3, float
                              cudaStream_t st)
 {
     const int Q = N / 2 + 1, n = Q * Q;
-    k_propagator_table<<<(n + 255) / 256, 256, 0, st>>>(Pq, N, d1, d2, d3, lambda, pi);
+    launch(k_propagator_table, (n + 255) / 256, 256, 0, st, Pq, N, d1, d2, d3, lambda, pi);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -127,7 +127,7 @@ __global__ void k_lens_table(cpx* __restrict__ tab, int N, LensParams lp, float 
 void launch_lens_table(cpx* tab, int N, const LensParams& lp, float extra_scale, cudaStream_t st, bool transposed)
 {
     const int n = N * N;
-    k_lens_table<<<(n + 255) / 256, 256, 0, st>>>(tab, N, lp, extra_scale, transposed ? 1 : 0);
+    launch(k_lens_table, (n + 255) / 256, 256, 0, st, tab, N, lp, extra_scale, transposed ? 1 : 0);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -172,7 +172,7 @@ __global__ void k_detector_table(float* __restrict__ tab, int N, DetectorParams 
 void launch_detector_table(float* tab, int N, const DetectorParams& dp, float scale, cudaStream_t st)
 {
     const int n = N * N;
-    k_detector_table<<<(n + 255) / 256, 256, 0, st>>>(tab, N, dp, scale);
+    launch(k_detector_table, (n + 255) / 256, 256, 0, st, tab, N, dp, scale);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -190,8 +190,8 @@ __global__ void k_fill_f32(float* p, size_t n, float v)
 }
 static int grid_for(size_t n) { size_t g = (n + 255) / 256; return (int)(g > 148 * 8 ? 148 * 8 : (g ? g : 1)); }
 
-void launch_fill_cpx(cpx* p, size_t n, cpx v, cudaStream_t st) { k_fill_cpx<<<grid_for(n), 256, 0, st>>>(p, n, v); }
-void launch_fill_f32(float* p, size_t n, float v, cudaStream_t st) { k_fill_f32<<<grid_for(n), 256, 0, st>>>(p, n, v); }
+void launch_fill_cpx(cpx* p, size_t n, cpx v, cudaStream_t st) { launch(k_fill_cpx, grid_for(n), 256, 0, st, p, n, v); }
+void launch_fill_f32(float* p, size_t n, float v, cudaStream_t st) { launch(k_fill_f32, grid_for(n), 256, 0, st, p, n, v); }
 
 // out[b][y][x] += weight * sum of scratch[b][y*bin + r][x*bin + c], r outer, c inner: bins straddle the CTAs of the
 // detector sweep, so they are summed here, one thread per output pixel, without atomics
@@ -211,7 +211,7 @@ __global__ void k_detector4d_finish(const float* __restrict__ scratch, float* __
 void launch_detector4d_finish(const float* scratch, float* out, int Q, int bin, float weight, int batch, cudaStream_t st)
 {
     const size_t n = (size_t)batch * (Q / bin) * (Q / bin);
-    k_detector4d_finish<<<grid_for(n), 256, 0, st>>>(scratch, out, Q, bin, weight, n);
+    launch(k_detector4d_finish, grid_for(n), 256, 0, st, scratch, out, Q, bin, weight, n);
 }
 
 __global__ void k_plane_wave_rowspace(cpx* Psi, int N, size_t n)
@@ -222,7 +222,7 @@ __global__ void k_plane_wave_rowspace(cpx* Psi, int N, size_t n)
 void launch_plane_wave_rowspace(cpx* Psi, int N, int batch, cudaStream_t st)
 {
     const size_t n = (size_t)batch * N * N;
-    k_plane_wave_rowspace<<<grid_for(n), 256, 0, st>>>(Psi, N, n);
+    launch(k_plane_wave_rowspace, grid_for(n), 256, 0, st, Psi, N, n);
 }
 
 __global__ void k_scale_cpx(cpx* p, size_t n, float s)
@@ -230,7 +230,7 @@ __global__ void k_scale_cpx(cpx* p, size_t n, float s)
     for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
         p[i] = make_float2(p[i].x * s, p[i].y * s);
 }
-void launch_scale_cpx(cpx* p, size_t n, float s, cudaStream_t st) { k_scale_cpx<<<grid_for(n), 256, 0, st>>>(p, n, s); }
+void launch_scale_cpx(cpx* p, size_t n, float s, cudaStream_t st) { launch(k_scale_cpx, grid_for(n), 256, 0, st, p, n, s); }
 
 __global__ void k_absorptive_factor(cpx* V, size_t n, float imPot)
 {
@@ -239,7 +239,7 @@ __global__ void k_absorptive_factor(cpx* V, size_t n, float imPot)
 }
 void launch_absorptive_factor(cpx* V, size_t n, float imPot, cudaStream_t st)
 {
-    k_absorptive_factor<<<grid_for(n), 256, 0, st>>>(V, n, imPot);
+    launch(k_absorptive_factor, grid_for(n), 256, 0, st, V, n, imPot);
 }
 
 __global__ void k_zero_outband(cpx* Psi, int N, int lo_end, int hi_start, size_t n)
@@ -252,7 +252,7 @@ __global__ void k_zero_outband(cpx* Psi, int N, int lo_end, int hi_start, size_t
 void launch_zero_outband(cpx* Psi, int N, int lo_end, int hi_start, int batch, cudaStream_t st)
 {
     const size_t n = (size_t)batch * N * N;
-    k_zero_outband<<<grid_for(n), 256, 0, st>>>(Psi, N, lo_end, hi_start, n);
+    launch(k_zero_outband, grid_for(n), 256, 0, st, Psi, N, lo_end, hi_start, n);
 }
 
 // deterministic two-stage sum of |p|^2: fixed grid, fixed per-thread strides, tree in shared memory
@@ -286,8 +286,8 @@ __global__ void k_norm2_stage2(const double* __restrict__ partial, double* __res
 }
 void launch_norm2(const cpx* p, size_t n, double* partial, double* result, cudaStream_t st)
 {
-    k_norm2_stage1<<<NORM_BLOCKS, NORM_THREADS, 0, st>>>(p, n, partial);
-    k_norm2_stage2<<<1, NORM_BLOCKS, 0, st>>>(partial, result);
+    launch(k_norm2_stage1, NORM_BLOCKS, NORM_THREADS, 0, st, p, n, partial);
+    launch(k_norm2_stage2, 1, NORM_BLOCKS, 0, st, partial, result);
 }
 
 // tiltBeam_d, src/multisliceSimulation.cu:89-120
@@ -309,7 +309,7 @@ __global__ void k_tilt_beam(cpx* psi, int N, float d1, float d2, float lambda, f
 void launch_tilt_beam(cpx* psi, int N, float d1, float d2, float lambda, float tb_x, float tb_y,
                       float pi, int flag, cudaStream_t st)
 {
-    k_tilt_beam<<<(N * N + 255) / 256, 256, 0, st>>>(psi, N, d1, d2, lambda, tb_x, tb_y, pi, flag);
+    launch(k_tilt_beam, (N * N + 255) / 256, 256, 0, st, psi, N, d1, d2, lambda, tb_x, tb_y, pi, flag);
 }
 
 // taperedCosineWindow_d, src/multisliceSimulation.cu:123-156
@@ -331,7 +331,7 @@ __global__ void k_tukey_window(cpx* psi, int N, int dn1, int dn2, float pi)
 }
 void launch_tukey_window(cpx* psi, int N, int dn1, int dn2, float pi, cudaStream_t st)
 {
-    k_tukey_window<<<(N * N + 255) / 256, 256, 0, st>>>(psi, N, dn1, dn2, pi);
+    launch(k_tukey_window, (N * N + 255) / 256, 256, 0, st, psi, N, dn1, dn2, pi);
 }
 
 // areaMask + areaWeighting against a constant-1 field (applyMaskFiltering,
@@ -351,7 +351,7 @@ __global__ void k_area_mask_blend(cpx* psi, int N, int dn1, int dn2)
 }
 void launch_area_mask_blend(cpx* psi, int N, int dn1, int dn2, cudaStream_t st)
 {
-    k_area_mask_blend<<<(N * N + 255) / 256, 256, 0, st>>>(psi, N, dn1, dn2);
+    launch(k_area_mask_blend, (N * N + 255) / 256, 256, 0, st, psi, N, dn1, dn2);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -381,7 +381,7 @@ __global__ void k_peer_sum(float4* __restrict__ dst, PeerSources src, size_t n4,
 void launch_peer_sum(float* dst, const PeerSources& src, size_t n, cudaStream_t st)
 {
     const size_t n4 = n / 4;
-    k_peer_sum<<<(unsigned)std::max<size_t>(1, std::min<size_t>((n4 + 255) / 256, 148 * 8)), 256, 0, st>>>(reinterpret_cast<float4*>(dst), src, n4, n);
+    launch(k_peer_sum, (unsigned)std::max<size_t>(1, std::min<size_t>((n4 + 255) / 256, 148 * 8)), 256, 0, st, reinterpret_cast<float4*>(dst), src, n4, n);
 }
 
 }  // namespace fdes

@@ -28,58 +28,12 @@
 
 namespace fdes {
 
-// CUDA errors become exceptions (capi.cu turns them into return codes / fdes_b200_last_error()).
-#define FDES_CUDA_CHECK(x)                                                                       \
-    do {                                                                                         \
-        cudaError_t e_ = (x);                                                                    \
-        if (e_ != cudaSuccess)                                                                   \
-            throw std::runtime_error(std::string("CUDA error: ") + cudaGetErrorString(e_) +      \
-                                     " at " + __FILE__ + ":" + std::to_string(__LINE__));        \
-    } while (0)
-// after every <<<>>>: a launch that the driver refuses (bad configuration, missing shared-memory
-// opt-in on this device, ...) must not pass silently
-#define FDES_LAUNCH_CHECK() FDES_CUDA_CHECK(cudaGetLastError())
-
-// Function attributes are per DEVICE: remember per kernel (one static per call site and template
-// instantiation) on which devices the dynamic shared-memory limit was already raised.
-struct DeviceOnce {
-    std::atomic<unsigned long long> mask{0};
-    bool done(int dev) const { return (mask.load(std::memory_order_acquire) >> (dev & 63)) & 1ULL; }
-    void mark(int dev) { mask.fetch_or(1ULL << (dev & 63), std::memory_order_release); }
-};
-#define FDES_ALLOW_SMEM(kernel, bytes)                                                           \
-    do {                                                                                         \
-        if ((size_t)(bytes) > 48 * 1024) {                                                       \
-            static DeviceOnce once_;                                                             \
-            int dev_ = 0;                                                                        \
-            FDES_CUDA_CHECK(cudaGetDevice(&dev_));                                               \
-            if (!once_.done(dev_)) {                                                             \
-                FDES_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(bytes))); \
-                once_.mark(dev_);                                                                \
-            }                                                                                    \
-        }                                                                                        \
-    } while (0)
-
-// Programmatic dependent launch for the sweeps of the slice loop (about sixty dependent launches per
-// batch): a sweep is launched with programmatic stream serialisation, signals at its very start that its
-// dependents may be scheduled, and waits for its own prerequisites before it touches memory.  The CTAs of
-// sweep i+1 are then resident (index arithmetic, barrier set-up done) when the last CTAs of sweep i drain,
-// instead of being launched after the grid has completed.
+// Start of every sweep launched with launch_pdl (launch.cuh): let the next sweep be scheduled, then wait until the
+// previous one has finished before touching memory.
 __device__ __forceinline__ void pdl_prologue()
 {
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     asm volatile("griddepcontrol.wait;" ::: "memory");
-}
-template <class... KArgs, class... Args>
-void launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args)
-{
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at; cfg.numAttrs = 1;
-    FDES_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...));
 }
 
 // register budget per thread that __launch_bounds__ asks the compiler to respect
@@ -225,10 +179,10 @@ static int pipe_grid(int ntiles)
     if (n == 0) {
         static std::atomic<int> sms[64];
         int dev = 0;
-        FDES_CUDA_CHECK(cudaGetDevice(&dev));
+        CK(cudaGetDevice(&dev));
         n = sms[dev & 63].load();
         if (n == 0) {
-            FDES_CUDA_CHECK(cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev));
+            CK(cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev));
             sms[dev & 63].store(n);
         }
     }
@@ -307,11 +261,9 @@ void launch_density_rows_n(const SweepGeom& g, cpx* A, const int* rowptr, const 
 {
     using C = RowCfg<NN>;
     const size_t smem = C::SMEM + (size_t)C::RPB * NN * sizeof(cpx);
-    FDES_ALLOW_SMEM((k_density_rows<NN>), smem);
     dim3 grid(NN / C::RPB, nZ, batch);
     launch_pdl(k_density_rows<NN>, dim3(grid), dim3(C::THREADS), smem, st, A, rowptr, rec_col, rec_w, slice, slice2, nZ,
                                                       rec_stride, rowptr_stride, cfg_stride, cfg_off2, g.tw);
-    FDES_LAUNCH_CHECK();
 }
 
 // =============================================================================================
@@ -462,7 +414,6 @@ void launch_potential_cols_n(const SweepGeom& g, cpx* B, const cpx* A, const flo
     if (g.mask_off <= 0) throw std::runtime_error("S2 needs the row masks of the deposit records (SweepGeom::mask_off)");
     if constexpr (pipe_supported<NN>()) {
         using P = PipeCfg<NN>;
-        FDES_ALLOW_SMEM((k_potential_cols_tma<NN>), P::SMEM);
         const int tiles_x = NN / P::CW, ntiles = tiles_x * batch;
         CUtensorMap mapA, mapB;
         tile_map(&mapA, A, NN, batch * nZ, P::CW, P::BR);
@@ -471,12 +422,10 @@ void launch_potential_cols_n(const SweepGeom& g, cpx* B, const cpx* A, const flo
                                                                               nZ, rowptr_stride, g.mask_off, cfg_stride, cfg_off2, tiles_x, ntiles, g.tw);
     } else {
         using C = ColCfg<NN>;
-        FDES_ALLOW_SMEM((k_potential_cols<NN>), C::SMEM);
         dim3 grid(NN / C::CW, batch);
         launch_pdl(k_potential_cols<NN>, dim3(grid), dim3(C::THREADS), C::SMEM, st, B, A, Gq, rowptr, slice, slice2, nZ,
                                                                rowptr_stride, g.mask_off, cfg_stride, cfg_off2, g.tw);
     }
-    FDES_LAUNCH_CHECK();
 }
 
 // =============================================================================================
@@ -731,16 +680,13 @@ void launch_transmit_rows_n(const SweepGeom& g, const cpx* W, cpx* D, int npair,
     if constexpr (NN == 2048) {
         using S = SplitRowCfg<NN>;
         const size_t smem = S::SMEM_FFT + (size_t)S::RPB * NN * 2 * sizeof(float);
-        FDES_ALLOW_SMEM((k_transmit_rows_split<NN>), smem);
         launch_pdl(k_transmit_rows_split<NN>, dim3(NN / S::RPB, batch), dim3(S::THREADS), smem, st, W, D, npair, imPot, g.tw);
     } else {
         using C = RowCfg<NN>;
         const size_t smem = C::SMEM + (size_t)C::RPB * NN * 2 * sizeof(float);
-        FDES_ALLOW_SMEM((k_transmit_rows<NN>), smem);
         dim3 grid(NN / C::RPB, batch);
         launch_pdl(k_transmit_rows<NN>, dim3(grid), dim3(C::THREADS), smem, st, W, D, npair, imPot, g.tw);
     }
-    FDES_LAUNCH_CHECK();
 }
 
 // =============================================================================================
@@ -824,7 +770,6 @@ void launch_bandlimit_cols_n(const SweepGeom& g, cpx* W, int batch, int npair, c
 {
     if constexpr (pipe_supported<NN>()) {
         using P = PipeCfg<NN>;
-        FDES_ALLOW_SMEM((k_bandlimit_cols_tma<NN>), P::SMEM);
         const int nimg = npair == 0 ? batch : 2 * batch;     // images in the stack
         const int tiles_x = band_cols(g) / P::CW, ntiles = tiles_x * (npair == 0 ? batch : batch * npair);
         CUtensorMap map;
@@ -833,11 +778,9 @@ void launch_bandlimit_cols_n(const SweepGeom& g, cpx* W, int batch, int npair, c
                                                                               tiles_x, ntiles, g.tw);
     } else {
         using C = ColCfg<NN>;
-        FDES_ALLOW_SMEM((k_bandlimit_cols<NN>), C::SMEM);
         dim3 grid(band_cols(g) / C::CW, npair == 0 ? batch : batch * npair);
         launch_pdl(k_bandlimit_cols<NN>, dim3(grid), dim3(C::THREADS), C::SMEM, st, W, npair, g.lo_end, g.hi_start, g.tw);
     }
-    FDES_LAUNCH_CHECK();
 }
 
 // =============================================================================================
@@ -994,17 +937,14 @@ void launch_multiply_rows_n(const SweepGeom& g, cpx* Psi, const cpx* E, size_t e
     if constexpr (NN == 2048) {
         using S = SplitRowCfg<NN>;
         const size_t smem = S::SMEM_FFT + (size_t)S::RPB * NN * sizeof(cpx);
-        FDES_ALLOW_SMEM((k_multiply_rows_split<NN>), smem);
         launch_pdl(k_multiply_rows_split<NN>, dim3(NN / S::RPB, batch), dim3(S::THREADS), smem, st, Psi, E, e_batch_stride,
                    psi_full ? 1 : 0, g.tw);
     } else {
         using C = RowCfg<NN>;
         const size_t smem = C::SMEM + (size_t)C::RPB * NN * sizeof(cpx);
-        FDES_ALLOW_SMEM((k_multiply_rows<NN>), smem);
         dim3 grid(NN / C::RPB, batch);
         launch_pdl(k_multiply_rows<NN>, dim3(grid), dim3(C::THREADS), smem, st, Psi, E, e_batch_stride, psi_full ? 1 : 0, g.tw);
     }
-    FDES_LAUNCH_CHECK();
 }
 
 // =============================================================================================
@@ -1086,7 +1026,6 @@ void launch_propagate_cols_n(const SweepGeom& g, cpx* Psi, const cpx* Pq, int ba
 {
     if constexpr (pipe_supported<NN>()) {
         using P = PipeCfg<NN>;
-        FDES_ALLOW_SMEM((k_propagate_cols_tma<NN>), P::SMEM);
         const int tiles_x = band_cols(g) / P::CW, ntiles = tiles_x * batch;
         CUtensorMap map;
         tile_map(&map, Psi, NN, batch, P::CW, P::BR);
@@ -1094,11 +1033,9 @@ void launch_propagate_cols_n(const SweepGeom& g, cpx* Psi, const cpx* Pq, int ba
                                                                               (const cpx*)nullptr, g.lo_end, g.hi_start, tiles_x, ntiles, g.tw);
     } else {
         using C = ColCfg<NN>;
-        FDES_ALLOW_SMEM((k_propagate_cols<NN>), C::SMEM);
         dim3 grid(band_cols(g) / C::CW, batch);
         launch_pdl(k_propagate_cols<NN>, dim3(grid), dim3(C::THREADS), C::SMEM, st, Psi, Pq, g.lo_end, g.hi_start, g.tw);
     }
-    FDES_LAUNCH_CHECK();
 }
 
 // S6 reading the band columns of another image stack (launch_propagate_cols_from, kernels.cuh): pipelined kernels only
@@ -1107,7 +1044,6 @@ void launch_propagate_cols_from_n(const SweepGeom& g, cpx* Psi, const cpx* src, 
                                   int batch, bool times_n, const cpx* lens, cudaStream_t st)
 {
     using P = PipeCfg<NN>;
-    FDES_ALLOW_SMEM((k_propagate_cols_tma<NN>), P::SMEM);
     const int tiles_x = band_cols(g) / P::CW, ntiles = tiles_x * batch;
     CUtensorMap map_in, map_out;
     tile_map(&map_in, src, NN, src_images, P::CW, P::BR);
@@ -1115,7 +1051,6 @@ void launch_propagate_cols_from_n(const SweepGeom& g, cpx* Psi, const cpx* src, 
     // times_n: S5 with psi = 1 returns FFT_row(IFFT_row(D)) = N * D (unnormalised transforms): the same factor here
     launch_pdl(k_propagate_cols_tma<NN>, dim3(pipe_grid(ntiles)), dim3(P::THREADS), P::SMEM, st, map_in, map_out, src_img_stride,
                times_n ? (float)NN : 1.f, Pq, lens, g.lo_end, g.hi_start, tiles_x, ntiles, g.tw);
-    FDES_LAUNCH_CHECK();
 }
 
 // =============================================================================================
@@ -1177,12 +1112,7 @@ static void rows_fft_epi(const SweepGeom& g, const void* in, void* out, RowEpilo
     using C = RowCfg<N>;
     dim3 grid(N / C::RPB, batch);
 #define FDES_ROWS_CASE(EPI_)                                                                     \
-    case EPI_: {                                                                                 \
-        FDES_ALLOW_SMEM((k_rows_fft<N, DIR, EPI_>), C::SMEM);                                    \
-        k_rows_fft<N, DIR, EPI_><<<grid, C::THREADS, C::SMEM, st>>>(in, out, o, g.lo_end,        \
-                                                                   g.hi_start, g.tw);            \
-        FDES_LAUNCH_CHECK();                                                                     \
-    } break;
+    case EPI_: launch(k_rows_fft<N, DIR, EPI_>, grid, C::THREADS, C::SMEM, st, in, out, o, g.lo_end, g.hi_start, g.tw); break;
     switch (epi) {
         FDES_ROWS_CASE(ROW_STORE)
         FDES_ROWS_CASE(ROW_ACCUM)
@@ -1259,13 +1189,9 @@ void launch_rows_fft_sum_n(const SweepGeom& g, const cpx* in, void* out, int dir
     using C = RowCfg<NN>;
     dim3 grid(NN / C::RPB);
     if (dir > 0 && epi == ROW_ACCUM) {
-        FDES_ALLOW_SMEM((k_rows_fft_sum<NN, 1, ROW_ACCUM>), C::SMEM);
-        k_rows_fft_sum<NN, 1, ROW_ACCUM><<<grid, C::THREADS, C::SMEM, st>>>(in, out, o, nb, g.lo_end, g.hi_start, g.tw);
-        FDES_LAUNCH_CHECK();
+        launch(k_rows_fft_sum<NN, 1, ROW_ACCUM>, grid, C::THREADS, C::SMEM, st, in, out, o, nb, g.lo_end, g.hi_start, g.tw);
     } else if (dir > 0 && epi == ROW_INTENS_ACCUM) {
-        FDES_ALLOW_SMEM((k_rows_fft_sum<NN, 1, ROW_INTENS_ACCUM>), C::SMEM);
-        k_rows_fft_sum<NN, 1, ROW_INTENS_ACCUM><<<grid, C::THREADS, C::SMEM, st>>>(in, out, o, nb, g.lo_end, g.hi_start, g.tw);
-        FDES_LAUNCH_CHECK();
+        launch(k_rows_fft_sum<NN, 1, ROW_INTENS_ACCUM>, grid, C::THREADS, C::SMEM, st, in, out, o, nb, g.lo_end, g.hi_start, g.tw);
     } else {
         throw std::runtime_error("launch_rows_fft_sum supports inverse transforms with ROW_ACCUM / ROW_INTENS_ACCUM");
     }
@@ -1332,10 +1258,8 @@ static void cols_fft_one(const SweepGeom& g, const cpx* in, void* out, const voi
                          float scale, int batch, cudaStream_t st)
 {
     using C = ColCfg<N>;
-    FDES_ALLOW_SMEM((k_cols_fft<N, DIR, OP>), C::SMEM);
     dim3 grid(N / C::CW, batch);
-    k_cols_fft<N, DIR, OP><<<grid, C::THREADS, C::SMEM, st>>>(in, out, table, scale, g.tw);
-    FDES_LAUNCH_CHECK();
+    launch(k_cols_fft<N, DIR, OP>, grid, C::THREADS, C::SMEM, st, in, out, table, scale, g.tw);
 }
 
 // COL_MUL_CPX_INV on the band columns only, pipelined (col_pipe.cuh): out = scale * IFFT_col( FFT_col(in) * tab ),
@@ -1382,14 +1306,12 @@ void launch_cols_fft_n(const SweepGeom& g, const cpx* in, void* out, int dir, Co
     if constexpr (pipe_supported<NN>()) {
         if (op == COL_MUL_CPX_INV && g.lo_end < g.hi_start) {
             using P = PipeCfg<NN>;
-            FDES_ALLOW_SMEM((k_ctf_cols_tma<NN>), P::SMEM);
             const int tiles_x = band_cols(g) / P::CW, ntiles = tiles_x * batch;
             CUtensorMap map_in, map_out;
             tile_map(&map_in, in, NN, batch, P::CW, P::BR);
             tile_map(&map_out, out, NN, batch, P::CW, P::BR);
-            k_ctf_cols_tma<NN><<<pipe_grid(ntiles), P::THREADS, P::SMEM, st>>>(map_in, map_out, static_cast<const cpx*>(table),
-                                                                            scale, g.lo_end, g.hi_start, tiles_x, ntiles, g.tw);
-            FDES_LAUNCH_CHECK();
+            launch(k_ctf_cols_tma<NN>, pipe_grid(ntiles), P::THREADS, P::SMEM, st, map_in, map_out, static_cast<const cpx*>(table),
+                   scale, g.lo_end, g.hi_start, tiles_x, ntiles, g.tw);
             return;
         }
     }
@@ -1448,10 +1370,8 @@ void launch_probe_cols_n(const SweepGeom& g, cpx* Psi, const cpx* PSI0, const fl
                        cudaStream_t st)
 {
     using C = ColCfg<NN>;
-    FDES_ALLOW_SMEM((k_probe_cols<NN>), C::SMEM);
     dim3 grid(band_cols(g) / C::CW, batch);
-    k_probe_cols<NN><<<grid, C::THREADS, C::SMEM, st>>>(Psi, PSI0, shifts, g.lo_end, g.hi_start, g.tw);
-    FDES_LAUNCH_CHECK();
+    launch(k_probe_cols<NN>, grid, C::THREADS, C::SMEM, st, Psi, PSI0, shifts, g.lo_end, g.hi_start, g.tw);
 }
 
 // partial[b][tile][d] = sum over the tile's columns and all ky of |FFT_col(Psi_b)|^2 inside the
@@ -1528,15 +1448,12 @@ void launch_detector_cols_n(const SweepGeom& g, const cpx* Psi, float* partial, 
                           float d1, float d2, float weight, int batch, cudaStream_t st)
 {
     using C = ColCfg<NN>;
-    FDES_ALLOW_SMEM((k_detector_cols<NN>), C::SMEM);
     const int tiles = band_cols(g) / C::CW;
     dim3 grid(tiles, batch);
-    k_detector_cols<NN><<<grid, C::THREADS, C::SMEM, st>>>(Psi, partial, rings, 1.f / ((float)NN * d1),
-                                                          1.f / ((float)NN * d2), g.lo_end, g.hi_start, g.tw);
-    FDES_LAUNCH_CHECK();
+    launch(k_detector_cols<NN>, grid, C::THREADS, C::SMEM, st, Psi, partial, rings, 1.f / ((float)NN * d1), 1.f / ((float)NN * d2),
+           g.lo_end, g.hi_start, g.tw);
     const int n = batch * rings.n;
-    k_detector_finish<<<(n + 127) / 128, 128, 0, st>>>(partial, out, tiles, rings.n, batch, weight);
-    FDES_LAUNCH_CHECK();
+    launch(k_detector_finish, (n + 127) / 128, 128, 0, st, partial, out, tiles, rings.n, batch, weight);
 }
 
 // 4D-STEM: scratch[b][qy][qx] = |FFT_col(Psi_b)|^2 at the window pixel (qy, qx) of the fftshifted pattern, for the
@@ -1581,12 +1498,9 @@ void launch_detector4d_cols_n(const SweepGeom& g, const cpx* Psi, float* scratch
 {
     using C = ColCfg<NN>;
     static_assert((size_t)NN * (C::CW + 1) * sizeof(float) <= C::SMEM, "intensity tile must fit the line buffers");
-    FDES_ALLOW_SMEM((k_detector4d_cols<NN>), C::SMEM);
     dim3 grid(band_cols(g) / C::CW, batch);
-    k_detector4d_cols<NN><<<grid, C::THREADS, C::SMEM, st>>>(Psi, scratch, Q, g.lo_end, g.hi_start, g.tw);
-    FDES_LAUNCH_CHECK();
+    launch(k_detector4d_cols<NN>, grid, C::THREADS, C::SMEM, st, Psi, scratch, Q, g.lo_end, g.hi_start, g.tw);
     launch_detector4d_finish(scratch, out, Q, bin, weight, batch, st);
-    FDES_LAUNCH_CHECK();
 }
 
 // ---------------------------------------------------------------------------------------------

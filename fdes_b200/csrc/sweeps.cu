@@ -3,6 +3,8 @@
 // one-thread-per-pixel chain of the reference's per-slice loop (phaseGrating,
 // src/crystalMaker.cu:507-536; forwardPropagation, src/multisliceSimulation.cu:538-611).
 #include "sweep_vtable.h"
+#include <map>
+#include <mutex>
 #include <stdexcept>
 #include <string>
 
@@ -11,6 +13,43 @@ namespace fdes {
 // read by pipe_grid (sweep_kernels.cuh), which every size's translation unit compiles
 thread_local int pipe_cta_cap = 0;
 thread_local int pipe_last_grid = 0;
+thread_local long long launch_tally = 0;
+
+// Function attributes are per device: the dynamic shared-memory limit is raised per kernel and device, and only
+// when a launch needs more than was set before, so launches into a stream capture do not touch the attribute.
+static void allow_smem(const void* kernel, size_t bytes)
+{
+    if (bytes <= 48 * 1024) return;
+    static std::mutex mu;
+    static std::map<std::pair<const void*, int>, size_t> have;
+    int dev = 0;
+    CK(cudaGetDevice(&dev));
+    std::lock_guard<std::mutex> lk(mu);
+    size_t& cur = have[{kernel, dev}];
+    if (bytes > cur) {
+        CK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+        cur = bytes;
+    }
+}
+
+void launch_args(const void* kernel, dim3 grid, dim3 block, size_t smem, cudaStream_t st, bool pdl, void** args)
+{
+    allow_smem(kernel, smem);
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = at; cfg.numAttrs = pdl ? 1 : 0;
+    const cudaError_t e = cudaLaunchKernelExC(&cfg, kernel, args);
+    if (e != cudaSuccess) {
+        cudaGetLastError();     // reported here; not again by a later check
+        const char* name = nullptr;
+        if (cudaFuncGetName(&name, kernel) != cudaSuccess || !name) name = "?";
+        throw std::runtime_error(std::string("CUDA error: ") + cudaGetErrorString(e) + " launching " + name);
+    }
+    launch_tally++;
+}
 
 static const SweepVTable* find_fast_vtable(int N)
 {

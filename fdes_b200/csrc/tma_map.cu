@@ -36,7 +36,7 @@ std::vector<Entry> g_cache;
 void tile_map(CUtensorMap_st* out, const void* base, int N, int nimg, int CW, int BR)
 {
     int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) throw std::runtime_error("cudaGetDevice failed");
+    CK(cudaGetDevice(&dev));
     std::lock_guard<std::mutex> lk(g_mutex);
     for (const Entry& e : g_cache)
         if (e.base == base && e.N == N && e.nimg == nimg && e.CW == CW && e.BR == BR && e.dev == dev) { *out = e.map; return; }

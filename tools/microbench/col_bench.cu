@@ -9,8 +9,6 @@
 #include <cstring>
 using namespace fdes;
 
-#define CK(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) { printf("CUDA error %s at line %d\n", cudaGetErrorString(e_), __LINE__); exit(1);} } while (0)
-
 // copy of k_propagate_cols_tma with the debug switches of ColPipe and per-CTA cycle counters:
 // dbg[cta] = {total, waiting for the landed tile, waiting for the previous store to drain, release}
 template <int N, int DBG>
