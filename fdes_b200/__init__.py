@@ -368,6 +368,9 @@ def fft2d(a: np.ndarray, direction: int = -1, gpu_index: int = 0) -> np.ndarray:
 SWEEP_GEOM, SWEEP_DENSITY, SWEEP_POTENTIAL, SWEEP_TRANSMIT, SWEEP_BANDLIMIT, SWEEP_MULTIPLY, SWEEP_PROPAGATE, \
     SWEEP_PROPAGATE_FROM, SWEEP_COLS_FFT, SWEEP_ROWS_FFT_SUM, SWEEP_ROWS_FFT, SWEEP_PROBE, SWEEP_DETECTOR = range(13)
 SWEEP_DETECTOR4D = 13
+# the set-up, per-pixel and atom kernels through the same hook
+SCATTER_TABLE, PROP_TABLE, LENS_TABLE, DETECTOR_TABLE, TILT_BEAM, TUKEY, AREA_MASK, NORM2, PEER_SUM, JITTER, ANSCOMBE, \
+    RECORDS, PLANE_WAVE, ZERO_OUTBAND, ABSORPTIVE, SCALE_CPX = range(14, 30)
 # ColOp and RowEpilogue values (fdes_b200/csrc/kernels.cuh)
 COL_PLAIN, COL_MUL_CPX_INV, COL_MUL_REAL_INV, COL_DP_ACCUM = range(4)
 ROW_STORE, ROW_ACCUM, ROW_INTENS_ACCUM, ROW_STORE_SHIFT, ROW_CROP_REAL = range(5)

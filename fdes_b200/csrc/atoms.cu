@@ -304,4 +304,15 @@ void launch_row_masks(int* rowptr, size_t rp_stride, int nkeys, int N, int E, in
     launch(k_row_masks, dim3((nwords + 255) / 256, nconf), 256, 0, st, rowptr, rp_stride, nkeys, N, E);
 }
 
+void launch_build_records(const float* xyz, const int* zidx, const float* occ, int nAt, const BinGeom& bg,
+                          const SortBuffers& sb, int* rowptr, size_t rp_stride, int key_bits, int mask_E, int nconf,
+                          cudaStream_t st)
+{
+    const int nrec = 4 * nAt, nkeys = bg.m3 * bg.nZ * bg.m2;
+    launch_bin_atoms(xyz, zidx, occ, nAt, bg, sb.keys, sb.cols, sb.w, nullptr, nconf, st);
+    launch_radix_sort(sb, nrec, key_bits, nconf, st);
+    launch_row_pointers(sb.keys, nrec, rowptr, nkeys, nconf, st, rp_stride);
+    if (mask_E > 0) launch_row_masks(rowptr, rp_stride, nkeys, bg.m1, mask_E, nconf, st);
+}
+
 }  // namespace fdes

@@ -592,7 +592,10 @@ int fdes_b200_sweep_test(int op, int N, int batch, const int* iargs, int n_iargs
         if (i >= nbufs || !bufs[i] || buf_elems[i] < (long long)words)
             throw std::runtime_error("sweep test: buffer " + std::to_string(i) + " needs " + std::to_string(words) + " words");
     };
-    if (!fft_size_supported(N)) throw std::runtime_error("unsupported FFT size");
+    // ops from FDES_B200_SCATTER_TABLE on run no sweep: N is any grid size or element count
+    const bool sweep = op < FDES_B200_SCATTER_TABLE;
+    if (sweep && !fft_size_supported(N)) throw std::runtime_error("unsupported FFT size");
+    if (N < 1) throw std::runtime_error("sweep test: N must be >= 1");
     if (op == FDES_B200_SWEEP_GEOM) {
         need(0, 5);
         const SweepGeom g = make_sweep_geom(N, nullptr, 0);
@@ -613,10 +616,14 @@ int fdes_b200_sweep_test(int op, int N, int batch, const int* iargs, int n_iargs
     // copy of this call is queued on the same stream, so the row masks and the sweep see the uploaded data
     CK(cudaStreamCreateWithFlags(&da.st, cudaStreamNonBlocking));
     const cudaStream_t st = da.st;
-    const std::vector<cpx> twh = make_twiddles(N);
-    cpx* tw = static_cast<cpx*>(da.get(twh.size() * sizeof(cpx)));
-    CK(cudaMemcpyAsync(tw, twh.data(), twh.size() * sizeof(cpx), cudaMemcpyHostToDevice, st));
-    SweepGeom g = make_sweep_geom(N, tw, 0);
+    std::vector<cpx> twh;
+    SweepGeom g{};
+    if (sweep) {
+        twh = make_twiddles(N);
+        cpx* tw = static_cast<cpx*>(da.get(twh.size() * sizeof(cpx)));
+        CK(cudaMemcpyAsync(tw, twh.data(), twh.size() * sizeof(cpx), cudaMemcpyHostToDevice, st));
+        g = make_sweep_geom(N, tw, 0);
+    }
     // row pointers of S1 / S2 (buffer rp_buf) go up in the engine's layout, not word for word
     int rp_buf = -1, nconf = 0, nkeys = 0;
     RecordRows rows;
@@ -767,6 +774,125 @@ int fdes_b200_sweep_test(int op, int N, int batch, const int* iargs, int n_iargs
             CK(cudaMemcpyAsync(scratch, h.data(), h.size() * sizeof(float), cudaMemcpyHostToDevice, st));
             launch_detector4d_cols(g, c(0), scratch, d[1], Q, bin, fa(0), batch, st);
             CK(cudaStreamSynchronize(st));     // h goes out of scope
+        } break;
+        case FDES_B200_SCATTER_TABLE:
+            need(0, Q * Q);
+            launch_scattering_table(d[0], N, kirkland_row(ia(0)), fa(0), fa(1), fa(2), Params().cst_pi, st);
+            break;
+        case FDES_B200_PROP_TABLE:
+            need(0, 2 * Q * Q);
+            launch_propagator_table(c(0), N, fa(0), fa(1), fa(2), fa(3), Params().cst_pi, st);
+            break;
+        case FDES_B200_LENS_TABLE: {
+            need(0, IMG);
+            LensParams lp;
+            for (int a = 0; a < AB_COUNT; a++) { lp.ab0[a] = fa(a); lp.ab1[a] = fa(AB_COUNT + a); }
+            lp.defocus_k = fa(28); lp.defocspread = fa(29); lp.lambda = fa(30); lp.d1 = fa(31); lp.d2 = fa(32);
+            lp.ObjAp = fa(33); lp.pi = Params().cst_pi; lp.mode = ia(0);
+            launch_lens_table(c(0), N, lp, fa(34), st, ia(1) != 0);
+        } break;
+        case FDES_B200_DETECTOR_TABLE: {
+            need(0, NN);
+            DetectorParams dp;
+            dp.mtfa = fa(0); dp.mtfb = fa(1); dp.mtfc = fa(2); dp.mtfd = fa(3); dp.illangle = fa(4); dp.defocus_k = fa(5);
+            dp.lambda = fa(6); dp.d1 = fa(7); dp.d2 = fa(8); dp.pi = Params().cst_pi;
+            dp.mode = ia(0); dp.use_incoherence = ia(1); dp.use_mtf = ia(2);
+            launch_detector_table(d[0], N, dp, fa(9), st);
+        } break;
+        case FDES_B200_TILT_BEAM:
+            if (ia(0) != 1 && ia(0) != -1) throw std::runtime_error("sweep test: flag must be +1 or -1");
+            need(0, IMG);
+            launch_tilt_beam(c(0), N, fa(0), fa(1), fa(2), fa(3), fa(4), Params().cst_pi, ia(0), st);
+            break;
+        case FDES_B200_TUKEY:
+        case FDES_B200_AREA_MASK:
+            if (ia(0) < 0 || ia(0) > N || ia(1) < 0 || ia(1) > N) throw std::runtime_error("sweep test: dn1, dn2 must be in [0, N]");
+            need(0, IMG);
+            if (op == FDES_B200_TUKEY) launch_tukey_window(c(0), N, ia(0), ia(1), Params().cst_pi, st);
+            else launch_area_mask_blend(c(0), N, ia(0), ia(1), st);
+            break;
+        case FDES_B200_NORM2: {
+            need(0, 2 * (size_t)N); need(1, 2);
+            double* dd = static_cast<double*>(da.get(257 * sizeof(double)));
+            launch_norm2(c(0), (size_t)N, dd, dd + 256, st);
+            CK(cudaMemcpyAsync(d[1], dd + 256, sizeof(double), cudaMemcpyDeviceToDevice, st));
+        } break;
+        case FDES_B200_PEER_SUM: {
+            PeerSources src{};
+            src.n = ia(0);
+            if (src.n < 1 || src.n > MAX_PEERS) throw std::runtime_error("sweep test: 1.." + std::to_string(MAX_PEERS) + " sources");
+            for (int r = 0; r <= src.n; r++) need(r, (size_t)N);
+            for (int r = 0; r < src.n; r++) src.p[r] = d[1 + r];
+            launch_peer_sum(d[0], src, (size_t)N, st);
+        } break;
+        case FDES_B200_JITTER: {
+            const size_t n3 = 3 * (size_t)N;
+            if (n_iargs < 2 || n_iargs % 2) throw std::runtime_error("sweep test: (burn, nconf) pairs expected");
+            long long confs = 0;
+            for (int i = 0; i < n_iargs; i += 2) {
+                if (ia(i) >= 0 && ia(i + 1) < 1) throw std::runtime_error("sweep test: nconf must be >= 1");
+                if (ia(i) >= 0) confs += ia(i + 1);
+            }
+            if (n3 > INT_MAX) throw std::runtime_error("sweep test: too many atoms");
+            need(0, n3); need(1, (size_t)N); need(2, (size_t)confs * n3);
+            void* states = da.get(rng_state_bytes() * n3);
+            launch_rng_init(states, (int)n3, 1ULL, st);
+            float* out = d[2];
+            for (int i = 0; i < n_iargs; i += 2) {
+                if (ia(i) < 0) { launch_rng_init(states, (int)n3, 1ULL, st); continue; }   // the streams start again
+                launch_atom_jitter(out, d[0], d[1], N, states, ia(i), ia(i + 1), st);
+                out += (size_t)ia(i + 1) * n3;
+            }
+        } break;
+        case FDES_B200_ANSCOMBE: {
+            const bool second = nbufs > 1 && buf_elems[1] > 0;
+            need(0, 2 * (size_t)N);
+            if (second) need(1, 2 * (size_t)N);
+            void* states = da.get(rng_state_bytes() * (size_t)N);
+            launch_rng_init(states, N, (unsigned long long)ia(0), st);
+            launch_anscombe_noise(c(0), (size_t)N, fa(0), states, st);
+            if (second) launch_anscombe_noise(c(1), (size_t)N, fa(0), states, st);
+        } break;
+        case FDES_B200_PLANE_WAVE:
+            need(0, (size_t)batch * IMG);
+            launch_plane_wave_rowspace(c(0), N, batch, st);
+            break;
+        case FDES_B200_ZERO_OUTBAND:
+            if (ia(0) < 0 || ia(1) < ia(0) || ia(1) > N) throw std::runtime_error("sweep test: need 0 <= lo_end <= hi_start <= N");
+            need(0, (size_t)batch * IMG);
+            launch_zero_outband(c(0), N, ia(0), ia(1), batch, st);
+            break;
+        case FDES_B200_ABSORPTIVE:
+            need(0, 2 * (size_t)N);
+            launch_absorptive_factor(c(0), (size_t)N, fa(0), st);
+            break;
+        case FDES_B200_SCALE_CPX:
+            need(0, 2 * (size_t)N);
+            launch_scale_cpx(c(0), (size_t)N, fa(0), st);
+            break;
+        case FDES_B200_RECORDS: {
+            const int m3 = ia(0), nZ = ia(1), nconf_r = ia(2);
+            const int nAt = nbufs > 1 ? (int)std::min<long long>(buf_elems[1], INT_MAX / 4) : 0;
+            if (m3 < 1 || nZ < 1 || nconf_r < 1 || nAt < 1) throw std::runtime_error("sweep test: bad records arguments");
+            if ((long long)m3 * nZ * N >= (1LL << 31) - 2) throw std::runtime_error("sweep test: too many row keys");
+            const int nk = m3 * nZ * N, nrec = 4 * nAt;
+            int key_bits = 0;
+            while ((1LL << key_bits) <= (long long)nk) key_bits++;
+            const int E = fft_size_supported(N) ? line_points(N) : 0;
+            const size_t rp_stride = (size_t)nk + 1 + (E > 0 ? (size_t)(nk / N) * (N / E) : 0);
+            const size_t nr = (size_t)nconf_r * nrec;
+            need(0, (size_t)nconf_r * 3 * nAt); need(2, nAt); need(3, nr); need(4, nr); need(5, nr);
+            need(6, (size_t)nconf_r * rp_stride);
+            const int* zi = reinterpret_cast<const int*>(bufs[1]);
+            for (int i = 0; i < nAt; i++)
+                if (zi[i] < 0 || zi[i] >= nZ) throw std::runtime_error("sweep test: species index outside [0, nZ)");
+            SortBuffers sb{reinterpret_cast<uint32_t*>(d[3]), static_cast<uint32_t*>(da.get(nr * 4)),
+                           reinterpret_cast<int*>(d[4]), static_cast<int*>(da.get(nr * 4)), d[5],
+                           static_cast<float*>(da.get(nr * 4)),
+                           static_cast<unsigned int*>(da.get((size_t)nconf_r * 256 * sort_num_blocks(nrec) * 4))};
+            const BinGeom bg{N, N, m3, nZ, fa(0), fa(1), fa(2)};
+            launch_build_records(d[0], reinterpret_cast<const int*>(d[1]), d[2], nAt, bg, sb, reinterpret_cast<int*>(d[6]),
+                                 rp_stride, key_bits, E, nconf_r, st);
         } break;
         default: throw std::runtime_error("sweep test: unknown op " + std::to_string(op));
     }

@@ -35,10 +35,6 @@ struct PhaseTimer {
 };
 }  // namespace
 
-static const KirklandRow kKirkland[103] = {
-#include "kirkland_table.inc"
-};
-
 // Every public entry point runs on the engine's own device, whatever the caller's current device
 // is (torch switching devices, several engines of one process on different GPUs), and restores
 // the caller's device on the way out (Engine::Call).
@@ -337,16 +333,8 @@ void Engine::setup_tables()
 
     launch_propagator_table(Pq_, N_, p_.d1, p_.d2, p_.d3, p_.lambda, p_.cst_pi, st_);
     const size_t Q = (size_t)(N_ / 2 + 1);
-    for (int z = 0; z < nZ_; z++) {
-        KirklandRow kr;
-        const int Z = Zlist_[z];
-        if (Z >= 1 && Z <= 103) kr = kKirkland[Z - 1];
-        else {   // unknown element: a = 0, b = 1, c = 1, d = 0 (src/projectedPotential.cu:2984-3009)
-            const float fb[12] = {0, 1, 0, 1, 0, 1, 1, 0, 1, 0, 1, 0};
-            memcpy(kr.v, fb, sizeof fb);
-        }
-        launch_scattering_table(Gq_ + (size_t)z * Q * Q, N_, kr, p_.d1, p_.d2, p_.sigma, p_.cst_pi, st_);
-    }
+    for (int z = 0; z < nZ_; z++)
+        launch_scattering_table(Gq_ + (size_t)z * Q * Q, N_, kirkland_row(Zlist_[z]), p_.d1, p_.d2, p_.sigma, p_.cst_pi, st_);
 }
 
 void Engine::tilt(float* xyz, float t0, float t1, float t2)
@@ -435,14 +423,10 @@ void Engine::bin_and_sort(int b0, int nconf, const float* xyz_dev, int set, cuda
     if (!st) st = st_;
     const RecordSet& r = rs_[set];
     BinGeom bg{N_, N_, p_.m3, nZ_, p_.d1, p_.d2, p_.d3};
-    uint32_t* keys = r.keys + (size_t)b0 * nrec_;
-    int* cols = r.cols + (size_t)b0 * nrec_;
-    float* w = r.w + (size_t)b0 * nrec_;
-    launch_bin_atoms(xyz_dev, zidx_, occ_, nAt_, bg, keys, cols, w, nullptr, nconf, st);
-    SortBuffers sb{keys, keys_tmp_, cols, cols_tmp_, w, w_tmp_, hist_};
-    launch_radix_sort(sb, nrec_, key_bits_, nconf, st);
-    launch_row_pointers(keys, nrec_, r.rowptr + (size_t)b0 * rp_stride_, nkeys_, nconf, st, rp_stride_);
-    if (mask_E_ > 0) launch_row_masks(r.rowptr + (size_t)b0 * rp_stride_, rp_stride_, nkeys_, N_, mask_E_, nconf, st);
+    SortBuffers sb{r.keys + (size_t)b0 * nrec_, keys_tmp_, r.cols + (size_t)b0 * nrec_, cols_tmp_,
+                   r.w + (size_t)b0 * nrec_, w_tmp_, hist_};
+    launch_build_records(xyz_dev, zidx_, occ_, nAt_, bg, sb, r.rowptr + (size_t)b0 * rp_stride_, rp_stride_, key_bits_,
+                         mask_E_, nconf, st);
 }
 
 // jitter + bin + sort + row pointers for the configurations of one batch (slots 0 .. nb-1)

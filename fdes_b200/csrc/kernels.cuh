@@ -135,6 +135,9 @@ void launch_cols_fft(const SweepGeom& g, const cpx* in, void* out, int dir, ColO
 
 // ---- set-up kernels (tables follow the reference's float32 expressions) ------------------
 struct KirklandRow { float v[12]; };  // a0 b0 a1 b1 a2 b2 c0 d0 c1 d1 c2 d2
+// parameters of atomic number Z (kirkland_table.inc, Z = 1..103); any other Z: the reference's unknown-element
+// fallback a = 0, b = 1, c = 1, d = 0 (src/projectedPotential.cu:2984-3009)
+KirklandRow kirkland_row(int Z);
 // Gq[(N/2+1)^2]: scattering factor * sinc correction * normalisation (projectedPotential_d +
 // divideBySinc, reference src/projectedPotential.cu:30-73, src/crystalMaker.cu:136-158)
 void launch_scattering_table(float* Gq, int N, KirklandRow kr, float d1, float d2, float sigma,
@@ -228,5 +231,11 @@ void launch_radix_sort(const SortBuffers& sb, int n, int key_bits, int nconf, cu
 void launch_row_masks(int* rowptr, size_t rp_stride, int nkeys, int N, int E, int nconf, cudaStream_t st);
 void launch_row_pointers(const uint32_t* keys_sorted, int n, int* rowptr, int nkeys, int nconf,
                          cudaStream_t st, size_t rp_stride = 0);   // rp_stride 0: nkeys + 1
+// The deposit records of nconf configurations as the slice loop reads them: binning of xyz [nconf][nAt][3] into
+// sb.keys / cols / w [nconf][4 nAt], the stable sort (key_bits: bits of the largest key, nkeys = m3 * nZ * m2),
+// row pointers and, when mask_E > 0, the row masks of an N = bg.m1 grid; rowptr: [nconf][rp_stride]
+void launch_build_records(const float* xyz, const int* zidx, const float* occ, int nAt, const BinGeom& bg,
+                          const SortBuffers& sb, int* rowptr, size_t rp_stride, int key_bits, int mask_E, int nconf,
+                          cudaStream_t st);
 
 }  // namespace fdes

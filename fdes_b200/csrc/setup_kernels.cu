@@ -41,6 +41,16 @@ __global__ void k_scattering_table(float* __restrict__ Gq, int N, KirklandRow kr
     Gq[i] = V * inv_sinc;
 }
 
+static const KirklandRow kKirkland[103] = {
+#include "kirkland_table.inc"
+};
+
+KirklandRow kirkland_row(int Z)
+{
+    if (Z >= 1 && Z <= 103) return kKirkland[Z - 1];
+    return KirklandRow{{0, 1, 0, 1, 0, 1, 1, 0, 1, 0, 1, 0}};
+}
+
 void launch_scattering_table(float* Gq, int N, KirklandRow kr, float d1, float d2, float sigma,
                              float pi, cudaStream_t st)
 {

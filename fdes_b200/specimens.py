@@ -84,12 +84,20 @@ def write_cnf(path, *, image_size: int, border_size: int, slices: int, pixel_siz
               mtf: Sequence[float] = (1.0, 0.0, 0.0, 0.0), aberrations: Optional[Dict[str, Tuple[float, float]]] = None,
               specimen_tilts: Optional[Iterable[Tuple[float, float]]] = None,
               beam_tilts: Optional[Iterable[Tuple[float, float]]] = None, defoci: Optional[Iterable[float]] = None,
-              tilt_offset: Sequence[float] = (0.0, 0.0, 0.0), comment: str = "fdes_b200 synthetic specimen") -> pathlib.Path:
+              tilt_offset: Sequence[float] = (0.0, 0.0, 0.0), comment: str = "fdes_b200 synthetic specimen",
+              pixel_size_y: Optional[float] = None, image_size_y: Optional[int] = None,
+              border_size_y: Optional[int] = None) -> pathlib.Path:
     """Write a parameter file (atoms optional: FDES() takes them as an array).  The file does not
-    end with a newline: the reference reader would read the last atom twice otherwise."""
+    end with a newline: the reference reader would read the last atom twice otherwise.  The y sizes default to the
+    x ones; the sample stays square (image_size + 2 border_size == image_size_y + 2 border_size_y)."""
+    py = pixel_size if pixel_size_y is None else pixel_size_y
+    ny = image_size if image_size_y is None else image_size_y
+    by = border_size if border_size_y is None else border_size_y
     ab = {k: (0.0, 0.0) for k in _ABERRATIONS}
     ab.update(aberrations or {})
     m = image_size + 2 * border_size
+    if ny + 2 * by != m:
+        raise ValueError(f"image_size_y + 2 border_size_y = {ny + 2 * by} != {m}: the sample must be square")
     L = [f"comment: {comment}", f"voltage: {voltage:.9g}", f"focus_spread: {focus_spread:.9g}",
          f"illumination_angle: {illumination_angle:.9g}", f"mtf_a: {mtf[0]:.9g}", f"mtf_b: {mtf[1]:.9g}",
          f"mtf_c: {mtf[2]:.9g}", f"mtf_d: {mtf[3]:.9g}", f"objective_aperture: {objective_aperture:.9g}"]
@@ -97,9 +105,9 @@ def write_cnf(path, *, image_size: int, border_size: int, slices: int, pixel_siz
         L.append(f"{k}: {ab[k][0]:.9g}" if k in _ROUND else f"{k}: {ab[k][0]:.9g} {ab[k][1]:.9g}")
     sub = slice_thickness if sub_slice_thickness is None else sub_slice_thickness
     L += [f"mode: {mode}", f"sample_size_x: {m}", f"sample_size_y: {m}", f"sample_size_z: {slices}",
-          f"pixel_size_x: {pixel_size:.9g}", f"pixel_size_y: {pixel_size:.9g}", f"pixel_size_z: {slice_thickness:.9g}",
-          f"border_size_x: {border_size}", f"border_size_y: {border_size}", f"image_size_x: {image_size}",
-          f"image_size_y: {image_size}", f"image_size_z: {image_size_z}",
+          f"pixel_size_x: {pixel_size:.9g}", f"pixel_size_y: {py:.9g}", f"pixel_size_z: {slice_thickness:.9g}",
+          f"border_size_x: {border_size}", f"border_size_y: {by}", f"image_size_x: {image_size}",
+          f"image_size_y: {ny}", f"image_size_z: {image_size_z}",
           f"specimen_tilt_offset_x: {tilt_offset[0]:.9g}", f"specimen_tilt_offset_y: {tilt_offset[1]:.9g}",
           f"specimen_tilt_offset_z: {tilt_offset[2]:.9g}", f"frozen_phonons: {frozen_phonons}", "pixel_dose: 0.0",
           f"subpixel_size_z: {sub:.9g}", "sample_name: synthetic", "material: synthetic",

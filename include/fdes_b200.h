@@ -243,7 +243,43 @@ int fdes_b200_sort_records(unsigned int* keys, int* cols, float* w, int n, int n
  *   FDES_B200_SWEEP_DETECTOR4D Q bin                                        weight  Psi [batch], out [batch][Q/bin]
  *                                                                                   [Q/bin] (accumulated into); the
  *                                                                                   [batch][Q][Q] scratch starts as
- *                                                                                   NaN in the band columns */
+ *                                                                                   NaN in the band columns
+ * The set-up, per-pixel and atom kernels, each through its production launcher (no FFT size needed; N is the
+ * grid size unless noted; pi is the engine's 3.1415927f):
+ *   FDES_B200_SCATTER_TABLE   Z (kirkland_row: 1..103, else the          d1 d2   Gq [(N/2+1)^2] out, [|kx|][|ky|]
+ *                             unknown-element fallback)                   sigma   (ky fastest)
+ *   FDES_B200_PROP_TABLE      -                                     d1 d2 d3 lambda Pq [(N/2+1)^2] out
+ *   FDES_B200_LENS_TABLE      mode transposed                       ab0[14] ab1[14] tab [N*N] out ([ky][kx]; [kx][ky]
+ *                                                                   defocus spread  when transposed)
+ *                                                                   lambda d1 d2
+ *                                                                   ObjAp extra_scale
+ *   FDES_B200_DETECTOR_TABLE  mode use_incoherence use_mtf          mtfa mtfb mtfc  tab float [N*N] out
+ *                                                                   mtfd illangle
+ *                                                                   defocus lambda
+ *                                                                   d1 d2 scale
+ *   FDES_B200_TILT_BEAM       flag (+1 / -1)                        d1 d2 lambda    psi [N*N] in/out
+ *                                                                   tb_x tb_y
+ *   FDES_B200_TUKEY           dn1 dn2 (0..N)                        -       psi [N*N] in/out
+ *   FDES_B200_AREA_MASK       dn1 dn2 (0..N)                        -       psi [N*N] in/out
+ *   FDES_B200_NORM2           - (N = elements)                      -       p [N] (complex), out: the double sum of
+ *                                                                           |p|^2 in 2 words
+ *   FDES_B200_PEER_SUM        nsrc (1..15) (N = floats)             -       dst float [N] in/out, src_1..src_nsrc [N]
+ *   FDES_B200_JITTER          (burn, nconf) pairs (N = atoms):      -       xyz [N][3], dwf [N], out [sum nconf][N][3]
+ *                             streams curand_init(1, i, 0), i < 3N,         (the calls' configurations in order)
+ *                             then one launch_atom_jitter per pair;
+ *                             burn < 0: the streams start again
+ *   FDES_B200_ANSCOMBE        seed (N = pixels)                     dose    f [N] in/out (complex, real part
+ *                                                                           used), optional f2 [N]: a second call
+ *                                                                           on the same streams (0 words: none)
+ *   FDES_B200_RECORDS         m3 nZ nconf (N = m1 = m2)             d1 d2   xyz [nconf][nAt][3], zidx (int) [nAt],
+ *                             launch_build_records as the engine    d3      occ [nAt], keys (uint), cols (int), w
+ *                             runs it: binning, sort, row pointers,         [nconf][4 nAt] out, rowptr (int)
+ *                             row masks (where the size has them)           [nconf][rp_stride] out, rp_stride = nkeys
+ *                                                                           + 1 + mask words, nkeys = m3 nZ N
+ *   FDES_B200_PLANE_WAVE      - (batch images)                      -       Psi [batch][N*N] out
+ *   FDES_B200_ZERO_OUTBAND    lo_end hi_start (batch images)        -       Psi [batch][N*N] in/out
+ *   FDES_B200_ABSORPTIVE      - (N = elements)                      imPot   V [N] in/out (complex)
+ *   FDES_B200_SCALE_CPX       - (N = elements)                      s       p [N] in/out (complex) */
 #define FDES_B200_SWEEP_GEOM 0
 #define FDES_B200_SWEEP_DENSITY 1
 #define FDES_B200_SWEEP_POTENTIAL 2
@@ -258,6 +294,22 @@ int fdes_b200_sort_records(unsigned int* keys, int* cols, float* w, int n, int n
 #define FDES_B200_SWEEP_PROBE 11
 #define FDES_B200_SWEEP_DETECTOR 12
 #define FDES_B200_SWEEP_DETECTOR4D 13
+#define FDES_B200_SCATTER_TABLE 14
+#define FDES_B200_PROP_TABLE 15
+#define FDES_B200_LENS_TABLE 16
+#define FDES_B200_DETECTOR_TABLE 17
+#define FDES_B200_TILT_BEAM 18
+#define FDES_B200_TUKEY 19
+#define FDES_B200_AREA_MASK 20
+#define FDES_B200_NORM2 21
+#define FDES_B200_PEER_SUM 22
+#define FDES_B200_JITTER 23
+#define FDES_B200_ANSCOMBE 24
+#define FDES_B200_RECORDS 25
+#define FDES_B200_PLANE_WAVE 26
+#define FDES_B200_ZERO_OUTBAND 27
+#define FDES_B200_ABSORPTIVE 28
+#define FDES_B200_SCALE_CPX 29
 int fdes_b200_sweep_test(int op, int N, int batch, const int* iargs, int n_iargs, const float* fargs, int n_fargs,
                          float** bufs, const long long* buf_elems, int nbufs, int gpu_index, int pipe_ctas,
                          int* pipe_grid_out);
